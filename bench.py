@@ -54,7 +54,32 @@ def parse():
     ap.add_argument("--extras-budget-s", type=float, default=150.0, help="wall-clock budget of the extras")
     ap.add_argument("--n-context", type=int, default=None)
     ap.add_argument("--n-target", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (loss, log_prob, bpd) as DIR/<name>.npy (float32, at most "
+                         "64 MB: a fixed sample of log_prob above that); rank 0 only")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64 << 20       # cap on everything --dump-outputs writes
+
+
+def dump_outputs(d, loss, lp, bpd):
+    """The arrays a caller of the timed path receives, from its last step.  Inputs and weights are seeded, so two builds run
+    with the same arguments can be compared output for output.  log_prob [B, N] is 4*B*N bytes (0.5 MB at the default shape);
+    above the cap, log_prob_sample.npy holds a fixed sample of its points (seed 0, ascending flat index b*N + n) and
+    log_prob_sample_index.npy those flat indices (float64, exact below 2**53)."""
+    os.makedirs(d, exist_ok=True)
+    lp = lp.detach().float()
+    arrays = {"loss": loss.detach().float(), "bpd": bpd.detach().float()}
+    budget = DUMP_BYTES - 4096          # room for the .npy headers and the two scalars
+    if 4 * lp.numel() <= budget:
+        arrays["log_prob"] = lp
+    else:
+        idx = torch.randperm(lp.numel(), generator=torch.Generator().manual_seed(0))[:budget // 12].sort().values
+        arrays["log_prob_sample"] = lp.reshape(-1)[idx.to(lp.device)]
+        arrays["log_prob_sample_index"] = idx.double()
+    for name, t in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), t.cpu().numpy())
 
 
 def peaks():
@@ -149,8 +174,10 @@ def run_reference(args):
             port.inner_loop(a, fsd, esd, dcfg, batch["eps"])
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            port.inner_loop(a, fsd, esd, dcfg, batch["eps"])
+            loss, lp, bpd = port.inner_loop(a, fsd, esd, dcfg, batch["eps"])
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss, lp, bpd)
     v = args.steps / dt
     out = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
            "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -448,6 +475,8 @@ def main():
         dist.barrier()
     ms = ev0.elapsed_time(ev1)
     note("timed region done")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, lp, bpd)
     if world > 1:   # outside the timed region: collect the per-cloud nats of every rank (what a caller would do once)
         dist.all_gather(gathered, lp.mean(dim=1))
     launches = lib.launch_count() - n0

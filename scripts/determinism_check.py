@@ -1,5 +1,5 @@
 import sys, os, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from flowcompare_b200 import configs, engine, spec
 torch.set_grad_enabled(False)
 cfg = configs.get_config("dgcnn_attn", n_flow_layers=12)

@@ -6,8 +6,9 @@ fc_group_points, through flowcompare_b200.pointops -> ctypes -> C ABI) against
   * the CPU restatement oracle/pointops_ref.c (which the PAConv goldens were generated with), so that restatement is
     pinned to the compiled reference too.
 
-/root/reference is not needed at run time: the .so travels with the repo snapshot.  If it is absent the reference
-comparisons are skipped and only the restatement is checked.
+The reference library is built from the reference's source tree, which is not part of the repository; without it the
+reference comparisons are skipped.  test_outputs_equal_pinned_digests then still catches any change of these kernels' outputs,
+against this project's own pinned outputs (tests/pointops_cases.py; not reference data).
 """
 import time
 
@@ -17,28 +18,19 @@ import torch
 from flowcompare_b200 import configs, pointops as fpo, spec
 from oracle import pointops_refcuda as ref
 from oracle import port_paconv
+from tests import pointops_cases as pc
+from tests.pointops_cases import FPS_CASES, KNN_CASES, NN_CASES
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 needs_ref = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libpointops_ref.so not built (needs /root/reference once)")
-
-
-def _cloud(B, n, seed, duplicates=False):
-    g = torch.Generator().manual_seed(seed)
-    x = torch.rand(B, n, 3, generator=g) * 2 - 1
-    if duplicates:   # the reference's loader oversamples small voxels: exact duplicate points (utils.py:362-370)
-        x[:, n // 2:] = x[:, : n - n // 2]
-    return x.contiguous()
-
-
-FPS_CASES = [(3, 1250, 312, False), (2, 312, 78, False), (2, 78, 19, False), (2, 19, 4, False), (1, 4096, 1024, False),
-             (2, 5000, 1250, False), (2, 1250, 312, True), (1, 2500, 700, True), (1, 33, 33, False)]
+_cloud = pc.cloud
 
 
 @needs_ref
 @pytest.mark.parametrize("B,n,m,dup", FPS_CASES)
 def test_fps_bit_exact_vs_reference_kernel(B, n, m, dup):
-    x = _cloud(B, n, n + m, dup).to(DEV)
+    x = pc.fps_inputs(B, n, m, dup)
     want = ref.furthestsampling(x, m)
     got, nx = fpo.furthestsampling(x, m, return_xyz=True)
     assert torch.equal(got, want)
@@ -71,15 +63,10 @@ def test_fps_lowest_index_tie_rule():
     assert got == want
 
 
-KNN_CASES = [(2, 1250, 312, 32, False), (2, 312, 78, 32, False), (2, 78, 19, 32, False), (2, 19, 4, 32, False),
-             (2, 1250, 312, 32, True), (1, 700, 700, 16, False), (1, 3000, 129, 40, False)]
-
-
 @needs_ref
 @pytest.mark.parametrize("B,n,m,k,dup", KNN_CASES)
 def test_knn_heap_bit_exact_vs_reference_kernel(B, n, m, k, dup):
-    x = _cloud(B, n, 3 * n + k, dup).to(DEV)
-    q = x[:, torch.randperm(n, generator=torch.Generator().manual_seed(n))[:m]].contiguous()
+    x, q = pc.knn_inputs(B, n, m, k, dup)
     want_idx, want_d2 = ref.knnquery_heap(k, x, q)
     got_idx, got_d2 = fpo.knnquery_heap(k, x, q, return_dist2=True)
     assert torch.equal(got_idx, want_idx)      # including the heap's order of exactly equal distances and the k > n padding
@@ -93,14 +80,10 @@ def test_knn_heap_matches_cpu_restatement(B, n, m, k, dup):
     assert torch.equal(fpo.knnquery_heap(k, x.to(DEV), q.to(DEV)).cpu(), port_paconv.knnquery_heap(k, x, q))
 
 
-NN_CASES = [(2, 1250, 312, False), (2, 312, 78, False), (2, 19, 4, False), (1, 7, 2, False), (2, 1250, 312, True), (1, 5000, 1250, False)]
-
-
 @needs_ref
 @pytest.mark.parametrize("B,n,m,dup", NN_CASES)
 def test_three_nn_bit_exact_vs_reference_kernel(B, n, m, dup):
-    u = _cloud(B, n, n + 7 * m, dup).to(DEV)
-    kn = u[:, :m].contiguous() if dup else _cloud(B, m, m, False).to(DEV)
+    u, kn = pc.nn_inputs(B, n, m, dup)
     want_d2, want_idx = ref.nearestneighbor(u, kn)
     got_d2, got_idx = fpo.nearestneighbor(u, kn, squared=True)
     assert torch.equal(got_idx, want_idx)
@@ -117,18 +100,18 @@ def test_three_nn_matches_cpu_restatement(B, n, m, dup):
 
 @needs_ref
 def test_interpolation_and_grouping_vs_reference_kernels():
-    g = torch.Generator().manual_seed(3)
-    B, c, m, n, k = 2, 67, 312, 1250, 32
-    feats = torch.randn(B, c, m, generator=g).to(DEV)
-    u, kn = _cloud(B, n, 1).to(DEV), _cloud(B, m, 2).to(DEV)
-    d, idx = fpo.nearestneighbor(u, kn)
-    w = 1.0 / (d + 1e-8)
-    w = (w / w.sum(dim=2, keepdim=True)).contiguous()
+    feats, idx, w, gidx, fidx = pc.interp_group_gather_inputs(fpo)
     assert torch.equal(fpo.interpolation(feats, idx, w), ref.interpolation(feats, idx, w))
-    gidx = torch.randint(0, m, (B, 100, k), generator=g, dtype=torch.int32).to(DEV)
     assert torch.equal(fpo.grouping(feats, gidx), ref.grouping(feats, gidx))
-    fidx = torch.randint(0, m, (B, 50), generator=g, dtype=torch.int32).to(DEV)
     assert torch.equal(fpo.gathering(feats, fidx), ref.gathering(feats, fidx))
+
+
+def test_outputs_equal_pinned_digests():
+    """Every output of every case above (indices, squared distances, interpolated / grouped / gathered features) is bit-identical
+    to this project's pinned outputs.  A regression check of these kernels, not a comparison with the reference."""
+    got, want = pc.output_digests(fpo), pc.load_pinned()
+    assert sorted(got) == sorted(want)
+    assert [k for k in sorted(got) if got[k] != want[k]] == []
 
 
 @needs_ref
