@@ -318,8 +318,15 @@ extern "C" int64_t fc_flow_workspace_bytes(const fc_flow* f, int B, int N, int N
 }
 
 // ------------------------------------------------------------------------------------------ forward
+// Which attention blocks' softmax weights a forward pass writes (fc_flow_attention_maps).  Slot 0 is the augmenter's attention,
+// slot l + 1 coupling layer l's; `slots` strictly increasing; the i-th captured block's maps [B, n_query, Nc] start at
+// out + i * B * n_query * Nc.
+struct FcCapture { const int32_t* slots; int n_slots; const int32_t* qidx; int n_query; float* out; };
+
+// maps: where this block's weights go (nullptr: not captured; `cap` then unused)
 static int run_attention_block(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const float* lat, int ldx, int K_in,
-                               const float* context, int B, int N, int Nc, FlowWs& w, int precision, cudaStream_t s) {
+                               const float* context, int B, int N, int Nc, FlowWs& w, int precision, cudaStream_t s,
+                               float* maps = nullptr, const FcCapture* cap = nullptr) {
     const int M = B * N;
     FcMlpIn in{lat, ldx, nullptr, 0, nullptr, 0, 0};
     (void)K_in;
@@ -341,6 +348,14 @@ static int run_attention_block(const fc_flow* f, const FcMlp& pre, const FcAttn&
     }
     // reference models/perceiver.py:104: scale = inner_dim ** -0.5
     const float scale = 1.0f / sqrtf((float)f->inner);
+    if (maps) {
+        // k through the plain epilogue into w.kv: the forward's own to_kv below either rewrites w.kv with the same values or
+        // (tensor-core path) writes its split copies elsewhere and never reads it, so the forward is unchanged by the capture
+        rc = gemm_plain(at.kv, context, f->E, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.kv, 128, B * Nc, precision, s);
+        if (rc) return rc;
+        rc = fc_launch_attention_maps(w.q, 64, w.kv, 128, cap->qidx, cap->n_query, maps, B, N, Nc, scale, s);
+        if (rc) return rc;
+    }
     static int attn_kind = -1;   // FC_ATTN=mma: warp-level MMA kernel; FC_ATTN=split: tcgen05 with a separate split pass (A/B runs)
     if (attn_kind < 0) { const char* e = getenv("FC_ATTN"); attn_kind = !e ? 0 : (e[0] == 'm' ? 1 : (e[0] == 's' ? 2 : 0)); }
     if (precision == 1 && attn_kind == 0 && at.kv.N == 128 && at.kv.whi) {
@@ -402,7 +417,7 @@ static int run_cif_block(const fc_flow* f, const FcFlowLayer& y, float* lat, Flo
 
 static int flow_forward(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
                         const float* eps_cif, float* log_prob_out, float* z_out, int B, int N, int Nc, void* workspace,
-                        int64_t workspace_bytes, int precision, fc_stream_t stream_) {
+                        int64_t workspace_bytes, int precision, fc_stream_t stream_, const FcCapture* cap = nullptr) {
     FC_REQUIRE(f && x && context && log_prob_out && B > 0 && N > 0 && Nc > 0);
     FC_REQUIRE(eps || !f->has_aug);
     FC_REQUIRE(eps_cif || !f->cif_dim);
@@ -437,10 +452,16 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
         if (rc) return rc;
     }
     auto cb_ptr = [&](int slot) -> const float* { return f->has_cb ? w.cb + (size_t)slot * f->hid : nullptr; };
+    int n_captured = 0;
+    auto maps_for = [&](int slot) -> float* {
+        if (!cap || n_captured >= cap->n_slots || cap->slots[n_captured] != slot) return nullptr;
+        return cap->out + (size_t)(n_captured++) * (size_t)B * (size_t)cap->n_query * (size_t)Nc;
+    };
 
     // ---- transforms.0: augment (reference models/augmenter.py:15-19, :49-63); latent_dim == input_dim: IdentityTransform
     if (f->has_aug && !f->is_global) {
-        rc = run_attention_block(f, f->augpre, f->augattn, w.lat0, w.ldx, f->d_in, context, B, N, Nc, w, precision, s);
+        rc = run_attention_block(f, f->augpre, f->augattn, w.lat0, w.ldx, f->d_in, context, B, N, Nc, w, precision, s,
+                                 maps_for(0), cap);
         if (rc) return rc;
     }
     if (f->has_aug) {
@@ -466,7 +487,8 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
             if (rc) return rc;
         }
         if (!f->is_global) {
-            rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, f->half, context, B, N, Nc, w, precision, s);
+            rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, f->half, context, B, N, Nc, w, precision, s,
+                                     maps_for(l + 1), cap);
             if (rc) return rc;
         }
         FcMlpIn in{lat, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(l + 1), w.cb_ld, N};
@@ -539,6 +561,22 @@ extern "C" int fc_flow_log_prob_cif(const fc_flow* f, const float* x, const floa
                                     const float* eps, const float* eps_cif, float* log_prob_out, int B, int N, int Nc,
                                     void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream_) {
     return flow_forward(f, x, context, extra, eps, eps_cif, log_prob_out, nullptr, B, N, Nc, workspace, workspace_bytes, precision, stream_);
+}
+
+// The forward pass that also writes the softmax weights of the attention blocks listed in slots_host (see FcCapture).
+extern "C" int fc_flow_attention_maps(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
+                                      const float* eps_cif, const int32_t* slots_host, int n_slots, const int32_t* query_idx,
+                                      int n_query, float* maps_out, float* log_prob_out, int B, int N, int Nc, void* workspace,
+                                      int64_t workspace_bytes, int precision, fc_stream_t stream_) {
+    FC_REQUIRE(f && slots_host && n_slots > 0 && maps_out && n_query > 0);
+    if (f->is_global) return FC_ERR_UNSUPPORTED;       // no attention over context points: the device never runs one
+    FC_REQUIRE(query_idx || n_query == N);
+    for (int i = 0; i < n_slots; ++i)
+        FC_REQUIRE(slots_host[i] >= 0 && slots_host[i] <= f->L && (i == 0 || slots_host[i] > slots_host[i - 1]));
+    FC_REQUIRE(slots_host[0] != 0 || f->has_aug);     // an identity augmenter has no attention
+    const FcCapture cap{slots_host, n_slots, query_idx, n_query, maps_out};
+    return flow_forward(f, x, context, extra, eps, eps_cif, log_prob_out, nullptr, B, N, Nc, workspace, workspace_bytes, precision,
+                        stream_, &cap);
 }
 
 extern "C" int fc_flow_cif_noise_dim(const fc_flow* f) { return f ? (f->cif_dim ? f->cif_dim - f->D : 0) : FC_ERR_INVALID_ARG; }

@@ -137,6 +137,9 @@ void fc_attention_tc_scratch_layout(int B, int Nc, float* scratch, float** khi, 
                                     int* ncp, int fmt);
 int fc_launch_cross_attention_tc(const float* q, int ldq, const float* kv, int ldkv, float* out, int ldo, int B, int N,
                                  int Nc, int d, float scale, float* scratch, int presplit, int fmt, cudaStream_t stream);
+// the softmax weights of one attention block, P [B, n_query, Nc] (attention_maps.cu); qidx: device list of query rows or null
+int fc_launch_attention_maps(const float* q, int ldq, const float* kv, int ldkv, const int32_t* qidx, int n_query,
+                             float* out, int B, int N, int Nc, float scale, cudaStream_t stream);
 int fc_launch_edgeconv_gather_max(const float* PQ, int ldpq, const int32_t* idx, int B, int N, int k, int Cout,
                                   float* out, int ldo, cudaStream_t stream);
 int fc_knn_launch(const float* q, int ldq, long long q_bstride, const float* t, int ldt, long long t_bstride,

@@ -225,6 +225,62 @@ class FlowCompareB200:
             _lib.check(rc, "fc_flow_forward")
         return out, z
 
+    @property
+    def attention_layer_names(self):
+        """Module names (the reference's, e.g. 'transforms.0.attn', 'transforms.1.pre_conditioner.attn') of the attention
+        blocks whose weights `attention_maps` returns, in transform order; empty for global-embedding configs."""
+        return packing.attention_block_names(self.config)
+
+    def attention_maps(self, x, context, extra_context=None, layers=None, queries=None, eps=None, eps_cif=None):
+        """The conditioners' cross-attention weights softmax(q k^T / 8) (reference models/perceiver.py:108-115) from the forward
+        pass `log_prob` runs -- what the reference's attention visualisation shows: which context points a target point's
+        conditioner attends to, layer by layer.
+
+        Arguments as `log_prob` (`context` is the embedding: `engine.embed(extract_0)`); `layers`: names from
+        `attention_layer_names` (None: all); `queries`: indices into the N points of x, any order, repeats allowed (None: all).
+        Returns (log_prob [B,N], {name: weights [B, n_query, Nc]}); log_prob is bitwise what `log_prob` returns with the same
+        eps, and the maps are views of one allocation."""
+        if self.is_global:
+            raise _lib.FlowCompareError("attention_maps: global-embedding configs attend to no context points")
+        names = self.attention_layer_names
+        first_slot = 0 if self.D > self.d_in else 1      # slot 0 is the augmenter's attention (absent for an identity augmenter)
+        if layers is None:
+            layers = names
+        unknown = [n for n in layers if n not in names]
+        if unknown or not layers:
+            raise _lib.FlowCompareError(f"attention_maps: unknown layer names {unknown}; choose from attention_layer_names"
+                                        if unknown else "attention_maps: no layers requested")
+        slots = sorted({names.index(n) + first_slot for n in layers})
+        with torch.cuda.device(self.device):
+            x = _f32c(x[..., :self.d_in], self.device)
+            B, N = x.shape[0], x.shape[1]
+            context, Nc, extra = self._prep_context(context, extra_context, B)
+            qidx, n_query = None, N
+            if queries is not None:
+                q = torch.as_tensor(queries).reshape(-1)
+                if q.numel() == 0 or q.is_floating_point() or int(q.min()) < 0 or int(q.max()) >= N:
+                    raise _lib.FlowCompareError(f"attention_maps: query indices must be integers in [0, {N})")
+                qidx = q.to(device=self.device, dtype=torch.int32).contiguous()
+                n_query = qidx.numel()
+            eps = self.draw_eps(B, N) if eps is None else _f32c(eps, self.device)
+            assert eps.shape == (B, N, self.D - self.d_in), eps.shape
+            eps_arg = eps if self.D > self.d_in else None
+            if self.cif_S:
+                eps_cif = self.draw_eps_cif(B, N) if eps_cif is None else _f32c(eps_cif, self.device)
+                assert eps_cif.shape == (self.L, B, N, self.cif_S), eps_cif.shape
+            else:
+                eps_cif = None
+            slots_host = np.asarray(slots, dtype=np.int32)
+            maps = torch.empty((len(slots), B, n_query, Nc), dtype=torch.float32, device=self.device)
+            out = torch.empty((B, N), dtype=torch.float32, device=self.device)
+            nbytes = self.lib.fc_flow_workspace_bytes(self._flow["handle"], B, N, Nc)
+            ws = self._workspace(nbytes)
+            rc = self.lib.fc_flow_attention_maps(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra), _ptr(eps_arg),
+                                                 _ptr(eps_cif), slots_host.ctypes.data, len(slots), _ptr(qidx), n_query,
+                                                 maps.data_ptr(), out.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
+            _lib.check(rc, "fc_flow_attention_maps")
+        return out, {names[s - first_slot]: maps[i] for i, s in enumerate(slots)}
+
     # ------------------------------------------------------------------ inverse / sampling pass
     def _ensure_inverse(self):
         if self._inv is None:

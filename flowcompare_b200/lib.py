@@ -47,6 +47,7 @@ SIGNATURES = {
     "fc_cross_attention_tc_scratch_bytes": (c_i64, [c_int, c_int]),
     "fc_cross_attention_tc": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, c_i64, c_vp]),
     "fc_cross_attention_tc_f16": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, c_i64, c_vp]),
+    "fc_attention_maps": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_f, c_vp]),
     "fc_fps_points": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_vp]),
     "fc_co_unit_sphere": (c_int, [c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp]),
     "fc_flow_create": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_i64, ctypes.POINTER(c_vp)]),
@@ -58,6 +59,8 @@ SIGNATURES = {
     "fc_rq_spline": (c_int, [c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_int, c_vp]),
     "fc_expm_action": (c_int, [c_vp, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp]),
     "fc_flow_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
+    "fc_flow_attention_maps": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_int, c_int, c_int,
+                                       c_vp, c_i64, c_int, c_vp]),
     "fc_flow_set_inverse": (c_int, [c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_i64]),
     "fc_flow_sample": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
     "fc_flow_sample_cif": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),

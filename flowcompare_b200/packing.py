@@ -252,6 +252,28 @@ def fold_inverse_actnorm_lu(flow_sd, config):
     return out
 
 
+def _coupling_prefix(cfg, layer):
+    """Module prefix of flow layer `layer`'s coupling block (its CIF block for CIF flows) in the transform list of reference
+    model_initialization.py:134-152: transforms.0 is the augmenter, then per layer the block, [ActNorm], permuter."""
+    stride = 1 + (1 if cfg["act_norm"] else 0) + 1
+    return f"transforms.{1 + layer * stride}"
+
+
+def attention_block_names(config):
+    """Module names of the attention blocks the flow's conditioners run over the context points, in transform order -- the
+    order of the capture slots of fc_flow_attention_maps, which number the augmenter's attention 0 and layer l's l + 1 (an
+    identity augmenter has none, so the list then starts at slot 1).  Empty for global-embedding flows."""
+    cfg = derive(config)
+    if cfg["global"]:
+        return []
+    cif = cfg["latent_dim"] < cfg["cif_latent_dim"]
+    names = ["transforms.0.attn"] if cfg["latent_dim"] > cfg["input_dim"] else []
+    for layer in range(cfg["n_flow_layers"]):
+        p = _coupling_prefix(cfg, layer)
+        names.append(f"{p}.flow.pre_conditioner.attn" if cif else f"{p}.pre_conditioner.attn")
+    return names
+
+
 INV_MAGIC = 0x46435F49
 
 
@@ -264,10 +286,9 @@ def pack_flow_inverse(flow_sd, config, tc_format="tf32"):
     D, L = cfg["latent_dim"], cfg["n_flow_layers"]
     cif = D < cfg["cif_latent_dim"]
     pairs = fold_inverse_actnorm_lu(flow_sd, config)
-    stride = 1 + (1 if cfg["act_norm"] else 0) + 1      # transforms per layer: block, [ActNorm], permuter
     for layer in range(L):
         if cif:
-            p = f"transforms.{1 + layer * stride}"
+            p = _coupling_prefix(cfg, layer)
             shift, log_scale = _d(flow_sd, f"{p}.act_norm.shift")[0], _d(flow_sd, f"{p}.act_norm.log_scale")[0]
             sc = torch.exp(-log_scale).flip(0)
             bi = -shift.flip(0) * sc
@@ -414,7 +435,7 @@ def pack_flow(flow_sd, config, tc_format="tf32"):
     hid = n_hid = pre_hid = n_pre = 0
     cif_hid = n_cif = affcif_hid = n_affcif = 0
     for layer in range(L):
-        p = f"transforms.{t}"
+        p = _coupling_prefix(cfg, layer)
         if cif:
             cif_hid, n_cif, affcif_hid, n_affcif, ldj_cif = _pack_cif(ar, flow_sd, p, cfg)
             ldj_const += ldj_cif

@@ -176,6 +176,14 @@ FC_API int fc_cross_attention_tc_f16(const float* q, int ldq, const float* kv, i
                               int B, int N, int Nc, int d, float scale, void* scratch, int64_t scratch_bytes,
                               fc_stream_t stream);
 
+/* The softmax weights of the same product, P = softmax(q k^T * scale) over the keys, written out (the flash kernels above never
+ * form them): out [B, n_query, Nc], out[b, r, j] for query row query_idx[r] of cloud b (q row b*N + query_idx[r]; query_idx a
+ * device int32 list, the same for every cloud, or NULL for all N rows with n_query == N).  Exact fp32: the dot product is a
+ * sequential fma chain over the d = 64 dimensions, so every weight is deterministic and independent of the batch and of the
+ * query list.  The kernel fc_flow_attention_maps runs per captured block.                                              */
+FC_API int fc_attention_maps(const float* q, int ldq, const float* kv, int ldkv, const int32_t* query_idx, int n_query,
+                      float* out, int B, int N, int Nc, float scale, fc_stream_t stream);
+
 /* ------------------------------------------------------------------ data-side ops ----------
  * What the reference's loader does between reading a voxel and calling `inner_loop` (SURVEY.md 8f rank 4).
  * fc_fps_points replaces `voxel[fps(voxel, batch, ratio=n_samples/len(voxel), random_start=False)][:n_samples]`
@@ -246,6 +254,21 @@ FC_API int fc_expm_action(const float* params, int ldp, float* x, int ldx, int n
 FC_API int fc_flow_forward(const fc_flow* h, const float* x, const float* context, const float* extra,
                     const float* eps, float* log_prob_out, float* z_out, int B, int N, int Nc,
                     void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream);
+
+/* The same forward pass, additionally writing the cross-attention weights of chosen attention blocks: the
+ * softmax(q k^T * 64^-1/2) over the context points of reference models/perceiver.py:108-115, which the flash kernels never form.
+ * Slot 0 is the augmenter's attention (transforms.0.attn), slot l+1 coupling layer l's pre-conditioner attention.
+ *   slots_host [n_slots]: HOST array, strictly increasing, each in [0, n_flow_layers]; query_idx [n_query]: device int32 rows of
+ *   x (the same for every cloud, repeats allowed, each in [0, N): the caller's contract) or NULL for all N rows (n_query == N);
+ *   maps_out [n_slots, B, n_query, Nc]: maps_out[i, b, r, j] = weight of context point j for query row query_idx[r] of cloud b in
+ *   block slots_host[i]; rows sum to 1.  The rest as fc_flow_log_prob_cif (eps_cif NULL for flows without CIF blocks);
+ *   log_prob_out is bitwise what fc_flow_log_prob returns.  fc_flow_workspace_bytes(h, B, N, Nc) sizes the workspace.
+ * FC_ERR_INVALID_ARG for slot 0 of a flow with an identity augmenter, unsorted or out-of-range slots, or query_idx == NULL with
+ * n_query != N; FC_ERR_UNSUPPORTED for global-embedding flows (their conditioners attend to no context points).          */
+FC_API int fc_flow_attention_maps(const fc_flow* h, const float* x, const float* context, const float* extra, const float* eps,
+                           const float* eps_cif, const int32_t* slots_host, int n_slots, const int32_t* query_idx, int n_query,
+                           float* maps_out, float* log_prob_out, int B, int N, int Nc, void* workspace,
+                           int64_t workspace_bytes, int precision, fc_stream_t stream);
 
 /* Inverse / sampling pass: fc_flow_sample replaces `Flow.sample` after its base draw (reference models/transform.py:79-84,
  * called by `make_sample`, model_initialization.py:231-245): the transforms walked backwards with each `.inverse`
