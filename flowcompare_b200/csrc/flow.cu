@@ -89,11 +89,12 @@ __global__ void build_cb_input_kernel(const float* __restrict__ extra, const flo
     out[i] = v;
 }
 
-// log_prob[row] = sum(augment partials) + sum(coupling partials) + const + sum_d(-0.5 z_d^2 - 0.5 log 2pi)
-// (reference models/distributions.py:192-195 for the base density).  One warp per row.
+// log_prob = sum(augment partials) + sum(coupling partials) + const + sum_d(-0.5 z_d^2 - 0.5 log 2pi)
+// (reference models/distributions.py:192-195 for the base density).  One warp per row.  K > 1: rows are in the K-draw
+// layout (b*K + k)*N + n and the value goes to log_prob[k][b][n] (draw-major); K == 1: to log_prob[row].
 __global__ void finalize_kernel(const float* __restrict__ z, int ldz, int D, const float* __restrict__ apart,
                                 int n_apart, const float* __restrict__ cpart, int n_cpart, int M, float ldj_const,
-                                float* __restrict__ log_prob) {
+                                float* __restrict__ log_prob, int N, int K) {
     const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (row >= M) return;
@@ -105,7 +106,8 @@ __global__ void finalize_kernel(const float* __restrict__ z, int ldz, int D, con
         float acc = 0.f;
         for (int i = 0; i < n_apart; ++i) acc += apart[(size_t)i * M + row];
         for (int i = 0; i < n_cpart; ++i) acc += cpart[(size_t)i * M + row];
-        log_prob[row] = (acc + ldj_const) + s;
+        const int out = K == 1 ? row : ((row / N) % K) * (M / K) + (row / (K * N)) * N + row % N;
+        log_prob[out] = (acc + ldj_const) + s;
     }
 }
 
@@ -415,25 +417,35 @@ static int run_cif_block(const fc_flow* f, const FcFlowLayer& y, float* lat, Flo
     return FC_OK;
 }
 
+// draws > 0: the K-draw pass of fc_flow_log_prob_draws.  The augmenter's network depends on (x, c) only, so it runs once over
+// the B*N points with x staged in lat1; its output GEMM then runs once per draw (eps + k*B*N*S) into that staging latent and
+// staging log-det slabs, and fc_launch_scatter_draw moves the result to rows (b*K + k)*N + n of lat0 / apart.  Every later
+// layer runs unchanged on K*N points per cloud.  Each launch a row goes through is the launch log_prob makes for it, so draw k
+// is bitwise fc_flow_log_prob with eps + k*B*N*S.  eps_cif is then [L, B, K, N, S]; log_prob_out [K, B, N].
 static int flow_forward(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
                         const float* eps_cif, float* log_prob_out, float* z_out, int B, int N, int Nc, void* workspace,
-                        int64_t workspace_bytes, int precision, fc_stream_t stream_, const FcCapture* cap = nullptr) {
-    FC_REQUIRE(f && x && context && log_prob_out && B > 0 && N > 0 && Nc > 0);
+                        int64_t workspace_bytes, int precision, fc_stream_t stream_, const FcCapture* cap = nullptr,
+                        int draws = 0) {
+    FC_REQUIRE(f && x && context && log_prob_out && B > 0 && N > 0 && Nc > 0 && draws >= 0);
     FC_REQUIRE(eps || !f->has_aug);
     FC_REQUIRE(eps_cif || !f->cif_dim);
     FC_REQUIRE((f->extra != 0) == (extra != nullptr));
-    FC_REQUIRE((int64_t)B * N < (1ll << 31) && (int64_t)B * Nc < (1ll << 31));
+    FC_REQUIRE(!draws || (!cap && !z_out));
+    const int K = draws ? draws : 1;
+    FC_REQUIRE((int64_t)B * N * K < (1ll << 31) && (int64_t)B * Nc < (1ll << 31));
     cudaStream_t s = (cudaStream_t)stream_;
     if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return FC_ERR_WORKSPACE;
-    FlowWs w = carve_flow_ws(f, B, N, Nc, workspace);
+    FlowWs w = carve_flow_ws(f, B, K * N, Nc, workspace);
     if (w.total_bytes > workspace_bytes) return FC_ERR_WORKSPACE;
-    const int M = B * N;
+    const int NK = K * N;            // points per cloud after the augmenter
+    const int M = B * NK, M0 = B * N;
+    float* xin = draws ? w.lat1 : w.lat0;     // the latent the augmenter reads x from and writes its draw into
     int rc;
 
     // x -> latent columns [0, d_in)
     {
-        const long long tot = (long long)M * f->d_in;
-        copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(x, f->d_in, w.lat0, w.ldx, M, f->d_in);
+        const long long tot = (long long)M0 * f->d_in;
+        copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(x, f->d_in, xin, w.ldx, M0, f->d_in);
         fc_count_launch();
         FC_LAUNCH_OK();
     }
@@ -460,22 +472,41 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
 
     // ---- transforms.0: augment (reference models/augmenter.py:15-19, :49-63); latent_dim == input_dim: IdentityTransform
     if (f->has_aug && !f->is_global) {
-        rc = run_attention_block(f, f->augpre, f->augattn, w.lat0, w.ldx, f->d_in, context, B, N, Nc, w, precision, s,
+        rc = run_attention_block(f, f->augpre, f->augattn, xin, w.ldx, f->d_in, context, B, N, Nc, w, precision, s,
                                  maps_for(0), cap);
         if (rc) return rc;
     }
     if (f->has_aug) {
-        FcMlpIn in{w.lat0, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(0), w.cb_ld, N};
+        FcMlpIn in{xin, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(0), w.cb_ld, N};
         if (!f->has_cb) { in.bias = nullptr; in.bias_ld = 0; in.bias_group = 0; }
         float* last = nullptr;
-        rc = fc_run_mlp_hidden(f->aug, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
+        rc = fc_run_mlp_hidden(f->aug, in, M0, w.hA, w.hB, w.ldh, precision, s, &last);
         if (rc) return rc;
         GemmArgs g = fc_gemm_args_zero();
         g.A1 = last; g.lda1 = w.ldh; g.K1 = f->aug_hid; g.Wt = f->aug.out.w; g.ldw = f->aug.out.ldw; g.bias = f->aug.out.b; g.Whi = f->aug.out.whi; g.Wlo = f->aug.out.wlo; g.ldk = f->aug.out.ldk; g.tc_fmt = f->aug.out.tc_fmt;
-        g.M = M; g.N = f->aug.out.N; g.epi = FC_EPI_AUGMENT; g.x = w.lat0; g.ldx = w.ldx; g.col0 = f->d_in;
+        g.M = M0; g.N = f->aug.out.N; g.epi = FC_EPI_AUGMENT; g.x = xin; g.ldx = w.ldx; g.col0 = f->d_in;
         g.part = w.apart; g.eps = eps; g.ld_eps = f->D - f->d_in; g.precision = precision;
-        rc = fc_launch_gemm(g, s);
-        if (rc) return rc;
+        if (!draws) {
+            rc = fc_launch_gemm(g, s);
+            if (rc) return rc;
+        } else {
+            // staging slabs in the hidden buffer the output GEMM does not read; slabs the GEMM path leaves alone stay zero
+            float* spart = last == w.hA ? w.hB : w.hA;
+            FC_CUDA_OK(cudaMemsetAsync(spart, 0, (size_t)M0 * w.n_apart * sizeof(float), s));
+            g.part = spart;
+            for (int k = 0; k < K; ++k) {
+                g.eps = eps + (size_t)k * M0 * (f->D - f->d_in);
+                rc = fc_launch_gemm(g, s);
+                if (rc) return rc;
+                rc = fc_launch_scatter_draw(xin, w.ldx, f->D, spart, w.n_apart, w.lat0, w.ldx, w.apart, B, N, K, k, s);
+                if (rc) return rc;
+            }
+        }
+    } else if (draws) {
+        for (int k = 0; k < K; ++k) {    // identity augmenter (a CIF flow): the K copies of x
+            rc = fc_launch_scatter_draw(xin, w.ldx, f->D, nullptr, 0, w.lat0, w.ldx, nullptr, B, N, K, k, s);
+            if (rc) return rc;
+        }
     }
 
     // ---- coupling layers
@@ -487,11 +518,11 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
             if (rc) return rc;
         }
         if (!f->is_global) {
-            rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, f->half, context, B, N, Nc, w, precision, s,
+            rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, f->half, context, B, NK, Nc, w, precision, s,
                                      maps_for(l + 1), cap);
             if (rc) return rc;
         }
-        FcMlpIn in{lat, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(l + 1), w.cb_ld, N};
+        FcMlpIn in{lat, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(l + 1), w.cb_ld, NK};
         if (!f->has_cb) { in.bias = nullptr; in.bias_ld = 0; in.bias_group = 0; }
         float* last = nullptr;
         rc = fc_run_mlp_hidden(y.cpl, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
@@ -536,7 +567,7 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
     {
         const int wpb = 8;
         finalize_kernel<<<(M + wpb - 1) / wpb, wpb * 32, 0, s>>>(lat, w.ldx, f->D, w.apart, w.n_apart, w.cpart, w.n_cpart,
-                                                                 M, (float)f->ldj_const, log_prob_out);
+                                                                 M, (float)f->ldj_const, log_prob_out, N, K);
         fc_count_launch();
         FC_LAUNCH_OK();
     }
@@ -561,6 +592,38 @@ extern "C" int fc_flow_log_prob_cif(const fc_flow* f, const float* x, const floa
                                     const float* eps, const float* eps_cif, float* log_prob_out, int B, int N, int Nc,
                                     void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream_) {
     return flow_forward(f, x, context, extra, eps, eps_cif, log_prob_out, nullptr, B, N, Nc, workspace, workspace_bytes, precision, stream_);
+}
+
+// No stochastic transform (identity augmenter, no CIF block): every draw is the same log_prob, computed once.
+static bool flow_is_deterministic(const fc_flow* f) { return !f->has_aug && !f->cif_dim; }
+
+extern "C" int64_t fc_flow_log_prob_draws_workspace_bytes(const fc_flow* f, int B, int N, int Nc, int K) {
+    if (!f || B <= 0 || N <= 0 || Nc <= 0 || K <= 0) return FC_ERR_INVALID_ARG;
+    if (flow_is_deterministic(f)) K = 1;
+    if ((int64_t)K * B * N > FC_DRAWS_MAX_ROWS) return FC_ERR_INVALID_ARG;
+    return carve_flow_ws(f, B, K * N, Nc, nullptr).total_bytes;
+}
+
+// K augmentation draws of every point in one pass (flow_forward with draws = K): lp_draws_out[k] is bitwise what
+// fc_flow_log_prob(_cif) returns with eps + k*B*N*S (and draw k's CIF noise).
+extern "C" int fc_flow_log_prob_draws(const fc_flow* f, const float* x, const float* context, const float* extra,
+                                      const float* eps, const float* eps_cif, int K, float* lp_draws_out, int B, int N, int Nc,
+                                      void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream_) {
+    FC_REQUIRE(f && K > 0 && B > 0 && N > 0 && lp_draws_out);
+    if (flow_is_deterministic(f)) {
+        FC_REQUIRE((int64_t)B * N <= FC_DRAWS_MAX_ROWS);
+        const int rc = flow_forward(f, x, context, extra, eps, nullptr, lp_draws_out, nullptr, B, N, Nc, workspace,
+                                    workspace_bytes, precision, stream_);
+        if (rc) return rc;
+        const size_t bytes = (size_t)B * N * sizeof(float);
+        for (int k = 1; k < K; ++k)
+            FC_CUDA_OK(cudaMemcpyAsync(lp_draws_out + (size_t)k * B * N, lp_draws_out, bytes, cudaMemcpyDeviceToDevice,
+                                       (cudaStream_t)stream_));
+        return FC_OK;
+    }
+    FC_REQUIRE((int64_t)K * B * N <= FC_DRAWS_MAX_ROWS);
+    return flow_forward(f, x, context, extra, eps, eps_cif, lp_draws_out, nullptr, B, N, Nc, workspace, workspace_bytes, precision,
+                        stream_, nullptr, K);
 }
 
 // The forward pass that also writes the softmax weights of the attention blocks listed in slots_host (see FcCapture).

@@ -157,6 +157,12 @@ int fc_launch_expm_action(const float* params, int ldp, float* lat, int ldx, int
                           float* part, long long row0, int rows, int inverse, cudaStream_t s);
 int fc_expm_max_n();
 
+// K-draw forward (iw.cu): copies draw k's staged latent columns [0, cols) and log-det slabs, rows b*N + n, to rows
+// (b*K + k)*N + n of the K-draw layout
+int fc_launch_scatter_draw(const float* src, int lds, int cols, const float* part_src, int n_part, float* dst, int ldd,
+                           float* part_dst, int B, int N, int K, int k, cudaStream_t s);
+constexpr int64_t FC_DRAWS_MAX_ROWS = 1ll << 20;   // rows of one fc_flow_log_prob_draws pass
+
 // runs in/hidden layers of an MLP; returns the buffer holding the last hidden activation.
 // bufA/bufB: [M][ldh] scratch (ldh >= hidden width).  `in_bias`/group override the in-layer bias.
 struct FcMlpIn {

@@ -36,6 +36,15 @@ def _f32c(t, device):
     return t.to(device=device, dtype=torch.float32).contiguous()
 
 
+IW_MAX_PASS_ROWS = 1 << 20      # rows (draws x points) of one fc_flow_log_prob_draws pass
+
+
+def _n_draws(n, what):
+    if isinstance(n, bool) or not isinstance(n, (int, np.integer)) or n < 1:
+        raise _lib.FlowCompareError(f"{what}: the number of draws must be a positive int, got {n!r}")
+    return int(n)
+
+
 class FlowCompareB200:
     """Per-point conditional log-likelihood engine (eval mode only).
 
@@ -191,6 +200,87 @@ class FlowCompareB200:
                                                _ptr(eps_arg), out.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
                 _lib.check(rc, "fc_flow_log_prob")
         return out
+
+    def log_prob_iw(self, x, context, extra_context=None, n_draws=8, eps=None, eps_cif=None, return_draws=False,
+                    draws_per_pass=None, workspace_budget=None):
+        """Importance-weighted log p(x | context) over `n_draws` augmentation draws:
+        IW_K = log((1/K) sum_k exp(lp_k)), lp_k = `log_prob(x, context, eps=eps[k])`.
+
+        `log_prob` is a single-sample estimate: the augmenter's noise dims (and every CIF block's) are drawn from q(e | x, c), so
+        exp(lp_k) is an unbiased estimate of p(x | c) and lp_k itself is noisy.  IW_K is never below the mean of its draws and
+        approaches log p(x | c) as K grows; K = 1 is exactly the reference's `Flow.log_prob`.
+        Arguments as `log_prob` (`context` is the embedding); eps [K,B,N,latent-input_dim] and eps_cif
+        [K,L,B,N,cif_latent_dim-latent_dim] (CIF flows) optional, drawn on the device by default.  The draws run in passes of at
+        most 2^20 rows (K_pass*B*N), fewer with `draws_per_pass` or when a pass's workspace would exceed `workspace_budget`
+        bytes; the result does not depend on the split.  Returns IW [B,N], or (IW, draws [K,B,N]) with `return_draws`:
+        draws[k] is bitwise `log_prob(x, context, eps=eps[k], eps_cif=eps_cif[k])`."""
+        K = _n_draws(n_draws, "log_prob_iw")
+        if draws_per_pass is not None:
+            _n_draws(draws_per_pass, "log_prob_iw: draws_per_pass")
+        with torch.cuda.device(self.device):
+            x = _f32c(x[..., :self.d_in], self.device)
+            B, N = x.shape[0], x.shape[1]
+            context, Nc, extra = self._prep_context(context, extra_context, B)
+            S = self.D - self.d_in
+            if eps is not None:
+                eps = _f32c(eps, self.device)
+                if tuple(eps.shape) != (K, B, N, S):
+                    raise _lib.FlowCompareError(f"log_prob_iw: eps must be [{K}, {B}, {N}, {S}], got {list(eps.shape)}")
+            if eps_cif is not None:
+                if not self.cif_S:
+                    raise _lib.FlowCompareError("log_prob_iw: eps_cif given but this flow has no CIF blocks")
+                eps_cif = _f32c(eps_cif, self.device)
+                if tuple(eps_cif.shape) != (K, self.L, B, N, self.cif_S):
+                    raise _lib.FlowCompareError(f"log_prob_iw: eps_cif must be [{K}, {self.L}, {B}, {N}, {self.cif_S}], "
+                                                f"got {list(eps_cif.shape)}")
+            deterministic = S == 0 and not self.cif_S       # every draw is the same log_prob: one pass
+            if N > IW_MAX_PASS_ROWS:
+                raise _lib.FlowCompareError(f"log_prob_iw: {N} points per cloud exceed one pass of {IW_MAX_PASS_ROWS} rows")
+            h = self._flow["handle"]
+            wsb = lambda bc, kp: self.lib.fc_flow_log_prob_draws_workspace_bytes(h, bc, N, Nc, kp)
+            bc = min(B, IW_MAX_PASS_ROWS // N)                                  # clouds per pass
+            kp = K if deterministic else max(1, min(K, IW_MAX_PASS_ROWS // (bc * N)))   # draws per pass
+            if draws_per_pass is not None and not deterministic:
+                kp = min(kp, int(draws_per_pass))
+            if workspace_budget is not None:
+                while not deterministic and kp > 1 and wsb(bc, kp) > workspace_budget:
+                    kp -= 1
+                while bc > 1 and wsb(bc, kp) > workspace_budget:
+                    bc = (bc + 1) // 2
+            draws = torch.empty((K, B, N), dtype=torch.float32, device=self.device)
+            for b0 in range(0, B, bc):
+                b1 = min(B, b0 + bc)
+                nb = b1 - b0
+                for k0 in range(0, K, kp):
+                    k1 = min(K, k0 + kp)
+                    nk = k1 - k0
+                    pe = pc = None
+                    if S and not deterministic:
+                        if eps is None:
+                            pe = torch.empty((nk, nb, N, S), dtype=torch.float32, device=self.device)
+                            _lib.check(self.lib.fc_fill_normal(pe.data_ptr(), pe.numel(), self._next_seed(), 0, _stream()),
+                                       "fc_fill_normal")
+                        else:
+                            pe = eps[k0:k1, b0:b1].contiguous()
+                    if self.cif_S:
+                        if eps_cif is None:   # iid draws: the layout [L, B, K, N, S] the pass reads needs no permute
+                            pc = torch.empty((self.L, nb, nk, N, self.cif_S), dtype=torch.float32, device=self.device)
+                            _lib.check(self.lib.fc_fill_normal(pc.data_ptr(), pc.numel(), self._next_seed(), 1 << 40, _stream()),
+                                       "fc_fill_normal")
+                        else:
+                            pc = eps_cif[k0:k1, :, b0:b1].permute(1, 2, 0, 3, 4).contiguous()
+                    out = draws[k0:k1] if nb == B else torch.empty((nk, nb, N), dtype=torch.float32, device=self.device)
+                    nbytes = wsb(nb, nk)
+                    ws = self._workspace(nbytes)
+                    rc = self.lib.fc_flow_log_prob_draws(h, x[b0:b1].data_ptr(), context[b0:b1].data_ptr(),
+                                                         _ptr(None if extra is None else extra[b0:b1]), _ptr(pe), _ptr(pc), nk,
+                                                         out.data_ptr(), nb, N, Nc, ws, nbytes, self.precision, _stream())
+                    _lib.check(rc, "fc_flow_log_prob_draws")
+                    if nb != B:
+                        draws[k0:k1, b0:b1].copy_(out)
+            iw = torch.empty((B, N), dtype=torch.float32, device=self.device)
+            _lib.check(self.lib.fc_logmeanexp(draws.data_ptr(), K, B * N, iw.data_ptr(), _stream()), "fc_logmeanexp")
+        return (iw, draws) if return_draws else iw
 
     def _prep_context(self, context, extra_context, B):
         context = context.to(self.device)
@@ -423,7 +513,7 @@ class FlowCompareB200:
         return out_stats[0], out_log_prob, out_stats[1]
 
     # ------------------------------------------------------------------ consumers
-    def change_maps(self, batch_1_0, batch_0_0, batch_0_1, batch_1_1, multiple=3.0, hard_cutoff=None, eps=None):
+    def change_maps(self, batch_1_0, batch_0_0, batch_0_1, batch_1_1, multiple=3.0, hard_cutoff=None, eps=None, n_draws=1):
         """The four `inner_loop` passes + two `log_prob_to_change` calls of `DatasetViewer.view_index`
         (reference test_flow.py:39-62) as ONE batched pass: the four batches (1|0, 0|0, 0|1, 1|1; each
         (extract_0, extract_1, extra_context)) are stacked along the batch axis -- cloud pairs are independent and a
@@ -431,7 +521,11 @@ class FlowCompareB200:
         formed per direction exactly as the reference does.  eps: optional [4B, N, latent-input_dim] noise.
         Returns a dict of CUDA tensors: log_prob_{1_0,0_0,0_1,1_1} [B,N], change_1_0, change_0_1 [B,N], loss_{1_0,...}
         (= -mean log_prob, `inner_loop`'s first return) and nats_{1_0,...} (= loss * log2(e) / input_dim, its third return, which
-        the reference's evaluation prints as "nats", test_flow.py:160,224)."""
+        the reference's evaluation prints as "nats", test_flow.py:160,224).
+        n_draws > 1: every log_prob is `log_prob_iw` over that many augmentation draws (the same stacked batches; eps
+        [n_draws, 4B, N, latent-input_dim]), so the change masks and loss / nats are those of the importance-weighted estimate.
+        n_draws = 1 is the reference's single-draw estimator and runs the path above unchanged."""
+        K = _n_draws(n_draws, "change_maps")
         batches = (batch_1_0, batch_0_0, batch_0_1, batch_1_1)
         B = batches[0][0].shape[0]
         for b in batches:
@@ -454,10 +548,13 @@ class FlowCompareB200:
             else:
                 slot.append(len(uniq))
                 uniq.append(b[0])
-        if len(uniq) < 4 and not self.cif_S and self.D > self.d_in:
+        if K > 1 or (len(uniq) < 4 and not self.cif_S and self.D > self.d_in):
             emb = self.embed(torch.cat([u[:, :, :self.d_in].to(self.device, torch.float32) for u in uniq], dim=0))
             ctx = torch.cat([emb[j * B:(j + 1) * B] for j in slot], dim=0)
-            lp = self.log_prob(e1, ctx, extra_context=extra, eps=eps)
+            if K > 1:
+                lp = self.log_prob_iw(e1, ctx, extra_context=extra, n_draws=K, eps=eps)
+            else:
+                lp = self.log_prob(e1, ctx, extra_context=extra, eps=eps)
         else:
             _, lp, _ = self.inner_loop((e0, e1, extra), eps=eps)
         names = ("1_0", "0_0", "0_1", "1_1")
@@ -470,13 +567,17 @@ class FlowCompareB200:
         out["change_0_1"] = log_prob_to_change(out["log_prob_0_1"], out["log_prob_1_1"], multiple, hard_cutoff)
         return out
 
-    def evaluate_on_batches(self, batches, multiple=5.4, hard_cutoff=None, eps=None):
+    def evaluate_on_batches(self, batches, multiple=5.4, hard_cutoff=None, eps=None, n_draws=1):
         """The evaluation loop of `evaluate_on_test` (reference test_flow.py:147-226) over an iterable of
         `(batch_1_0, batch_0_0)` pairs, each batch `(extract_0, extract_1, extra_context)` as the reference assembles them
         (test_flow.py:155-158): the two passes run as ONE stacked pass, then `log_prob_to_change(lp_1_0, lp_0_0, multiple)`,
         the per-cloud change means `(change > 0).float().mean(-1)` (:172) and the running average of the 1|0 pass's nats
         (:224-226).  eps: optional iterable of [2B, N, latent-input_dim] noise per batch (1|0 rows first).
-        Returns `(nats_avg, change_mean_list)` as Python floats, like the reference."""
+        Returns `(nats_avg, change_mean_list)` as Python floats, like the reference.
+        n_draws > 1: the log-probs are `log_prob_iw` over that many augmentation draws (eps per batch [n_draws, 2B, N,
+        latent-input_dim]), so the change means and nats are those of the importance-weighted estimate; n_draws = 1 is the
+        reference's single-draw estimator and runs the path above unchanged."""
+        K = _n_draws(n_draws, "evaluate_on_batches")
         nats_avg, change_mean_list = 0.0, []
         eps_it = iter(eps) if eps is not None else None
         for batch_ind, (b10, b00) in enumerate(batches):
@@ -488,7 +589,11 @@ class FlowCompareB200:
                 if b10[2] is None or b00[2] is None:
                     raise _lib.FlowCompareError("this config uses extra context but a batch has none")
                 extra = torch.cat([b[2].reshape(-1).to(self.device, torch.float32) for b in (b10, b00)], dim=0)
-            _, lp, _ = self.inner_loop((e0, e1, extra), eps=None if eps_it is None else next(eps_it))
+            eps_b = None if eps_it is None else next(eps_it)
+            if K > 1:
+                lp = self.log_prob_iw(e1, self.embed(e0), extra_context=extra, n_draws=K, eps=eps_b)
+            else:
+                _, lp, _ = self.inner_loop((e0, e1, extra), eps=eps_b)
             lp10, lp00 = lp[:B], lp[B:]
             change = log_prob_to_change(lp10, lp00, multiple, hard_cutoff)
             change_mean_list.extend((change > 0).float().mean(dim=-1).tolist())

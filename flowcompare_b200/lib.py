@@ -56,6 +56,10 @@ SIGNATURES = {
     "fc_flow_log_prob": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
     "fc_flow_log_prob_cif": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
     "fc_flow_cif_noise_dim": (c_int, [c_vp]),
+    "fc_flow_log_prob_draws_workspace_bytes": (c_i64, [c_vp, c_int, c_int, c_int, c_int]),
+    "fc_flow_log_prob_draws": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int,
+                                       c_vp]),
+    "fc_logmeanexp": (c_int, [c_vp, c_int, c_i64, c_vp, c_vp]),
     "fc_rq_spline": (c_int, [c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_vp, c_int, c_vp]),
     "fc_expm_action": (c_int, [c_vp, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_int, c_vp]),
     "fc_flow_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),

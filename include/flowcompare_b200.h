@@ -234,6 +234,29 @@ FC_API int fc_flow_log_prob_cif(const fc_flow* h, const float* x, const float* c
                          void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream);
 FC_API int fc_flow_cif_noise_dim(const fc_flow* h);
 
+/* Multi-draw log-likelihood.  A log-prob is a single-sample estimate of log p(x | c): the augmenter's noise dims are drawn from
+ * q(e | x, c) (reference models/augmenter.py:49-63) and every CIF block draws again.  fc_flow_log_prob_draws scores K draws per
+ * point in one pass: the augmenter's network runs once per point, only its output layer once per draw, and the coupling layers
+ * see K*N points per cloud (the context's to_kv runs once per layer per cloud, not per draw).
+ *   eps [K, B, N, latent-input_dim] (NULL for an identity augmenter); eps_cif [L, B, K, N, fc_flow_cif_noise_dim(h)] (draw k of
+ *   cloud b at eps_cif[l][b][k]; NULL for flows without CIF blocks); lp_draws_out [K, B, N].  The rest as fc_flow_log_prob_cif.
+ *   lp_draws_out[k] is bitwise what fc_flow_log_prob / fc_flow_log_prob_cif return for eps[k] and draw k's eps_cif.
+ * One pass runs at most 2^20 rows: K*B*N <= 2^20 (B*N for a flow with no stochastic transform -- identity augmenter and no
+ * CIF block -- which is evaluated once and its log-prob copied to the K slots), else FC_ERR_INVALID_ARG; callers split the
+ * draws over several passes.  fc_flow_log_prob_draws_workspace_bytes(h, B, N, Nc, K) sizes the workspace (FC_ERR_WORKSPACE if
+ * it is smaller).                                                                                                          */
+FC_API int64_t fc_flow_log_prob_draws_workspace_bytes(const fc_flow* h, int B, int N, int Nc, int K);
+FC_API int fc_flow_log_prob_draws(const fc_flow* h, const float* x, const float* context, const float* extra,
+                           const float* eps, const float* eps_cif, int K, float* lp_draws_out, int B, int N, int Nc,
+                           void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream);
+
+/* The importance-weighted estimate over the leading axis: out[i] = log((1/K) sum_k exp(draws[k][i])) for draws [K, M], as
+ * m + (log(sum_k exp(draws[k][i] - m)) - log K), m = max_k draws[k][i], in fp32 with the draws folded in index order -- so the
+ * result depends on the point's K values only, not on M or on how the draws were split over passes.  Any NaN draw gives NaN,
+ * any +inf draw +inf; -inf draws drop out of the sum, all -inf gives -inf.  K equal finite draws give that value exactly.
+ * A caller that splits the draws over several fc_flow_log_prob_draws passes reduces once at the end.                     */
+FC_API int fc_logmeanexp(const float* draws, int K, int64_t M, float* out, fc_stream_t stream);
+
 /* Op-level entry points of the two couplings' elementwise tails (the conditioner MLP is a chain of fc_gemm calls).
  * fc_rq_spline replaces `unconstrained_rational_quadratic_spline(inputs, unnormalized_widths, unnormalized_heights,
  * unnormalized_derivatives, inverse)` (reference models/spline_coupling.py:24-66 over :69-169; 'linear' tails, tail bound 3,
