@@ -255,6 +255,7 @@ extern "C" int fc_flow_create(const int32_t* header, int n_header, const int64_t
 extern "C" void fc_flow_destroy(fc_flow* f) {
     if (!f) return;
     delete[] f->layers;
+    delete[] f->glayers;
     delete f;
 }
 
@@ -325,6 +326,9 @@ extern "C" int64_t fc_flow_workspace_bytes(const fc_flow* f, int B, int N, int N
 // out + i * B * n_query * Nc.
 struct FcCapture { const int32_t* slots; int n_slots; const int32_t* qidx; int n_query; float* out; };
 
+static int run_attention_core(const fc_flow* f, const FcAttn& at, const float* h4, int ldh4, const float* context, int B, int N,
+                              int Nc, FlowWs& w, int precision, cudaStream_t s, float* maps, const FcCapture* cap);
+
 // maps: where this block's weights go (nullptr: not captured; `cap` then unused)
 static int run_attention_block(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const float* lat, int ldx, int K_in,
                                const float* context, int B, int N, int Nc, FlowWs& w, int precision, cudaStream_t s,
@@ -338,11 +342,19 @@ static int run_attention_block(const fc_flow* f, const FcMlp& pre, const FcAttn&
     float* h4 = (last == w.hA) ? w.hB : w.hA;
     rc = gemm_plain(pre.out, last, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, h4, w.ldh, M, precision, s);
     if (rc) return rc;
-    rc = fc_launch_ln_stats(h4, w.ldh, M, f->attn_in, 1e-5f, w.mu, w.rstd, s);
+    return run_attention_core(f, at, h4, w.ldh, context, B, N, Nc, w, precision, s, maps, cap);
+}
+
+// LayerNorm statistics, to_q, to_kv and the attention of one block, from its pre-attention MLP's output h4 [M][ldh4]: w.o
+// (and w.q, w.mu, w.rstd) afterwards
+static int run_attention_core(const fc_flow* f, const FcAttn& at, const float* h4, int ldh4, const float* context, int B, int N,
+                              int Nc, FlowWs& w, int precision, cudaStream_t s, float* maps, const FcCapture* cap) {
+    const int M = B * N;
+    int rc = fc_launch_ln_stats(h4, ldh4, M, f->attn_in, 1e-5f, w.mu, w.rstd, s);
     if (rc) return rc;
     {
         GemmArgs g = fc_gemm_args_zero();
-        g.A1 = h4; g.lda1 = w.ldh; g.K1 = f->attn_in; g.Wt = at.q.w; g.ldw = at.q.ldw; g.bias = at.qbias; g.Whi = at.q.whi; g.Wlo = at.q.wlo; g.ldk = at.q.ldk; g.tc_fmt = at.q.tc_fmt;
+        g.A1 = h4; g.lda1 = ldh4; g.K1 = f->attn_in; g.Wt = at.q.w; g.ldw = at.q.ldw; g.bias = at.qbias; g.Whi = at.q.whi; g.Wlo = at.q.wlo; g.ldk = at.q.ldk; g.tc_fmt = at.q.tc_fmt;
         g.C = w.q; g.ldc = 64; g.M = M; g.N = f->inner; g.epi = FC_EPI_LNQ; g.row_mu = w.mu; g.row_rstd = w.rstd;
         g.csum = at.csum; g.precision = precision;
         rc = fc_launch_gemm(g, s);
@@ -425,8 +437,9 @@ static int run_cif_block(const fc_flow* f, const FcFlowLayer& y, float* lat, Flo
 static int flow_forward(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
                         const float* eps_cif, float* log_prob_out, float* z_out, int B, int N, int Nc, void* workspace,
                         int64_t workspace_bytes, int precision, fc_stream_t stream_, const FcCapture* cap = nullptr,
-                        int draws = 0) {
+                        int draws = 0, float* ckpt = nullptr) {
     FC_REQUIRE(f && x && context && log_prob_out && B > 0 && N > 0 && Nc > 0 && draws >= 0);
+    FC_REQUIRE(!ckpt || !draws);
     FC_REQUIRE(eps || !f->has_aug);
     FC_REQUIRE(eps_cif || !f->cif_dim);
     FC_REQUIRE((f->extra != 0) == (extra != nullptr));
@@ -511,8 +524,17 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
 
     // ---- coupling layers
     float* lat = w.lat0; float* lat_next = w.lat1;
+    // ckpt (input-gradient pass): the latent at the input of layer l into slot l of [L+1][M][ldx], the final latent into slot L --
+    // copied before the coupling updates x2 in place; the forward's own launches are unchanged
+    auto checkpoint = [&](int slot) -> int {
+        if (ckpt)
+            FC_CUDA_OK(cudaMemcpyAsync(ckpt + (size_t)slot * M * w.ldx, lat, (size_t)M * w.ldx * sizeof(float),
+                                       cudaMemcpyDeviceToDevice, s));
+        return FC_OK;
+    };
     for (int l = 0; l < f->L; ++l) {
         const FcFlowLayer& y = f->layers[l];
+        if ((rc = checkpoint(l))) return rc;
         if (f->cif_dim) {
             rc = run_cif_block(f, y, lat, w, M, eps_cif + (size_t)l * M * (f->cif_dim - f->D), precision, s);
             if (rc) return rc;
@@ -564,6 +586,7 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
             float* t = lat; lat = lat_next; lat_next = t;
         }
     }
+    if ((rc = checkpoint(f->L))) return rc;
     {
         const int wpb = 8;
         finalize_kernel<<<(M + wpb - 1) / wpb, wpb * 32, 0, s>>>(lat, w.ldx, f->D, w.apart, w.n_apart, w.cpart, w.n_cpart,
@@ -804,4 +827,269 @@ extern "C" int fc_flow_sample_cif(const fc_flow* f, const float* z, const float*
                                   const float* eps_cif, float* x_out, int B, int P, int Nc, void* workspace,
                                   int64_t workspace_bytes, int precision, fc_stream_t stream_) {
     return flow_sample(f, z, context, extra, eps_cif, x_out, B, P, Nc, workspace, workspace_bytes, precision, stream_);
+}
+
+// ------------------------------------------------------------------------------------------ input-gradient pass
+// d log_prob / d x of `Flow.log_prob` (reference models/transform.py:70-76) with eps held fixed, for affine-coupling flows.
+// The forward pass runs unchanged and copies the latent at the input of every coupling layer into a checkpoint slab; the layers
+// are then walked backwards: each one's forward is recomputed from its checkpoint with the intermediates its backward needs
+// (pre-activations, the LayerNorm input and statistics, q, the attention output, the raw coupling outputs), then its backward
+// runs.  Every backward contraction is a GEMM on the transposed weights fc_flow_set_grad attaches; the rest is flow_grad.cu.
+static FcMlpT read_mlp_t(FcCursor& c, int K_x, bool has_o, int hid, int n_hidden, int N_out) {
+    FcMlpT t;
+    if (n_hidden > FC_MAX_HIDDEN) { c.ok = false; return t; }
+    t.in_x = c.linear(hid, 0, K_x, false);
+    if (has_o) t.in_o = c.linear(hid, 0, 64, false);
+    for (int i = 0; i < n_hidden; ++i) t.hidden[i] = c.linear(hid, 0, hid, false);
+    t.out = c.linear(N_out, 0, hid, false);
+    return t;
+}
+
+extern "C" int fc_flow_set_grad(fc_flow* f, const int32_t* header, int n_header, const int64_t* table, int n_table,
+                                const float* arena, int64_t arena_floats) {
+    FC_REQUIRE(f && header && table && arena && n_header >= 4);
+    if (f->cpl_kind != FC_CPL_AFFINE || f->cif_dim) return FC_ERR_UNSUPPORTED;
+    if (header[0] != FC_GRAD_MAGIC || header[1] != FC_ARENA_VERSION) return FC_ERR_MODEL;
+    if (header[2] != f->L || header[3] != f->D || (reinterpret_cast<uintptr_t>(arena) & 15)) return FC_ERR_MODEL;
+    FcGradLayer* gl = new (std::nothrow) FcGradLayer[f->L];
+    if (!gl) return FC_ERR_MODEL;
+    FcGradLayer ga;
+    FcCursor c{table, n_table, 0, arena, arena_floats, true};
+    c.tc_fmt = 0;                                     // transposed weights: 3xTF32 copies whatever the model's format
+    const bool attn = !f->is_global;
+    if (f->has_aug) {
+        if (attn) {
+            ga.pre = read_mlp_t(c, f->d_in, false, f->augpre_hid, f->n_augpre_hid, f->attn_in);
+            ga.q = c.linear(f->inner, 0, f->attn_in, false);
+        }
+        ga.cpl = read_mlp_t(c, f->d_in, attn, f->aug_hid, f->n_aug_hid, 2 * (f->D - f->d_in));
+    }
+    for (int l = 0; l < f->L; ++l) {
+        FcGradLayer& y = gl[l];
+        if (attn) {
+            y.pre = read_mlp_t(c, f->half, false, f->pre_hid, f->n_pre_hid, f->attn_in);
+            y.q = c.linear(f->inner, 0, f->attn_in, false);
+        }
+        y.cpl = read_mlp_t(c, f->half, attn, f->hid, f->n_hid, 2 * (f->D - f->half));
+        if (f->layers[l].has_lu) y.lu = c.linear(f->D, 0, f->D, false);
+    }
+    if (!c.ok || c.pos != n_table) { delete[] gl; return FC_ERR_MODEL; }
+    delete[] f->glayers;
+    f->glayers = gl;
+    f->gaug = ga;
+    return FC_OK;
+}
+
+namespace {
+struct GradWs {
+    FlowWs fw;                                // the forward pass's own workspace (its buffers are reused by the recompute)
+    float* ckpt;                              // [L+1][M][ldx]
+    float *gA, *gB;                           // dL/d(latent), [M][ldx]
+    float* ppre[FC_MAX_HIDDEN + 1];           // pre-activations of the pre-attention MLP's in / hidden layers, [M][ldh]
+    float* cpre[FC_MAX_HIDDEN + 1];           // ... of the coupling (augmenter) MLP's
+    float* post[3];                           // activations of the recompute (h_i in post[i % 3])
+    float *h4, *dA, *dB, *raw, *dst, *dq, *dO;
+    int ldr;
+    int64_t total_bytes;
+};
+
+GradWs carve_grad_ws(const fc_flow* f, int B, int N, int Nc, void* base) {
+    GradWs g{};
+    g.fw = carve_flow_ws(f, B, N, Nc, base);
+    const int64_t M = (int64_t)B * N;
+    const int ldx = g.fw.ldx, ldh = g.fw.ldh;
+    const int n2 = f->D - f->half;
+    g.ldr = fc_round_up(2 * (n2 > f->D - f->d_in ? n2 : f->D - f->d_in), 4);
+    int64_t off = g.fw.total_bytes;
+    auto take = [&](int64_t floats) { float* p = base ? reinterpret_cast<float*>(reinterpret_cast<char*>(base) + off) : nullptr;
+                                      off += fc_round_up_ll(floats * 4, 256); return p; };
+    g.ckpt = take((int64_t)(f->L + 1) * M * ldx);
+    g.gA = take(M * ldx); g.gB = take(M * ldx);
+    const int np = f->is_global ? 0 : 1 + (f->n_pre_hid > f->n_augpre_hid ? f->n_pre_hid : f->n_augpre_hid);
+    const int nc = 1 + (f->n_hid > f->n_aug_hid ? f->n_hid : f->n_aug_hid);
+    for (int i = 0; i < np; ++i) g.ppre[i] = take(M * ldh);
+    for (int i = 0; i < nc; ++i) g.cpre[i] = take(M * ldh);
+    for (int i = 0; i < 3; ++i) g.post[i] = take(M * ldh);
+    g.h4 = take(f->is_global ? 0 : M * ldh);
+    g.dA = take(M * ldh); g.dB = take(M * ldh);
+    g.raw = take(M * g.ldr); g.dst = take(M * g.ldr);
+    g.dq = take(M * 64); g.dO = take(M * 64);
+    g.total_bytes = off;
+    return g;
+}
+}  // namespace
+
+extern "C" int64_t fc_flow_log_prob_grad_workspace_bytes(const fc_flow* f, int B, int N, int Nc) {
+    if (!f || B <= 0 || N <= 0 || Nc <= 0 || (int64_t)B * N > FC_GRAD_MAX_ROWS) return FC_ERR_INVALID_ARG;
+    return carve_grad_ws(f, B, N, Nc, nullptr).total_bytes;
+}
+
+// whether fc_launch_gemm runs this Linear on the tcgen05 path (whose epilogue evaluates GELU with fc_gelu_erf_fast)
+static bool runs_on_tc(const FcLinear& l, const float* A1, int lda1, const float* A2, int lda2, int M, int precision) {
+    if (precision != 1) return false;
+    GemmArgs g = fc_gemm_args_zero();
+    g.A1 = A1; g.lda1 = lda1; g.K1 = l.K1; g.A2 = A2; g.lda2 = lda2; g.K2 = l.K2;
+    g.Whi = l.whi; g.Wlo = l.wlo; g.ldk = l.ldk; g.M = M; g.N = l.N;
+    return fc_gemm_tc_supported(g);
+}
+
+// fc_run_mlp_hidden with every layer's pre-activation kept: the GEMM stores act's argument (residual included) in pre[i], the
+// forward's own activation for that GEMM path then gives h_i in post[i % 3].  Bitwise the forward's activations.
+static int mlp_recompute(const FcMlp& m, const FcMlpIn& in, int M, float* const* pre, float* const* post, int ldh, int precision,
+                         cudaStream_t s, const float** last) {
+    int rc = gemm_plain(m.in, in.A1, in.lda1, in.A2, in.lda2, in.bias, in.bias_ld, in.bias_group, nullptr, 0, FC_ACT_NONE, pre[0],
+                        ldh, M, precision, s);
+    if (rc) return rc;
+    rc = fc_launch_act_fwd(pre[0], ldh, post[0], ldh, M, m.in.N, m.act,
+                           runs_on_tc(m.in, in.A1, in.lda1, in.A2, in.lda2, M, precision), s);
+    if (rc) return rc;
+    for (int i = 0; i < m.n_hidden; ++i) {
+        const float* A = post[i % 3];
+        const float* res = (i & 1) ? post[(i + 2) % 3] : nullptr;     // odd i: h_{i-1} (reference models/nets.py:19-30)
+        rc = gemm_plain(m.hidden[i], A, ldh, nullptr, 0, nullptr, 0, 0, res, res ? ldh : 0, FC_ACT_NONE, pre[i + 1], ldh, M,
+                        precision, s);
+        if (rc) return rc;
+        rc = fc_launch_act_fwd(pre[i + 1], ldh, post[(i + 1) % 3], ldh, M, m.hidden[i].N, m.act,
+                               runs_on_tc(m.hidden[i], A, ldh, nullptr, 0, M, precision), s);
+        if (rc) return rc;
+    }
+    *last = post[m.n_hidden % 3];
+    return FC_OK;
+}
+
+// Backward through an MLP's hidden layers.  On entry *cur holds dL/d h_n (the last activation), *other is free; on exit *cur
+// holds dL/d pre_0.  Odd hidden layer i adds h_{i-1}: its dL/d pre_{i+1} stays in *other until it joins h_{i-1}'s gradient
+// through the next GEMM's residual.
+static int mlp_backward(const FcMlp& m, const FcMlpT& t, float* const* pre, int M, float** cur, float** other, int ldh,
+                        int precision, cudaStream_t s) {
+    const int hid = m.in.N;
+    int rc;
+    for (int i = m.n_hidden - 1; i >= 0; --i) {
+        rc = fc_launch_act_bwd(*cur, ldh, pre[i + 1], ldh, M, hid, m.act, s);
+        if (rc) return rc;
+        const bool add_res = !(i & 1) && i + 1 < m.n_hidden;
+        rc = gemm_plain(t.hidden[i], *cur, ldh, nullptr, 0, nullptr, 0, 0, add_res ? *other : nullptr, add_res ? ldh : 0,
+                        FC_ACT_NONE, *other, ldh, M, precision, s);
+        if (rc) return rc;
+        float* tmp = *cur; *cur = *other; *other = tmp;
+    }
+    return fc_launch_act_bwd(*cur, ldh, pre[0], ldh, M, hid, m.act, s);
+}
+
+// the forward of a pre-attention MLP and its attention block on lat[:, :pre.in.K1]: pre-activations in gw.ppre, the MLP's output
+// in gw.h4, q / o / mu / rstd in gw.fw, and k / v through the plain epilogue in gw.fw.kv (the tensor-core attention reads split
+// copies instead)
+static int attn_recompute(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const float* lat, int ldx, const float* context,
+                          int B, int N, int Nc, GradWs& gw, int precision, cudaStream_t s) {
+    const int M = B * N, ldh = gw.fw.ldh;
+    FcMlpIn in{lat, ldx, nullptr, 0, nullptr, 0, 0};
+    const float* last = nullptr;
+    int rc = mlp_recompute(pre, in, M, gw.ppre, gw.post, ldh, precision, s, &last);
+    if (rc) return rc;
+    rc = gemm_plain(pre.out, last, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.h4, ldh, M, precision, s);
+    if (rc) return rc;
+    rc = run_attention_core(f, at, gw.h4, ldh, context, B, N, Nc, gw.fw, precision, s, nullptr, nullptr);
+    if (rc) return rc;
+    return gemm_plain(at.kv, context, f->E, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.fw.kv, 128, B * Nc, precision, s);
+}
+
+// with dL/do in gw.dO: dq, then LayerNorm and the pre-attention MLP backwards; g[:, :K_in] += dL/d(its input)
+static int attn_backward(const fc_flow* f, const FcMlp& pre, const FcGradLayer& gl, int B, int N, int Nc, GradWs& gw, float* g,
+                         int ldg, int precision, cudaStream_t s) {
+    const int M = B * N, ldh = gw.fw.ldh;
+    int rc = fc_launch_attention_dq(gw.fw.q, gw.fw.kv, 128, gw.fw.o, gw.dO, gw.dq, B, N, Nc, 1.0f / sqrtf((float)f->inner), s);
+    if (rc) return rc;
+    rc = gemm_plain(gl.q, gw.dq, 64, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dA, ldh, M, precision, s);
+    if (rc) return rc;
+    rc = fc_launch_ln_bwd(gw.h4, ldh, gw.fw.mu, gw.fw.rstd, gw.dA, ldh, M, f->attn_in, s);
+    if (rc) return rc;
+    rc = gemm_plain(gl.pre.out, gw.dA, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dB, ldh, M, precision, s);
+    if (rc) return rc;
+    float* cur = gw.dB; float* other = gw.dA;
+    rc = mlp_backward(pre, gl.pre, gw.ppre, M, &cur, &other, ldh, precision, s);
+    if (rc) return rc;
+    return gemm_plain(gl.pre.in_x, cur, ldh, nullptr, 0, nullptr, 0, 0, g, ldg, FC_ACT_NONE, g, ldg, M, precision, s);
+}
+
+// One conditioner (a coupling layer's, or the augmenter's with aug = true) backwards.  lat: the block's input (its checkpoint);
+// g: dL/d(block output) on entry, dL/d(block input) on exit.
+static int conditioner_backward(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const FcMlp& net, const FcGradLayer& gl,
+                                bool aug, const float* lat, int cb_slot, const float* context, const float* eps, int B, int N, int Nc,
+                                GradWs& gw, float* g, int precision, cudaStream_t s) {
+    const int M = B * N, ldh = gw.fw.ldh, ldx = gw.fw.ldx;
+    const bool attn = !f->is_global;
+    int rc;
+    if (attn) {
+        rc = attn_recompute(f, pre, at, lat, ldx, context, B, N, Nc, gw, precision, s);
+        if (rc) return rc;
+    }
+    FcMlpIn in{lat, ldx, attn ? gw.fw.o : nullptr, 64, nullptr, 0, 0};
+    if (f->has_cb) { in.bias = gw.fw.cb + (size_t)cb_slot * f->hid; in.bias_ld = gw.fw.cb_ld; in.bias_group = N; }
+    const float* last = nullptr;
+    rc = mlp_recompute(net, in, M, gw.cpre, gw.post, ldh, precision, s, &last);
+    if (rc) return rc;
+    rc = gemm_plain(net.out, last, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.raw, gw.ldr, M, precision, s);
+    if (rc) return rc;
+    if (aug) rc = fc_launch_augment_tail_bwd(gw.raw, gw.ldr, eps, f->D - f->d_in, g, ldx, f->d_in, gw.dst, gw.ldr, M, s);
+    else     rc = fc_launch_coupling_tail_bwd(gw.raw, gw.ldr, lat, ldx, g, ldx, f->half, f->D - f->half, gw.dst, gw.ldr, M, s);
+    if (rc) return rc;
+    rc = gemm_plain(gl.cpl.out, gw.dst, gw.ldr, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dA, ldh, M, precision, s);
+    if (rc) return rc;
+    float* cur = gw.dA; float* other = gw.dB;
+    rc = mlp_backward(net, gl.cpl, gw.cpre, M, &cur, &other, ldh, precision, s);
+    if (rc) return rc;
+    rc = gemm_plain(gl.cpl.in_x, cur, ldh, nullptr, 0, nullptr, 0, 0, g, ldx, FC_ACT_NONE, g, ldx, M, precision, s);
+    if (rc || !attn) return rc;
+    rc = gemm_plain(gl.cpl.in_o, cur, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dO, 64, M, precision, s);
+    if (rc) return rc;
+    return attn_backward(f, pre, gl, B, N, Nc, gw, g, ldx, precision, s);
+}
+
+extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
+                                     float* log_prob_out, float* grad_out, int B, int N, int Nc, void* workspace,
+                                     int64_t workspace_bytes, int precision, fc_stream_t stream_) {
+    FC_REQUIRE(f && x && context && log_prob_out && grad_out && B > 0 && N > 0 && Nc > 0);
+    if (f->cpl_kind != FC_CPL_AFFINE || f->cif_dim) return FC_ERR_UNSUPPORTED;
+    if (!f->glayers) return FC_ERR_MODEL;
+    FC_REQUIRE((int64_t)B * N <= FC_GRAD_MAX_ROWS);
+    FC_REQUIRE(eps || !f->has_aug);
+    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return FC_ERR_WORKSPACE;
+    GradWs gw = carve_grad_ws(f, B, N, Nc, workspace);
+    if (gw.total_bytes > workspace_bytes) return FC_ERR_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream_;
+    int rc = flow_forward(f, x, context, extra, eps, nullptr, log_prob_out, nullptr, B, N, Nc, workspace, gw.fw.total_bytes, precision,
+                          stream_, nullptr, 0, gw.ckpt);
+    if (rc) return rc;
+    const int M = B * N, ldx = gw.fw.ldx;
+    auto slot = [&](int l) { return gw.ckpt + (size_t)l * M * ldx; };
+    // the base density N(0, I): d/dz sum(-z^2/2) = -z; ActNorm and LinearLU log-dets are constants
+    float* g = gw.gA; float* g_other = gw.gB;
+    rc = fc_launch_neg_copy(slot(f->L), ldx, g, ldx, M, f->D, s);
+    if (rc) return rc;
+    for (int l = f->L - 1; l >= 0; --l) {
+        const FcFlowLayer& y = f->layers[l];
+        const FcGradLayer& gl = f->glayers[l];
+        if (y.has_lu) {
+            // dz = g (W' - diag) + diag * g: the forward's off-diagonal / diagonal split, transposed
+            GemmArgs a = fc_gemm_args_zero();
+            a.A1 = g; a.lda1 = ldx; a.K1 = gl.lu.K1; a.Wt = gl.lu.w; a.ldw = gl.lu.ldw; a.Whi = gl.lu.whi; a.Wlo = gl.lu.wlo;
+            a.ldk = gl.lu.ldk; a.tc_fmt = gl.lu.tc_fmt; a.res = g; a.ldres = ldx; a.res_scale = y.lu_diag;
+            a.C = g_other; a.ldc = ldx; a.M = M; a.N = gl.lu.N; a.precision = precision;
+            rc = fc_launch_gemm(a, s);
+            if (rc) return rc;
+            float* t = g; g = g_other; g_other = t;
+        }
+        rc = conditioner_backward(f, y.pre, y.attn, y.cpl, gl, false, slot(l), l + 1, context, nullptr, B, N, Nc, gw, g, precision, s);
+        if (rc) return rc;
+    }
+    if (f->has_aug) {
+        rc = conditioner_backward(f, f->augpre, f->augattn, f->aug, f->gaug, true, slot(0), 0, context, eps, B, N, Nc, gw, g,
+                                  precision, s);
+        if (rc) return rc;
+    }
+    const long long tot = (long long)M * f->d_in;
+    copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(g, ldx, grad_out, f->d_in, M, f->d_in);
+    fc_count_launch();
+    FC_LAUNCH_OK();
+    return FC_OK;
 }

@@ -9,7 +9,8 @@ constexpr int FC_MAX_HIDDEN = 8;
 constexpr int32_t FC_FLOW_MAGIC = 0x46435F46;  // 'FC_F'
 constexpr int32_t FC_EMB_MAGIC = 0x46435F45;   // 'FC_E'
 constexpr int32_t FC_INV_MAGIC = 0x46435F49;   // 'FC_I': inverse ActNorm+LinearLU matrices of the sampling pass
-constexpr int32_t FC_ARENA_VERSION = 2;        // tensor-core weight copies: TF32 hi/lo (fp32 storage)
+constexpr int32_t FC_GRAD_MAGIC = 0x46435F47; // 'FC_G': transposed weights of the input-gradient pass
+constexpr int32_t FC_ARENA_VERSION = 2;       // tensor-core weight copies: TF32 hi/lo (fp32 storage)
 constexpr int32_t FC_ARENA_VERSION_F16 = 3;    // tensor-core weight copies: fp16 hi / scaled lo
 
 struct FcLinear {
@@ -55,6 +56,12 @@ struct FcFlowLayer {
     const float* cif_isc = nullptr; const float* cif_ibi = nullptr;   // its inverse (sampling pass, fc_flow_set_inverse)
 };
 
+// Transposed weights of the input-gradient pass (fc_flow_set_grad; flow_grad.cu).  Every backward contraction dX = dY W is a
+// Linear whose weight is W^T: `in_x` / `in_o` are the first layer's x columns and attention-output columns (the latter with the
+// out-projection folded in), hidden[i] / out the transposes of the forward's layers of the same index.
+struct FcMlpT { FcLinear in_x, in_o; FcLinear hidden[FC_MAX_HIDDEN]; FcLinear out; };
+struct FcGradLayer { FcMlpT pre, cpl; FcLinear q, lu; };   // q: Wq diag(gamma) transposed; lu: the off-diagonal part transposed
+
 struct fc_flow {
     int L, D, d_in, half, extra, is_global, E, inner, attn_in, hid, n_hid, pre_hid, n_pre_hid,
         aug_hid, n_aug_hid, augpre_hid, n_augpre_hid;
@@ -68,6 +75,8 @@ struct fc_flow {
     const float* arena = nullptr;
     int64_t arena_floats = 0;
     bool has_inverse = false;    // fc_flow_set_inverse was called (needed by fc_flow_sample)
+    FcGradLayer* glayers = nullptr;   // fc_flow_set_grad: per coupling layer, and the augmenter's in `gaug`
+    FcGradLayer gaug;
     // transforms no shipped config builds (SURVEY.md 8 a18; header words 19..): coupling kind 0 affine / 1 rational-quadratic
     // spline / 2 exponential, conditioner non-linearity, identity augmenter (latent_dim == input_dim), CIF block
     int cpl_kind = 0, num_bins = 0, act = FC_ACT_GELU, has_aug = 1;
@@ -162,6 +171,20 @@ int fc_expm_max_n();
 int fc_launch_scatter_draw(const float* src, int lds, int cols, const float* part_src, int n_part, float* dst, int ldd,
                            float* part_dst, int B, int N, int K, int k, cudaStream_t s);
 constexpr int64_t FC_DRAWS_MAX_ROWS = 1ll << 20;   // rows of one fc_flow_log_prob_draws pass
+
+// input-gradient pass (flow_grad.cu)
+int fc_launch_act_fwd(const float* pre, int ldp, float* post, int ldq, long long M, int width, int act, int fast, cudaStream_t s);
+int fc_launch_act_bwd(float* d, int ldd, const float* pre, int ldp, long long M, int width, int act, cudaStream_t s);
+int fc_launch_coupling_tail_bwd(const float* raw, int ldr, const float* x, int ldx, float* g, int ldg, int col0, int n2, float* dst,
+                                int ldd, int M, cudaStream_t s);
+int fc_launch_augment_tail_bwd(const float* raw, int ldr, const float* eps, int S, const float* g, int ldg, int col0, float* dst,
+                               int ldd, int M, cudaStream_t s);
+int fc_launch_ln_bwd(const float* h, int ldh, const float* mu, const float* rstd, float* d, int ldd, int M, int width, cudaStream_t s);
+int fc_launch_neg_copy(const float* z, int ldz, float* g, int ldg, long long M, int cols, cudaStream_t s);
+int fc_launch_attention_dq(const float* q, const float* kv, int ldkv, const float* o, const float* dO, float* dq, int B, int N,
+                           int Nc, float scale, cudaStream_t stream);
+constexpr int64_t FC_GRAD_MAX_ROWS = 1ll << 16;   // rows of one fc_flow_log_prob_grad pass
+bool fc_gemm_tc_supported(const GemmArgs& a);      // gemm_tc.cu
 
 // runs in/hidden layers of an MLP; returns the buffer holding the last hidden activation.
 // bufA/bufB: [M][ldh] scratch (ldh >= hidden width).  `in_bias`/group override the in-layer bias.

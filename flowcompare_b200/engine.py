@@ -37,6 +37,7 @@ def _f32c(t, device):
 
 
 IW_MAX_PASS_ROWS = 1 << 20      # rows (draws x points) of one fc_flow_log_prob_draws pass
+GRAD_MAX_PASS_ROWS = 1 << 16    # points of one fc_flow_log_prob_grad pass (11.8 GB of workspace at the shipped widths)
 
 
 def _n_draws(n, what):
@@ -89,6 +90,7 @@ class FlowCompareB200:
         self._tc_format = tc_format
         self._flow_sd_for_inverse = flow_sd      # the inverse ActNorm+LinearLU matrices are packed on the first make_sample
         self._inv = None
+        self._grad = None                        # the transposed weights of log_prob_grad are packed on its first call
         # reference Flow(sample_dist=Normal(loc, scale)) (model_initialization.py:154-161): buffers of the flow's state_dict
         self._sample_loc = float(flow_sd["sample_dist.loc"].reshape(-1)[0]) if "sample_dist.loc" in flow_sd else 0.0
         self._sample_scale = float(flow_sd["sample_dist.scale"].reshape(-1)[0]) if "sample_dist.scale" in flow_sd else 1.0
@@ -281,6 +283,62 @@ class FlowCompareB200:
             iw = torch.empty((B, N), dtype=torch.float32, device=self.device)
             _lib.check(self.lib.fc_logmeanexp(draws.data_ptr(), K, B * N, iw.data_ptr(), _stream()), "fc_logmeanexp")
         return (iw, draws) if return_draws else iw
+
+    def _ensure_grad(self):
+        bad = packing.grad_unsupported_transform(self.config)
+        if bad is not None:
+            raise _lib.FlowCompareError(f"log_prob_grad: input gradients through {bad} are not supported (affine couplings only)")
+        if self._grad is None:
+            header, table, arena = packing.pack_flow_grad(self._flow_sd_for_inverse, self.config)
+            with torch.cuda.device(self.device):
+                arena_dev = arena.to(self.device)
+                rc = self.lib.fc_flow_set_grad(self._flow["handle"], header.ctypes.data, len(header), table.ctypes.data, len(table),
+                                               arena_dev.data_ptr(), arena_dev.numel())
+            _lib.check(rc, "fc_flow_set_grad")
+            self._grad = {"arena": arena_dev, "header": header, "table": table}
+
+    def log_prob_grad(self, x, context, extra_context=None, eps=None, workspace_budget=None):
+        """Input gradients: (log_prob [B,N], grad [B,N,input_dim]) with grad[b,n] = d log_prob[b,n] / d x[b,n,:input_dim] -- what
+        `torch.autograd.grad(flow.log_prob(x, context=...).sum(), x)` gives on the reference (models/transform.py:70-76) with the
+        augmentation noise eps held fixed.  A point's log-prob depends on that point and the context only, so this per-point block
+        is the whole Jacobian: the gradient of sum(w * log_prob) is w[..., None] * grad.  The context, the extra context and the
+        weights are constants.  Arguments as `log_prob`; log_prob is bitwise `log_prob(x, context, eps=eps)`.
+        Clouds run in passes of at most 2^16 points (fewer when a pass's workspace would exceed `workspace_budget` bytes); the
+        result does not depend on the split.  Affine-coupling flows only: spline / exponential couplings and CIF blocks raise."""
+        self._ensure_grad()
+        with torch.cuda.device(self.device):
+            x = _f32c(x[..., :self.d_in], self.device)
+            B, N = x.shape[0], x.shape[1]
+            context, Nc, extra = self._prep_context(context, extra_context, B)
+            S = self.D - self.d_in
+            if eps is None:
+                eps = self.draw_eps(B, N)
+            else:
+                eps = _f32c(eps, self.device)
+                if tuple(eps.shape) != (B, N, S):
+                    raise _lib.FlowCompareError(f"log_prob_grad: eps must be [{B}, {N}, {S}], got {list(eps.shape)}")
+            if N > GRAD_MAX_PASS_ROWS:
+                raise _lib.FlowCompareError(f"log_prob_grad: {N} points per cloud exceed one pass of {GRAD_MAX_PASS_ROWS} rows")
+            h = self._flow["handle"]
+            wsb = lambda bc: self.lib.fc_flow_log_prob_grad_workspace_bytes(h, bc, N, Nc)
+            bc = min(B, GRAD_MAX_PASS_ROWS // N)                              # clouds per pass
+            if workspace_budget is not None:
+                while bc > 1 and wsb(bc) > workspace_budget:
+                    bc = (bc + 1) // 2
+            lp = torch.empty((B, N), dtype=torch.float32, device=self.device)
+            grad = torch.empty((B, N, self.d_in), dtype=torch.float32, device=self.device)
+            for b0 in range(0, B, bc):
+                b1 = min(B, b0 + bc)
+                nb = b1 - b0
+                nbytes = wsb(nb)
+                ws = self._workspace(nbytes)
+                pe = eps[b0:b1] if S else None
+                rc = self.lib.fc_flow_log_prob_grad(h, x[b0:b1].data_ptr(), context[b0:b1].data_ptr(),
+                                                    _ptr(None if extra is None else extra[b0:b1]), _ptr(pe),
+                                                    lp[b0:b1].data_ptr(), grad[b0:b1].data_ptr(), nb, N, Nc, ws, nbytes,
+                                                    self.precision, _stream())
+                _lib.check(rc, "fc_flow_log_prob_grad")
+        return lp, grad
 
     def _prep_context(self, context, extra_context, B):
         context = context.to(self.device)
@@ -650,6 +708,29 @@ def log_prob_to_change(log_prob_1_given_0, log_prob_0_given_0, multiple, hard_cu
 
 
 # ---------------------------------------------------------------------- drop-in adapters
+class _LogProbFunction(torch.autograd.Function):
+    """log_prob(x | context) with a backward for x: the forward is the plain `log_prob` with an explicit eps (so a caller that never
+    calls backward pays nothing extra), the backward `log_prob_grad` with that eps.  Context and extra context are constants."""
+
+    @staticmethod
+    def forward(ctx, x, context, extra_context, engine, eps):
+        ctx.engine, ctx.context, ctx.extra = engine, context, extra_context
+        ctx.save_for_backward(x, eps)
+        return engine.log_prob(x, context, extra_context, eps=eps)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            raise _lib.FlowCompareError("log_prob backward: gradients with respect to the context or the extra context are not "
+                                        "supported (only the target points x)")
+        x, eps = ctx.saved_tensors
+        _, g = ctx.engine.log_prob_grad(x.detach(), ctx.context, ctx.extra, eps=eps)
+        g = grad_output.to(g.device, g.dtype)[..., None] * g
+        if x.shape[-1] > g.shape[-1]:       # columns past input_dim do not enter the flow
+            g = torch.cat((g, g.new_zeros(g.shape[:-1] + (x.shape[-1] - g.shape[-1],))), dim=-1)
+        return g.to(x.device, x.dtype), None, None, None, None
+
+
 class _FlowAdapter:
     """Stands in for `models.Flow` inside a models_dict: same `log_prob` signature."""
 
@@ -659,6 +740,12 @@ class _FlowAdapter:
         self.z = None    # set to a tensor to inject the base draw of `sample` (parity tests)
 
     def log_prob(self, x, context=None, extra_context=None):
+        """`Flow.log_prob`.  With grad mode on and `x.requires_grad`, the result is differentiable with respect to x (the reference's
+        autograd through the flow, eps held at the value this call drew): backward runs `log_prob_grad`.  Otherwise this is the
+        plain call."""
+        if torch.is_grad_enabled() and isinstance(x, torch.Tensor) and x.requires_grad:
+            eps = self.eps if self.eps is not None else self.engine.draw_eps(x.shape[0], x.shape[1])
+            return _LogProbFunction.apply(x, context, extra_context, self.engine, eps)
         return self.engine.log_prob(x, context, extra_context, eps=self.eps)
 
     def sample(self, num_samples, n_points, context=None, sample_distrib=None, extra_context=None):

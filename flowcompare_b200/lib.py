@@ -68,6 +68,9 @@ SIGNATURES = {
     "fc_flow_set_inverse": (c_int, [c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_i64]),
     "fc_flow_sample": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
     "fc_flow_sample_cif": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
+    "fc_flow_set_grad": (c_int, [c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_i64]),
+    "fc_flow_log_prob_grad_workspace_bytes": (c_i64, [c_vp, c_int, c_int, c_int]),
+    "fc_flow_log_prob_grad": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
     "fc_embedder_create": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_i64, ctypes.POINTER(c_vp)]),
     "fc_embedder_destroy": (None, [c_vp]),
     "fc_embedder_workspace_bytes": (c_i64, [c_vp, c_int, c_int]),

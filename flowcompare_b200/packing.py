@@ -520,3 +520,80 @@ def pack_embedder(emb_sd, config, tc_format="tf32"):
     header = np.asarray([EMB_MAGIC, TC_FORMATS[tc_format], kind, cfg["input_dim"], cfg["n_neighbors"],
                          cfg["input_embedding_dim"], out_hid, n_out], dtype=np.int32)
     return header, table, arena
+
+
+GRAD_MAGIC = 0x46435F47
+
+
+def grad_unsupported_transform(config):
+    """The transform of this flow the input-gradient pass has no backward for (reference class name), or None."""
+    cfg = derive(config)
+    if cfg["latent_dim"] < cfg["cif_latent_dim"]:
+        return "CIFblock"
+    if cfg["flow_type"] != "AffineCoupling":
+        return cfg["flow_type"]
+    return None
+
+
+def _pack_mlp_t(ar, w_first, k_x, hidden, w_out, has_o):
+    """An MLP's backward contractions as Linears with the transposed weights: the first layer's x columns, its attention-output
+    columns (`has_o`), the hidden layers, the out layer (rows as the forward stores them)."""
+    ar.linear(w_first[:, :k_x].t(), None, w_first.shape[0])
+    if has_o:
+        ar.linear(w_first[:, k_x:].t(), None, w_first.shape[0])
+    for w, _ in hidden:
+        ar.linear(w.t(), None, w.shape[0])
+    ar.linear(w_out.t(), None, w_out.shape[0])
+
+
+def pack_flow_grad(flow_sd, config):
+    """Arena of the input-gradient pass (csrc/flow.cu: fc_flow_set_grad): the transpose W^T of every folded matrix the forward pass
+    runs, in the forward's order -- per conditioner the pre-attention MLP, to_q with the LayerNorm gain folded in (Wq diag(gamma)),
+    the coupling (augment) MLP with its first layer split into the x columns and the attention-output columns (out-projection
+    folded in), and the off-diagonal part of ActNorm + permuter.  Every backward contraction dX = dY W is then an ordinary Linear
+    with weight W^T.  The tensor-core copies are always 3xTF32 (fp32 exponent range): gradients are not bounded a priori, and the
+    3xFP16 format would turn values beyond fp16's range into NaN rows."""
+    cfg = derive(config)
+    bad = grad_unsupported_transform(cfg)
+    if bad is not None:
+        raise NotImplementedError(f"input gradients: no backward pass for {bad}")
+    L, D, d_in, ex = cfg["n_flow_layers"], cfg["latent_dim"], cfg["input_dim"], cfg["extra_context_dim"]
+    half = D // 2
+    is_global = bool(cfg["global"])
+    E = cfg["input_embedding_dim"]
+    ar = Arena("tf32")
+
+    def conditioner(pre_prefix, attn_prefix, mlp_prefix, k_x, fold_prefix):
+        if not is_global:
+            (w_in, _), hidden, (w_out, _) = _mlp_tensors(flow_sd, pre_prefix)
+            _pack_mlp_t(ar, w_in, k_x, hidden, w_out, False)
+            wq = _d(flow_sd, f"{attn_prefix}.fn.attention.to_q.weight")
+            gamma = _d(flow_sd, f"{attn_prefix}.norm.weight")
+            wq_f = (wq * gamma[None, :]).to(torch.float32).to(torch.float64)     # as pack_flow stores it
+            ar.linear(wq_f.t(), None, wq_f.shape[0])
+        w_g, _, _, _ = _conditioner_first_layer(flow_sd, mlp_prefix, fold_prefix, k_x, ex, is_global, E)   # as pack_flow folds it
+        (_, _), hidden, (w_out, b_out) = _mlp_tensors(flow_sd, mlp_prefix)
+        w_o, _ = _interleave_rows(w_out, b_out)
+        _pack_mlp_t(ar, w_g, k_x, hidden, w_o, not is_global)
+
+    if D > d_in:
+        conditioner("transforms.0.pre_attn_mlp", "transforms.0.attn", "transforms.0.augment.noise_dist.net", d_in,
+                    "transforms.0.attn")
+    t = 1
+    for layer in range(L):
+        p = _coupling_prefix(cfg, layer)
+        conditioner(f"{p}.pre_conditioner.pre_attention_mlp", f"{p}.pre_conditioner.attn", f"{p}.transform.nn", half,
+                    None if is_global else f"{p}.pre_conditioner.attn")
+        t += 1
+        if layer != L - 1:
+            if cfg["act_norm"]:
+                log_scale = _d(flow_sd, f"transforms.{t}.log_scale")[0]
+                t += 1
+            else:
+                log_scale = torch.zeros(D, dtype=torch.float64)
+            Wp = permuter_matrix(flow_sd, t, cfg)[0] @ torch.diag(torch.exp(-log_scale))
+            ar.linear((Wp - torch.diag(torch.diagonal(Wp))).t(), None, D)
+            t += 1
+    arena, table = ar.finish()
+    header = np.asarray([GRAD_MAGIC, ARENA_VERSION, L, D], dtype=np.int32)
+    return header, table, arena

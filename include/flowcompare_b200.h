@@ -315,6 +315,25 @@ FC_API int fc_flow_sample_cif(const fc_flow* h, const float* z, const float* con
                        const float* eps_cif, float* x_out, int B, int P, int Nc, void* workspace,
                        int64_t workspace_bytes, int precision, fc_stream_t stream);
 
+/* Input gradients: what autograd of `Flow.log_prob` (reference models/transform.py:70-76) gives with respect to the target
+ * points, `torch.autograd.grad(flow.log_prob(x, context=...).sum(), x)` with the augmentation noise eps held fixed.  A point's
+ * log-prob depends on that point and the context only, so grad_out[b, n, :] = d log_prob[b, n] / d x[b, n, :input_dim] is the
+ * whole Jacobian.  The context, the extra context and the weights are constants (no gradient flows to them).
+ *   fc_flow_set_grad attaches the transposed weights the backward GEMMs run (header/table/arena from packing.pack_flow_grad, always
+ *   3xTF32 tensor-core copies; the arena must outlive the handle); without it fc_flow_log_prob_grad returns FC_ERR_MODEL.
+ *   fc_flow_log_prob_grad: arguments as fc_flow_log_prob, plus grad_out [B, N, input_dim].  It runs the forward pass, keeping the
+ *   latent at the input of every coupling layer, then walks the layers backwards, recomputing each layer's forward from its
+ *   checkpoint.  log_prob_out is bitwise what fc_flow_log_prob returns.  Affine couplings only: flows with spline or exponential
+ *   couplings or CIF blocks return FC_ERR_UNSUPPORTED.  fc_flow_log_prob_grad_workspace_bytes(h, B, N, Nc) sizes the workspace
+ *   (about 181 KB per point at the shipped widths, most of it the checkpoints); one pass runs at most 2^16 points (B*N), else
+ *   FC_ERR_INVALID_ARG.                                      */
+FC_API int fc_flow_set_grad(fc_flow* h, const int32_t* header_host, int n_header, const int64_t* table_host, int n_table,
+                     const float* arena, int64_t arena_floats);
+FC_API int64_t fc_flow_log_prob_grad_workspace_bytes(const fc_flow* h, int B, int N, int Nc);
+FC_API int fc_flow_log_prob_grad(const fc_flow* h, const float* x, const float* context, const float* extra, const float* eps,
+                          float* log_prob_out, float* grad_out, int B, int N, int Nc, void* workspace,
+                          int64_t workspace_bytes, int precision, fc_stream_t stream);
+
 FC_API int fc_embedder_create(const int32_t* header_host, int n_header, const int64_t* table_host, int n_table,
                        const float* arena, int64_t arena_floats, fc_embedder** out);
 FC_API void fc_embedder_destroy(fc_embedder* h);
