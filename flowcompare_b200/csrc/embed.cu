@@ -106,14 +106,6 @@ extern "C" int64_t fc_embedder_workspace_bytes(const fc_embedder* e, int B, int 
     return carve_emb_ws(e, B, Nc, nullptr).total_bytes;
 }
 
-static int gemm_simple(const FcLinear& l, const float* A, int lda, int act, float* C, int ldc, int M, int precision,
-                       cudaStream_t s) {
-    GemmArgs g = fc_gemm_args_zero();
-    g.A1 = A; g.lda1 = lda; g.K1 = l.K1; g.Wt = l.w; g.ldw = l.ldw; g.bias = l.b; g.act = act; g.Whi = l.whi; g.Wlo = l.wlo; g.ldk = l.ldk; g.tc_fmt = l.tc_fmt;
-    g.C = C; g.ldc = ldc; g.M = M; g.N = l.N; g.precision = precision;
-    return fc_launch_gemm(g, s);
-}
-
 extern "C" int fc_embed(const fc_embedder* e, const float* pts, float* out, int B, int Nc, int32_t* knn_idx_out,
                         void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream_) {
     FC_REQUIRE(e && pts && out && B > 0 && Nc > 0);
@@ -135,19 +127,21 @@ extern "C" int fc_embed(const fc_embedder* e, const float* pts, float* out, int 
         if (rc) return rc;
         // the kNN is bit-exact by contract and its input feeds a discrete decision, so the [P|Q] GEMM
         // always runs in exact fp32
-        rc = gemm_simple(e->ec[i].pq, xin, ldin, FC_ACT_NONE, w.pq, 512, M, 0, s);
+        rc = fc_launch_gemm(fc_gemm_linear(e->ec[i].pq, xin, ldin, w.pq, 512, M, 0), s);
         if (rc) return rc;
         rc = fc_launch_edgeconv_gather_max(w.pq, 512, idx, B, Nc, e->k, e->ec[i].Cout, w.feat + col[i], 512, s);
         if (rc) return rc;
     }
-    rc = gemm_simple(e->conv5, w.feat, 512, FC_ACT_LRELU, w.pq, 512, M, 0, s);
+    GemmArgs g5 = fc_gemm_linear(e->conv5, w.feat, 512, w.pq, 512, M, 0);
+    g5.act = FC_ACT_LRELU;
+    rc = fc_launch_gemm(g5, s);
     if (rc) return rc;
     if (e->kind == 0) {
         FcMlpIn in{w.pq, 512, nullptr, 0, nullptr, 0, 0};
         float* last = nullptr;
         rc = fc_run_mlp_hidden(e->out_mlp, in, M, w.hA, w.hB, 512, precision, s, &last);
         if (rc) return rc;
-        return gemm_simple(e->out_mlp.out, last, 512, FC_ACT_NONE, out, e->E, M, precision, s);
+        return fc_launch_gemm(fc_gemm_linear(e->out_mlp.out, last, 512, out, e->E, M, precision), s);
     }
     pool_max_mean_kernel<<<dim3(512 / 32, B), 256, 0, s>>>(w.pq, 512, Nc, 512, w.pooled);
     fc_count_launch();
@@ -156,5 +150,5 @@ extern "C" int fc_embed(const fc_embedder* e, const float* pts, float* out, int 
     float* last = nullptr;
     rc = fc_run_mlp_hidden(e->out_mlp, in, B, w.hA, w.hB, 512, 0, s, &last);
     if (rc) return rc;
-    return gemm_simple(e->out_mlp.out, last, 512, FC_ACT_NONE, out, e->E, B, 0, s);
+    return fc_launch_gemm(fc_gemm_linear(e->out_mlp.out, last, 512, out, e->E, B, 0), s);
 }

@@ -13,7 +13,6 @@
 //   ActNorm + LinearLU folded into one 300x300 GEMM (act_norm.py:37-43, permuters.py:164-169)     1 GEMM
 // The running log-det never leaves fp32 registers/partials until the final reduction.
 #include "model.cuh"
-#include <cstdlib>
 #include <new>
 
 namespace {
@@ -125,36 +124,37 @@ int fc_launch_ln_stats(const float* h, int ldh, int M, int width, float eps, flo
     return FC_OK;
 }
 
-static int gemm_plain(const FcLinear& l, const float* A1, int lda1, const float* A2, int lda2, const float* bias,
-                      int bias_ld, int bias_group, const float* res, int ldres, int act, float* C, int ldc, int M,
-                      int precision, cudaStream_t stream) {
-    GemmArgs g = fc_gemm_args_zero();
-    g.A1 = A1; g.lda1 = lda1; g.K1 = l.K1; g.A2 = A2; g.lda2 = lda2; g.K2 = l.K2;
-    g.Wt = l.w; g.ldw = l.ldw; g.Whi = l.whi; g.Wlo = l.wlo; g.ldk = l.ldk; g.tc_fmt = l.tc_fmt;
-    if (bias) { g.bias = bias; g.bias_ld = bias_ld; g.bias_group = bias_group; }
-    else { g.bias = l.b; }
-    g.res = res; g.ldres = ldres; g.act = act; g.C = C; g.ldc = ldc; g.M = M; g.N = l.N;
-    g.precision = precision;
-    return fc_launch_gemm(g, stream);
+static int copy_cols(const float* src, int lds, float* dst, int ldd, long long M, int cols, cudaStream_t s) {
+    const long long tot = M * cols;
+    copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(src, lds, dst, ldd, M, cols);
+    fc_count_launch();
+    FC_LAUNCH_OK();
+    return FC_OK;
+}
+
+// an MLP's first layer on its input [A1 | A2], with the per-cloud bias in place of the packed one when `in` carries one
+static GemmArgs mlp_in_gemm(const FcMlp& m, const FcMlpIn& in, float* C, int ldc, int M, int precision) {
+    GemmArgs g = fc_gemm_linear(m.in, in.A1, in.lda1, C, ldc, M, precision);
+    g.A2 = in.A2; g.lda2 = in.lda2;
+    if (in.bias) { g.bias = in.bias; g.bias_ld = in.bias_ld; g.bias_group = in.bias_group; }
+    return g;
 }
 
 int fc_run_mlp_hidden(const FcMlp& m, const FcMlpIn& in, int M, float* bufA, float* bufB, int ldh, int precision,
                       cudaStream_t stream, float** last) {
     // reference models/nets.py:19-30: x = act(in(x)); even hidden i: res = x, x = act(layer(x));
     // odd i: x = act(res + layer(x))
-    int rc = gemm_plain(m.in, in.A1, in.lda1, in.A2, in.lda2, in.bias, in.bias_ld, in.bias_group, nullptr, 0,
-                        m.act, bufA, ldh, M, precision, stream);
+    GemmArgs g = mlp_in_gemm(m, in, bufA, ldh, M, precision);
+    g.act = m.act;
+    int rc = fc_launch_gemm(g, stream);
     if (rc) return rc;
     float* cur = bufA; float* other = bufB;
     for (int i = 0; i < m.n_hidden; ++i) {
-        if ((i & 1) == 0) {
-            rc = gemm_plain(m.hidden[i], cur, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, m.act, other, ldh, M,
-                            precision, stream);
-        } else {
-            // residual source is `other` (the activation before the previous layer); write in place over it
-            rc = gemm_plain(m.hidden[i], cur, ldh, nullptr, 0, nullptr, 0, 0, other, ldh, m.act, other, ldh, M,
-                            precision, stream);
-        }
+        g = fc_gemm_linear(m.hidden[i], cur, ldh, other, ldh, M, precision);
+        g.act = m.act;
+        // odd i: the residual source is `other` (the activation before the previous layer); written in place over it
+        if (i & 1) { g.res = other; g.ldres = ldh; }
+        rc = fc_launch_gemm(g, stream);
         if (rc) return rc;
         float* t = cur; cur = other; other = t;
     }
@@ -326,57 +326,38 @@ extern "C" int64_t fc_flow_workspace_bytes(const fc_flow* f, int B, int N, int N
 // out + i * B * n_query * Nc.
 struct FcCapture { const int32_t* slots; int n_slots; const int32_t* qidx; int n_query; float* out; };
 
-static int run_attention_core(const fc_flow* f, const FcAttn& at, const float* h4, int ldh4, const float* context, int B, int N,
-                              int Nc, FlowWs& w, int precision, cudaStream_t s, float* maps, const FcCapture* cap);
-
-// maps: where this block's weights go (nullptr: not captured; `cap` then unused)
-static int run_attention_block(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const float* lat, int ldx, int K_in,
-                               const float* context, int B, int N, int Nc, FlowWs& w, int precision, cudaStream_t s,
-                               float* maps = nullptr, const FcCapture* cap = nullptr) {
-    const int M = B * N;
-    FcMlpIn in{lat, ldx, nullptr, 0, nullptr, 0, 0};
-    (void)K_in;
-    float* last = nullptr;
-    int rc = fc_run_mlp_hidden(pre, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
-    if (rc) return rc;
-    float* h4 = (last == w.hA) ? w.hB : w.hA;
-    rc = gemm_plain(pre.out, last, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, h4, w.ldh, M, precision, s);
-    if (rc) return rc;
-    return run_attention_core(f, at, h4, w.ldh, context, B, N, Nc, w, precision, s, maps, cap);
+// a caller's workspace: 256-byte aligned and at least `need` bytes
+static bool ws_ok(const void* workspace, int64_t need, int64_t workspace_bytes) {
+    return workspace && !(reinterpret_cast<uintptr_t>(workspace) & 255) && need <= workspace_bytes;
 }
 
 // LayerNorm statistics, to_q, to_kv and the attention of one block, from its pre-attention MLP's output h4 [M][ldh4]: w.o
-// (and w.q, w.mu, w.rstd) afterwards
+// (and w.q, w.mu, w.rstd) afterwards.  maps: where this block's weights go (nullptr: not captured; `cap` then unused)
 static int run_attention_core(const fc_flow* f, const FcAttn& at, const float* h4, int ldh4, const float* context, int B, int N,
                               int Nc, FlowWs& w, int precision, cudaStream_t s, float* maps, const FcCapture* cap) {
     const int M = B * N;
     int rc = fc_launch_ln_stats(h4, ldh4, M, f->attn_in, 1e-5f, w.mu, w.rstd, s);
     if (rc) return rc;
     {
-        GemmArgs g = fc_gemm_args_zero();
-        g.A1 = h4; g.lda1 = ldh4; g.K1 = f->attn_in; g.Wt = at.q.w; g.ldw = at.q.ldw; g.bias = at.qbias; g.Whi = at.q.whi; g.Wlo = at.q.wlo; g.ldk = at.q.ldk; g.tc_fmt = at.q.tc_fmt;
-        g.C = w.q; g.ldc = 64; g.M = M; g.N = f->inner; g.epi = FC_EPI_LNQ; g.row_mu = w.mu; g.row_rstd = w.rstd;
-        g.csum = at.csum; g.precision = precision;
+        GemmArgs g = fc_gemm_linear(at.q, h4, ldh4, w.q, 64, M, precision);
+        g.bias = at.qbias; g.epi = FC_EPI_LNQ; g.row_mu = w.mu; g.row_rstd = w.rstd; g.csum = at.csum;
         rc = fc_launch_gemm(g, s);
         if (rc) return rc;
     }
     // reference models/perceiver.py:104: scale = inner_dim ** -0.5
     const float scale = 1.0f / sqrtf((float)f->inner);
+    const GemmArgs kv = fc_gemm_linear(at.kv, context, f->E, w.kv, 128, B * Nc, precision);
     if (maps) {
         // k through the plain epilogue into w.kv: the forward's own to_kv below either rewrites w.kv with the same values or
         // (tensor-core path) writes its split copies elsewhere and never reads it, so the forward is unchanged by the capture
-        rc = gemm_plain(at.kv, context, f->E, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.kv, 128, B * Nc, precision, s);
+        rc = fc_launch_gemm(kv, s);
         if (rc) return rc;
         rc = fc_launch_attention_maps(w.q, 64, w.kv, 128, cap->qidx, cap->n_query, maps, B, N, Nc, scale, s);
         if (rc) return rc;
     }
-    static int attn_kind = -1;   // FC_ATTN=mma: warp-level MMA kernel; FC_ATTN=split: tcgen05 with a separate split pass (A/B runs)
-    if (attn_kind < 0) { const char* e = getenv("FC_ATTN"); attn_kind = !e ? 0 : (e[0] == 'm' ? 1 : (e[0] == 's' ? 2 : 0)); }
-    if (precision == 1 && attn_kind == 0 && at.kv.N == 128 && at.kv.whi) {
+    if (precision == 1 && at.kv.N == 128 && at.kv.whi) {
         // to_kv writes the TF32 hi/lo copies of k and v^T the tcgen05 attention consumes, straight from its epilogue
-        GemmArgs g = fc_gemm_args_zero();
-        g.A1 = context; g.lda1 = f->E; g.K1 = at.kv.K1; g.Wt = at.kv.w; g.ldw = at.kv.ldw; g.bias = at.kv.b;
-        g.Whi = at.kv.whi; g.Wlo = at.kv.wlo; g.ldk = at.kv.ldk; g.tc_fmt = at.kv.tc_fmt; g.M = B * Nc; g.N = 128; g.precision = 1;
+        GemmArgs g = kv;
         g.epi = FC_EPI_KVSPLIT; g.ldc = 64; g.kv_nc = Nc;
         g.kv_f16 = at.kv.tc_fmt ? 1 : 0;      // 3xFP16 models run the attention on fp16 operands as well
         fc_attention_tc_scratch_layout(B, Nc, w.kvs, &g.C, &g.kv_klo, &g.kv_vthi, &g.kv_vtlo, &g.kv_ncp, g.kv_f16);
@@ -384,14 +365,102 @@ static int run_attention_core(const fc_flow* f, const FcAttn& at, const float* h
         if (rc) return rc;
         return fc_launch_cross_attention_tc(w.q, 64, nullptr, 0, w.o, 64, B, N, Nc, f->inner, scale, w.kvs, 1, g.kv_f16, s);
     }
-    rc = gemm_plain(at.kv, context, f->E, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.kv, 128, B * Nc,
-                    precision, s);
+    rc = fc_launch_gemm(kv, s);
     if (rc) return rc;
-    if (precision == 1) {
-        if (attn_kind == 1) return fc_launch_cross_attention_mma(w.q, 64, w.kv, 128, w.o, 64, B, N, Nc, f->inner, scale, s);
+    if (precision == 1)
         return fc_launch_cross_attention_tc(w.q, 64, w.kv, 128, w.o, 64, B, N, Nc, f->inner, scale, w.kvs, 0, at.kv.tc_fmt ? 1 : 0, s);
-    }
     return fc_launch_cross_attention(w.q, 64, w.kv, 128, w.o, 64, B, N, Nc, f->inner, scale, s);
+}
+
+// the pre-attention MLP on lat[:, :pre.in.K1], then run_attention_core
+static int run_attention_block(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const float* lat, int ldx,
+                               const float* context, int B, int N, int Nc, FlowWs& w, int precision, cudaStream_t s,
+                               float* maps = nullptr, const FcCapture* cap = nullptr) {
+    const int M = B * N;
+    FcMlpIn in{lat, ldx, nullptr, 0, nullptr, 0, 0};
+    float* last = nullptr;
+    int rc = fc_run_mlp_hidden(pre, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
+    if (rc) return rc;
+    float* h4 = (last == w.hA) ? w.hB : w.hA;
+    rc = fc_launch_gemm(fc_gemm_linear(pre.out, last, w.ldh, h4, w.ldh, M, precision), s);
+    if (rc) return rc;
+    return run_attention_core(f, at, h4, w.ldh, context, B, N, Nc, w, precision, s, maps, cap);
+}
+
+// per-cloud bias of every conditioner's first layer (extra context and/or global embedding) into w.cb
+static int run_cb_prologue(const fc_flow* f, const float* extra, const float* context, int B, FlowWs& w, cudaStream_t s) {
+    if (!f->has_cb) return FC_OK;
+    const int tot = B * w.cbA_ld;
+    build_cb_input_kernel<<<(tot + 255) / 256, 256, 0, s>>>(extra, context, f->E, f->extra, f->is_global, B, w.cbA_ld, w.cbA);
+    fc_count_launch();
+    FC_LAUNCH_OK();
+    return fc_launch_gemm(fc_gemm_linear(f->cb, w.cbA, w.cbA_ld, w.cb, w.cb_ld, B, 0 /* always exact fp32: tiny */), s);
+}
+
+// the first layer's input of a conditioner (slot 0: the augmenter's, l + 1: coupling layer l's) over N points per cloud: the
+// latent, the attention output (attention configs) and the per-cloud bias row of that slot
+static FcMlpIn conditioner_in(const fc_flow* f, const FlowWs& w, const float* lat, int slot, int N) {
+    FcMlpIn in{lat, w.ldx, f->is_global ? nullptr : w.o, 64, nullptr, 0, 0};
+    if (f->has_cb) { in.bias = w.cb + (size_t)slot * f->hid; in.bias_ld = w.cb_ld; in.bias_group = N; }
+    return in;
+}
+
+// an affine coupling in the epilogue of its conditioner's output GEMM, on latent columns from col0: x2 = x2 * s + t with the
+// log-det partials in w.cpart, or (inverse) x2 = (x2 - t) / s
+static int affine_coupling_gemm(const FcLinear& out, const float* last, float* lat, int col0, FlowWs& w, int M, int precision,
+                                bool inverse, cudaStream_t s) {
+    GemmArgs g = fc_gemm_linear(out, last, w.ldh, nullptr, 0, M, precision);
+    g.epi = inverse ? FC_EPI_COUPLING_INV : FC_EPI_COUPLING;
+    g.x = lat; g.ldx = w.ldx; g.col0 = col0; g.part = inverse ? nullptr : w.cpart;
+    return fc_launch_gemm(g, s);
+}
+
+// ActNorm + LinearLU as one GEMM, dst = diag.src + (W' - diag) src + b': the diagonal (~1) is applied to the fp32 latent in the
+// epilogue, the GEMM only carries the off-diagonal mixing, so its rounding (and the tensor core's accumulate truncation) acts on
+// the small part instead of shrinking z itself 114 times in a row.  The same split serves the inverse and, on the transposed
+// off-diagonal part, the input-gradient pass.
+static int lu_gemm(const FcLinear& l, const float* diag, const float* src, float* dst, int ldx, int M, int precision,
+                   cudaStream_t s) {
+    GemmArgs g = fc_gemm_linear(l, src, ldx, dst, ldx, M, precision);
+    g.res = src; g.ldres = ldx; g.res_scale = diag;
+    return fc_launch_gemm(g, s);
+}
+
+// Coupling layer l on lat (N points per cloud), forward or inverse: the conditioner reads the untouched half x1 (and the
+// attention output, the per-cloud bias) the same way in both directions; the transform then updates x2 = columns [half, D) in
+// place, the forward writing its log-det partials to w.cpart.  maps / cap: attention capture as in run_attention_core.
+static int run_coupling(const fc_flow* f, int l, float* lat, const float* context, int B, int N, int Nc, FlowWs& w, int precision,
+                        bool inverse, cudaStream_t s, float* maps = nullptr, const FcCapture* cap = nullptr) {
+    const FcFlowLayer& y = f->layers[l];
+    const int M = B * N, n2 = f->D - f->half, inv = inverse ? 1 : 0;
+    float* part = inverse ? nullptr : w.cpart;
+    int rc;
+    if (!f->is_global) {
+        rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, context, B, N, Nc, w, precision, s, maps, cap);
+        if (rc) return rc;
+    }
+    float* last = nullptr;
+    rc = fc_run_mlp_hidden(y.cpl, conditioner_in(f, w, lat, l + 1, N), M, w.hA, w.hB, w.ldh, precision, s, &last);
+    if (rc) return rc;
+    if (f->cpl_kind == FC_CPL_SPLINE) {
+        // reference models/spline_coupling.py:187-227: the conditioner's raw output, then the spline on x2 in place
+        rc = fc_launch_gemm(fc_gemm_linear(y.cpl.out, last, w.ldh, w.pbuf, w.ldp, M, precision), s);
+        if (rc) return rc;
+        return fc_launch_rq_spline(w.pbuf, w.ldp, lat, w.ldx, f->half, n2, f->num_bins, M, part, inv, s);
+    }
+    if (f->cpl_kind == FC_CPL_EXPO) {
+        // reference models/exponential_coupling.py:44-77, n^2 + n conditioner outputs per point: whole clouds at a time
+        for (int r0 = 0; r0 < M; r0 += w.p_rows) {
+            const int rows = M - r0 < w.p_rows ? M - r0 : w.p_rows;
+            rc = fc_launch_gemm(fc_gemm_linear(y.cpl.out, last + (size_t)r0 * w.ldh, w.ldh, w.pbuf, w.ldp, rows, precision), s);
+            if (rc) return rc;
+            rc = fc_launch_expm_action(w.pbuf, w.ldp, lat, w.ldx, f->half, n2, y.expo_sq, part, r0, rows, inv, s);
+            if (rc) return rc;
+        }
+        return FC_OK;
+    }
+    // reference models/affine_coupling.py:34-62
+    return affine_coupling_gemm(y.cpl.out, last, lat, f->half, w, M, precision, inverse, s);
 }
 
 // CIF block up to (not including) its attention-conditioned coupling, reference models/cif_block.py:71-93.  In the
@@ -408,20 +477,14 @@ static int run_cif_block(const fc_flow* f, const FcFlowLayer& y, float* lat, Flo
         float* last = nullptr;
         rc = fc_run_mlp_hidden(y.cifnet, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
         if (rc) return rc;
-        rc = gemm_plain(y.cifnet.out, last, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.pbuf, w.ldp_cif, M,
-                        precision, s);
+        rc = fc_launch_gemm(fc_gemm_linear(y.cifnet.out, last, w.ldh, w.pbuf, w.ldp_cif, M, precision), s);
         if (rc) return rc;
         rc = fc_launch_cond_normal(w.pbuf, w.ldp_cif, lat, w.ldx, D, S, eps_l, M, f->cif_clamp, w.cpart, pass, s);
         if (rc || pass == 1) return rc;
         FcMlpIn in2{lat + D, w.ldx, nullptr, 0, nullptr, 0, 0};
         rc = fc_run_mlp_hidden(y.affcif, in2, M, w.hA, w.hB, w.ldh, precision, s, &last);
         if (rc) return rc;
-        GemmArgs g = fc_gemm_args_zero();
-        const FcLinear& o = y.affcif.out;
-        g.A1 = last; g.lda1 = w.ldh; g.K1 = o.K1; g.Wt = o.w; g.ldw = o.ldw; g.bias = o.b; g.Whi = o.whi; g.Wlo = o.wlo; g.ldk = o.ldk;
-        g.tc_fmt = o.tc_fmt; g.M = M; g.N = o.N; g.epi = FC_EPI_COUPLING; g.x = lat; g.ldx = w.ldx; g.col0 = 0; g.part = w.cpart;
-        g.precision = precision;
-        rc = fc_launch_gemm(g, s);
+        rc = affine_coupling_gemm(y.affcif.out, last, lat, 0, w, M, precision, false, s);
         if (rc) return rc;
         rc = fc_launch_col_affine(lat, w.ldx, f->cif_dim, M, y.cif_sc, y.cif_bi, s);
         if (rc) return rc;
@@ -447,36 +510,20 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
     const int K = draws ? draws : 1;
     FC_REQUIRE((int64_t)B * N * K < (1ll << 31) && (int64_t)B * Nc < (1ll << 31));
     cudaStream_t s = (cudaStream_t)stream_;
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return FC_ERR_WORKSPACE;
     FlowWs w = carve_flow_ws(f, B, K * N, Nc, workspace);
-    if (w.total_bytes > workspace_bytes) return FC_ERR_WORKSPACE;
+    if (!ws_ok(workspace, w.total_bytes, workspace_bytes)) return FC_ERR_WORKSPACE;
     const int NK = K * N;            // points per cloud after the augmenter
     const int M = B * NK, M0 = B * N;
     float* xin = draws ? w.lat1 : w.lat0;     // the latent the augmenter reads x from and writes its draw into
     int rc;
 
     // x -> latent columns [0, d_in)
-    {
-        const long long tot = (long long)M0 * f->d_in;
-        copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(x, f->d_in, xin, w.ldx, M0, f->d_in);
-        fc_count_launch();
-        FC_LAUNCH_OK();
-    }
+    if ((rc = copy_cols(x, f->d_in, xin, w.ldx, M0, f->d_in, s))) return rc;
     // partial log-det slabs: the FFMA and tcgen05 GEMMs tile N differently (128 vs <=256 wide), so slabs a
     // path does not write must read as zero in finalize
     FC_CUDA_OK(cudaMemsetAsync(w.cpart, 0, (size_t)M * w.n_cpart * sizeof(float), s));
     FC_CUDA_OK(cudaMemsetAsync(w.apart, 0, (size_t)M * w.n_apart * sizeof(float), s));
-    // per-cloud bias of every conditioner's first layer (extra context and/or global embedding)
-    if (f->has_cb) {
-        const int tot = B * w.cbA_ld;
-        build_cb_input_kernel<<<(tot + 255) / 256, 256, 0, s>>>(extra, context, f->E, f->extra, f->is_global, B, w.cbA_ld, w.cbA);
-        fc_count_launch();
-        FC_LAUNCH_OK();
-        rc = gemm_plain(f->cb, w.cbA, w.cbA_ld, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.cb, w.cb_ld, B,
-                        0 /* always exact fp32: tiny */, s);
-        if (rc) return rc;
-    }
-    auto cb_ptr = [&](int slot) -> const float* { return f->has_cb ? w.cb + (size_t)slot * f->hid : nullptr; };
+    if ((rc = run_cb_prologue(f, extra, context, B, w, s))) return rc;
     int n_captured = 0;
     auto maps_for = [&](int slot) -> float* {
         if (!cap || n_captured >= cap->n_slots || cap->slots[n_captured] != slot) return nullptr;
@@ -485,20 +532,16 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
 
     // ---- transforms.0: augment (reference models/augmenter.py:15-19, :49-63); latent_dim == input_dim: IdentityTransform
     if (f->has_aug && !f->is_global) {
-        rc = run_attention_block(f, f->augpre, f->augattn, xin, w.ldx, f->d_in, context, B, N, Nc, w, precision, s,
-                                 maps_for(0), cap);
+        rc = run_attention_block(f, f->augpre, f->augattn, xin, w.ldx, context, B, N, Nc, w, precision, s, maps_for(0), cap);
         if (rc) return rc;
     }
     if (f->has_aug) {
-        FcMlpIn in{xin, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(0), w.cb_ld, N};
-        if (!f->has_cb) { in.bias = nullptr; in.bias_ld = 0; in.bias_group = 0; }
         float* last = nullptr;
-        rc = fc_run_mlp_hidden(f->aug, in, M0, w.hA, w.hB, w.ldh, precision, s, &last);
+        rc = fc_run_mlp_hidden(f->aug, conditioner_in(f, w, xin, 0, N), M0, w.hA, w.hB, w.ldh, precision, s, &last);
         if (rc) return rc;
-        GemmArgs g = fc_gemm_args_zero();
-        g.A1 = last; g.lda1 = w.ldh; g.K1 = f->aug_hid; g.Wt = f->aug.out.w; g.ldw = f->aug.out.ldw; g.bias = f->aug.out.b; g.Whi = f->aug.out.whi; g.Wlo = f->aug.out.wlo; g.ldk = f->aug.out.ldk; g.tc_fmt = f->aug.out.tc_fmt;
-        g.M = M0; g.N = f->aug.out.N; g.epi = FC_EPI_AUGMENT; g.x = xin; g.ldx = w.ldx; g.col0 = f->d_in;
-        g.part = w.apart; g.eps = eps; g.ld_eps = f->D - f->d_in; g.precision = precision;
+        GemmArgs g = fc_gemm_linear(f->aug.out, last, w.ldh, nullptr, 0, M0, precision);
+        g.epi = FC_EPI_AUGMENT; g.x = xin; g.ldx = w.ldx; g.col0 = f->d_in;
+        g.part = w.apart; g.eps = eps; g.ld_eps = f->D - f->d_in;
         if (!draws) {
             rc = fc_launch_gemm(g, s);
             if (rc) return rc;
@@ -539,49 +582,10 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
             rc = run_cif_block(f, y, lat, w, M, eps_cif + (size_t)l * M * (f->cif_dim - f->D), precision, s);
             if (rc) return rc;
         }
-        if (!f->is_global) {
-            rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, f->half, context, B, NK, Nc, w, precision, s,
-                                     maps_for(l + 1), cap);
-            if (rc) return rc;
-        }
-        FcMlpIn in{lat, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(l + 1), w.cb_ld, NK};
-        if (!f->has_cb) { in.bias = nullptr; in.bias_ld = 0; in.bias_group = 0; }
-        float* last = nullptr;
-        rc = fc_run_mlp_hidden(y.cpl, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
+        rc = run_coupling(f, l, lat, context, B, NK, Nc, w, precision, false, s, maps_for(l + 1), cap);
         if (rc) return rc;
-        if (f->cpl_kind == FC_CPL_SPLINE) {
-            // reference models/spline_coupling.py:187-210: the conditioner's raw output, then the spline on x2 in place
-            rc = gemm_plain(y.cpl.out, last, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.pbuf, w.ldp, M, precision, s);
-            if (rc) return rc;
-            rc = fc_launch_rq_spline(w.pbuf, w.ldp, lat, w.ldx, f->half, f->D - f->half, f->num_bins, M, w.cpart, 0, s);
-            if (rc) return rc;
-        } else if (f->cpl_kind == FC_CPL_EXPO) {
-            // reference models/exponential_coupling.py:44-58, n^2 + n conditioner outputs per point: whole clouds at a time
-            for (int r0 = 0; r0 < M; r0 += w.p_rows) {
-                const int rows = M - r0 < w.p_rows ? M - r0 : w.p_rows;
-                rc = gemm_plain(y.cpl.out, last + (size_t)r0 * w.ldh, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE,
-                                w.pbuf, w.ldp, rows, precision, s);
-                if (rc) return rc;
-                rc = fc_launch_expm_action(w.pbuf, w.ldp, lat, w.ldx, f->half, f->D - f->half, y.expo_sq, w.cpart, r0, rows, 0, s);
-                if (rc) return rc;
-            }
-        } else {
-            GemmArgs g = fc_gemm_args_zero();
-            g.A1 = last; g.lda1 = w.ldh; g.K1 = f->hid; g.Wt = y.cpl.out.w; g.ldw = y.cpl.out.ldw; g.bias = y.cpl.out.b; g.Whi = y.cpl.out.whi; g.Wlo = y.cpl.out.wlo; g.ldk = y.cpl.out.ldk; g.tc_fmt = y.cpl.out.tc_fmt;
-            g.M = M; g.N = y.cpl.out.N; g.epi = FC_EPI_COUPLING; g.x = lat; g.ldx = w.ldx; g.col0 = f->half;
-            g.part = w.cpart; g.precision = precision;
-            rc = fc_launch_gemm(g, s);
-            if (rc) return rc;
-        }
         if (y.has_lu) {
-            // z' = diag.z + (W' - diag) z + b': the diagonal (~1) is applied to the fp32 latent in the epilogue,
-            // the GEMM only carries the off-diagonal mixing, so its rounding (and the tensor core's accumulate
-            // truncation) acts on the small part instead of shrinking z itself 114 times in a row.
-            GemmArgs g = fc_gemm_args_zero();
-            g.A1 = lat; g.lda1 = w.ldx; g.K1 = y.lu.K1; g.Wt = y.lu.w; g.ldw = y.lu.ldw; g.Whi = y.lu.whi; g.Wlo = y.lu.wlo;
-            g.ldk = y.lu.ldk; g.tc_fmt = y.lu.tc_fmt; g.bias = y.lu.b; g.res = lat; g.ldres = w.ldx; g.res_scale = y.lu_diag;
-            g.C = lat_next; g.ldc = w.ldx; g.M = M; g.N = y.lu.N; g.precision = precision;
-            rc = fc_launch_gemm(g, s);
+            rc = lu_gemm(y.lu, y.lu_diag, lat, lat_next, w.ldx, M, precision, s);
             if (rc) return rc;
             float* t = lat; lat = lat_next; lat_next = t;
         }
@@ -594,12 +598,7 @@ static int flow_forward(const fc_flow* f, const float* x, const float* context, 
         fc_count_launch();
         FC_LAUNCH_OK();
     }
-    if (z_out) {   // the final latent, [B*N, D] contiguous
-        const long long tot = (long long)M * f->D;
-        copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(lat, w.ldx, z_out, f->D, M, f->D);
-        fc_count_launch();
-        FC_LAUNCH_OK();
-    }
+    if (z_out) return copy_cols(lat, w.ldx, z_out, f->D, M, f->D, s);   // the final latent, [B*N, D] contiguous
     return FC_OK;
 }
 
@@ -715,85 +714,31 @@ static int flow_sample(const fc_flow* f, const float* z, const float* context, c
     FC_REQUIRE((int64_t)B * P < (1ll << 31) && (int64_t)B * Nc < (1ll << 31));
     if (!f->has_inverse) return FC_ERR_MODEL;
     cudaStream_t s = (cudaStream_t)stream_;
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return FC_ERR_WORKSPACE;
     FlowWs w = carve_flow_ws(f, B, P, Nc, workspace);
-    if (w.total_bytes > workspace_bytes) return FC_ERR_WORKSPACE;
-    const int M = B * P;
-    const int n2 = f->D - f->half, S = f->cif_dim ? f->cif_dim - f->D : 0;
+    if (!ws_ok(workspace, w.total_bytes, workspace_bytes)) return FC_ERR_WORKSPACE;
+    const int M = B * P, S = f->cif_dim ? f->cif_dim - f->D : 0;
     int rc;
-    {
-        const long long tot = (long long)M * f->D;
-        copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(z, f->D, w.lat0, w.ldx, M, f->D);
-        fc_count_launch();
-        FC_LAUNCH_OK();
-    }
-    if (f->has_cb) {
-        const int tot = B * w.cbA_ld;
-        build_cb_input_kernel<<<(tot + 255) / 256, 256, 0, s>>>(extra, context, f->E, f->extra, f->is_global, B, w.cbA_ld, w.cbA);
-        fc_count_launch();
-        FC_LAUNCH_OK();
-        rc = gemm_plain(f->cb, w.cbA, w.cbA_ld, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.cb, w.cb_ld, B, 0, s);
-        if (rc) return rc;
-    }
-    auto cb_ptr = [&](int slot) -> const float* { return f->has_cb ? w.cb + (size_t)slot * f->hid : nullptr; };
-    auto coupling_inv_gemm = [&](const FcLinear& o, const float* last, float* lat) {
-        GemmArgs g = fc_gemm_args_zero();
-        g.A1 = last; g.lda1 = w.ldh; g.K1 = o.K1; g.Wt = o.w; g.ldw = o.ldw; g.bias = o.b; g.Whi = o.whi; g.Wlo = o.wlo;
-        g.ldk = o.ldk; g.tc_fmt = o.tc_fmt; g.M = M; g.N = o.N; g.epi = FC_EPI_COUPLING_INV; g.x = lat; g.ldx = w.ldx;
-        g.precision = precision;
-        return g;
-    };
+    if ((rc = copy_cols(z, f->D, w.lat0, w.ldx, M, f->D, s))) return rc;
+    if ((rc = run_cb_prologue(f, extra, context, B, w, s))) return rc;
     float* lat = w.lat0; float* lat_next = w.lat1;
     for (int l = f->L - 1; l >= 0; --l) {
         const FcFlowLayer& y = f->layers[l];
         if (y.has_lu) {
-            GemmArgs g = fc_gemm_args_zero();
-            g.A1 = lat; g.lda1 = w.ldx; g.K1 = y.lu_inv.K1; g.Wt = y.lu_inv.w; g.ldw = y.lu_inv.ldw; g.Whi = y.lu_inv.whi; g.Wlo = y.lu_inv.wlo;
-            g.ldk = y.lu_inv.ldk; g.tc_fmt = y.lu_inv.tc_fmt; g.bias = y.lu_inv.b; g.res = lat; g.ldres = w.ldx; g.res_scale = y.lu_inv_diag;
-            g.C = lat_next; g.ldc = w.ldx; g.M = M; g.N = y.lu_inv.N; g.precision = precision;
-            rc = fc_launch_gemm(g, s);
+            rc = lu_gemm(y.lu_inv, y.lu_inv_diag, lat, lat_next, w.ldx, M, precision, s);
             if (rc) return rc;
             float* t = lat; lat = lat_next; lat_next = t;
         }
-        // ---- the coupling's inverse: the conditioner reads the untouched half y1 exactly as in the forward pass
-        if (!f->is_global) {
-            rc = run_attention_block(f, y.pre, y.attn, lat, w.ldx, f->half, context, B, P, Nc, w, precision, s);
-            if (rc) return rc;
-        }
-        FcMlpIn in{lat, w.ldx, f->is_global ? nullptr : w.o, 64, cb_ptr(l + 1), w.cb_ld, P};
-        if (!f->has_cb) { in.bias = nullptr; in.bias_ld = 0; in.bias_group = 0; }
-        float* last = nullptr;
-        rc = fc_run_mlp_hidden(y.cpl, in, M, w.hA, w.hB, w.ldh, precision, s, &last);
+        rc = run_coupling(f, l, lat, context, B, P, Nc, w, precision, true, s);
         if (rc) return rc;
-        if (f->cpl_kind == FC_CPL_SPLINE) {            // reference models/spline_coupling.py:212-227
-            rc = gemm_plain(y.cpl.out, last, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.pbuf, w.ldp, M, precision, s);
-            if (rc) return rc;
-            rc = fc_launch_rq_spline(w.pbuf, w.ldp, lat, w.ldx, f->half, n2, f->num_bins, M, nullptr, 1, s);
-            if (rc) return rc;
-        } else if (f->cpl_kind == FC_CPL_EXPO) {       // reference models/exponential_coupling.py:60-77
-            for (int r0 = 0; r0 < M; r0 += w.p_rows) {
-                const int rows = M - r0 < w.p_rows ? M - r0 : w.p_rows;
-                rc = gemm_plain(y.cpl.out, last + (size_t)r0 * w.ldh, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE,
-                                w.pbuf, w.ldp, rows, precision, s);
-                if (rc) return rc;
-                rc = fc_launch_expm_action(w.pbuf, w.ldp, lat, w.ldx, f->half, n2, y.expo_sq, nullptr, r0, rows, 1, s);
-                if (rc) return rc;
-            }
-        } else {                                       // reference models/affine_coupling.py:48-62
-            GemmArgs g = coupling_inv_gemm(y.cpl.out, last, lat);
-            g.col0 = f->half;
-            rc = fc_launch_gemm(g, s);
-            if (rc) return rc;
-        }
         if (f->cif_dim) {
             // CIFblock.inverse after its flow (reference models/cif_block.py:102-111), Reverse folded as in the forward pass:
             // the sliced-off columns are SAMPLED from the ConditionalNormal of what was kept (models/slice.py:46-58), then the
             // inverse ActNorm on all cif_dim columns and x = (x - t(z2)) / s(z2); Augment.inverse drops the extra columns.
             FcMlpIn inc{lat, w.ldx, nullptr, 0, nullptr, 0, 0};
+            float* last = nullptr;
             rc = fc_run_mlp_hidden(y.cifnet, inc, M, w.hA, w.hB, w.ldh, precision, s, &last);
             if (rc) return rc;
-            rc = gemm_plain(y.cifnet.out, last, w.ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, w.pbuf, w.ldp_cif, M,
-                            precision, s);
+            rc = fc_launch_gemm(fc_gemm_linear(y.cifnet.out, last, w.ldh, w.pbuf, w.ldp_cif, M, precision), s);
             if (rc) return rc;
             rc = fc_launch_cond_normal(w.pbuf, w.ldp_cif, lat, w.ldx, f->D, S, eps_cif + (size_t)l * M * S, M, f->cif_clamp,
                                        w.cpart /* log-density not needed: scratch */, 0, s);
@@ -803,17 +748,11 @@ static int flow_sample(const fc_flow* f, const float* z, const float* context, c
             FcMlpIn in2{lat + f->D, w.ldx, nullptr, 0, nullptr, 0, 0};
             rc = fc_run_mlp_hidden(y.affcif, in2, M, w.hA, w.hB, w.ldh, precision, s, &last);
             if (rc) return rc;
-            GemmArgs g = coupling_inv_gemm(y.affcif.out, last, lat);
-            g.col0 = 0;
-            rc = fc_launch_gemm(g, s);
+            rc = affine_coupling_gemm(y.affcif.out, last, lat, 0, w, M, precision, true, s);
             if (rc) return rc;
         }
     }
-    const long long tot = (long long)M * f->d_in;
-    copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(lat, w.ldx, x_out, f->d_in, M, f->d_in);
-    fc_count_launch();
-    FC_LAUNCH_OK();
-    return FC_OK;
+    return copy_cols(lat, w.ldx, x_out, f->d_in, M, f->d_in, s);
 }
 
 extern "C" int fc_flow_sample(const fc_flow* f, const float* z, const float* context, const float* extra, float* x_out, int B,
@@ -924,33 +863,24 @@ extern "C" int64_t fc_flow_log_prob_grad_workspace_bytes(const fc_flow* f, int B
     return carve_grad_ws(f, B, N, Nc, nullptr).total_bytes;
 }
 
-// whether fc_launch_gemm runs this Linear on the tcgen05 path (whose epilogue evaluates GELU with fc_gelu_erf_fast)
-static bool runs_on_tc(const FcLinear& l, const float* A1, int lda1, const float* A2, int lda2, int M, int precision) {
-    if (precision != 1) return false;
-    GemmArgs g = fc_gemm_args_zero();
-    g.A1 = A1; g.lda1 = lda1; g.K1 = l.K1; g.A2 = A2; g.lda2 = lda2; g.K2 = l.K2;
-    g.Whi = l.whi; g.Wlo = l.wlo; g.ldk = l.ldk; g.M = M; g.N = l.N;
-    return fc_gemm_tc_supported(g);
-}
+// whether fc_launch_gemm runs this GEMM on the tcgen05 path (whose epilogue evaluates GELU with fc_gelu_erf_fast)
+static bool runs_on_tc(const GemmArgs& g) { return g.precision == 1 && fc_gemm_tc_supported(g); }
 
 // fc_run_mlp_hidden with every layer's pre-activation kept: the GEMM stores act's argument (residual included) in pre[i], the
 // forward's own activation for that GEMM path then gives h_i in post[i % 3].  Bitwise the forward's activations.
 static int mlp_recompute(const FcMlp& m, const FcMlpIn& in, int M, float* const* pre, float* const* post, int ldh, int precision,
                          cudaStream_t s, const float** last) {
-    int rc = gemm_plain(m.in, in.A1, in.lda1, in.A2, in.lda2, in.bias, in.bias_ld, in.bias_group, nullptr, 0, FC_ACT_NONE, pre[0],
-                        ldh, M, precision, s);
+    GemmArgs g = mlp_in_gemm(m, in, pre[0], ldh, M, precision);
+    int rc = fc_launch_gemm(g, s);
     if (rc) return rc;
-    rc = fc_launch_act_fwd(pre[0], ldh, post[0], ldh, M, m.in.N, m.act,
-                           runs_on_tc(m.in, in.A1, in.lda1, in.A2, in.lda2, M, precision), s);
+    rc = fc_launch_act_fwd(pre[0], ldh, post[0], ldh, M, m.in.N, m.act, runs_on_tc(g), s);
     if (rc) return rc;
     for (int i = 0; i < m.n_hidden; ++i) {
-        const float* A = post[i % 3];
-        const float* res = (i & 1) ? post[(i + 2) % 3] : nullptr;     // odd i: h_{i-1} (reference models/nets.py:19-30)
-        rc = gemm_plain(m.hidden[i], A, ldh, nullptr, 0, nullptr, 0, 0, res, res ? ldh : 0, FC_ACT_NONE, pre[i + 1], ldh, M,
-                        precision, s);
+        g = fc_gemm_linear(m.hidden[i], post[i % 3], ldh, pre[i + 1], ldh, M, precision);
+        if (i & 1) { g.res = post[(i + 2) % 3]; g.ldres = ldh; }     // odd i: h_{i-1} (reference models/nets.py:19-30)
+        rc = fc_launch_gemm(g, s);
         if (rc) return rc;
-        rc = fc_launch_act_fwd(pre[i + 1], ldh, post[(i + 1) % 3], ldh, M, m.hidden[i].N, m.act,
-                               runs_on_tc(m.hidden[i], A, ldh, nullptr, 0, M, precision), s);
+        rc = fc_launch_act_fwd(pre[i + 1], ldh, post[(i + 1) % 3], ldh, M, m.hidden[i].N, m.act, runs_on_tc(g), s);
         if (rc) return rc;
     }
     *last = post[m.n_hidden % 3];
@@ -967,9 +897,9 @@ static int mlp_backward(const FcMlp& m, const FcMlpT& t, float* const* pre, int 
     for (int i = m.n_hidden - 1; i >= 0; --i) {
         rc = fc_launch_act_bwd(*cur, ldh, pre[i + 1], ldh, M, hid, m.act, s);
         if (rc) return rc;
-        const bool add_res = !(i & 1) && i + 1 < m.n_hidden;
-        rc = gemm_plain(t.hidden[i], *cur, ldh, nullptr, 0, nullptr, 0, 0, add_res ? *other : nullptr, add_res ? ldh : 0,
-                        FC_ACT_NONE, *other, ldh, M, precision, s);
+        GemmArgs g = fc_gemm_linear(t.hidden[i], *cur, ldh, *other, ldh, M, precision);
+        if (!(i & 1) && i + 1 < m.n_hidden) { g.res = *other; g.ldres = ldh; }
+        rc = fc_launch_gemm(g, s);
         if (rc) return rc;
         float* tmp = *cur; *cur = *other; *other = tmp;
     }
@@ -986,29 +916,31 @@ static int attn_recompute(const fc_flow* f, const FcMlp& pre, const FcAttn& at, 
     const float* last = nullptr;
     int rc = mlp_recompute(pre, in, M, gw.ppre, gw.post, ldh, precision, s, &last);
     if (rc) return rc;
-    rc = gemm_plain(pre.out, last, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.h4, ldh, M, precision, s);
+    rc = fc_launch_gemm(fc_gemm_linear(pre.out, last, ldh, gw.h4, ldh, M, precision), s);
     if (rc) return rc;
     rc = run_attention_core(f, at, gw.h4, ldh, context, B, N, Nc, gw.fw, precision, s, nullptr, nullptr);
     if (rc) return rc;
-    return gemm_plain(at.kv, context, f->E, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.fw.kv, 128, B * Nc, precision, s);
+    return fc_launch_gemm(fc_gemm_linear(at.kv, context, f->E, gw.fw.kv, 128, B * Nc, precision), s);
 }
 
-// with dL/do in gw.dO: dq, then LayerNorm and the pre-attention MLP backwards; g[:, :K_in] += dL/d(its input)
+// with dL/do in gw.dO: dq, then LayerNorm and the pre-attention MLP backwards; g[:, :pre.in.K1] += dL/d(its input)
 static int attn_backward(const fc_flow* f, const FcMlp& pre, const FcGradLayer& gl, int B, int N, int Nc, GradWs& gw, float* g,
                          int ldg, int precision, cudaStream_t s) {
     const int M = B * N, ldh = gw.fw.ldh;
     int rc = fc_launch_attention_dq(gw.fw.q, gw.fw.kv, 128, gw.fw.o, gw.dO, gw.dq, B, N, Nc, 1.0f / sqrtf((float)f->inner), s);
     if (rc) return rc;
-    rc = gemm_plain(gl.q, gw.dq, 64, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dA, ldh, M, precision, s);
+    rc = fc_launch_gemm(fc_gemm_linear(gl.q, gw.dq, 64, gw.dA, ldh, M, precision), s);
     if (rc) return rc;
     rc = fc_launch_ln_bwd(gw.h4, ldh, gw.fw.mu, gw.fw.rstd, gw.dA, ldh, M, f->attn_in, s);
     if (rc) return rc;
-    rc = gemm_plain(gl.pre.out, gw.dA, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dB, ldh, M, precision, s);
+    rc = fc_launch_gemm(fc_gemm_linear(gl.pre.out, gw.dA, ldh, gw.dB, ldh, M, precision), s);
     if (rc) return rc;
     float* cur = gw.dB; float* other = gw.dA;
     rc = mlp_backward(pre, gl.pre, gw.ppre, M, &cur, &other, ldh, precision, s);
     if (rc) return rc;
-    return gemm_plain(gl.pre.in_x, cur, ldh, nullptr, 0, nullptr, 0, 0, g, ldg, FC_ACT_NONE, g, ldg, M, precision, s);
+    GemmArgs a = fc_gemm_linear(gl.pre.in_x, cur, ldh, g, ldg, M, precision);
+    a.res = g; a.ldres = ldg;
+    return fc_launch_gemm(a, s);
 }
 
 // One conditioner (a coupling layer's, or the augmenter's with aug = true) backwards.  lat: the block's input (its checkpoint);
@@ -1023,24 +955,24 @@ static int conditioner_backward(const fc_flow* f, const FcMlp& pre, const FcAttn
         rc = attn_recompute(f, pre, at, lat, ldx, context, B, N, Nc, gw, precision, s);
         if (rc) return rc;
     }
-    FcMlpIn in{lat, ldx, attn ? gw.fw.o : nullptr, 64, nullptr, 0, 0};
-    if (f->has_cb) { in.bias = gw.fw.cb + (size_t)cb_slot * f->hid; in.bias_ld = gw.fw.cb_ld; in.bias_group = N; }
     const float* last = nullptr;
-    rc = mlp_recompute(net, in, M, gw.cpre, gw.post, ldh, precision, s, &last);
+    rc = mlp_recompute(net, conditioner_in(f, gw.fw, lat, cb_slot, N), M, gw.cpre, gw.post, ldh, precision, s, &last);
     if (rc) return rc;
-    rc = gemm_plain(net.out, last, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.raw, gw.ldr, M, precision, s);
+    rc = fc_launch_gemm(fc_gemm_linear(net.out, last, ldh, gw.raw, gw.ldr, M, precision), s);
     if (rc) return rc;
     if (aug) rc = fc_launch_augment_tail_bwd(gw.raw, gw.ldr, eps, f->D - f->d_in, g, ldx, f->d_in, gw.dst, gw.ldr, M, s);
     else     rc = fc_launch_coupling_tail_bwd(gw.raw, gw.ldr, lat, ldx, g, ldx, f->half, f->D - f->half, gw.dst, gw.ldr, M, s);
     if (rc) return rc;
-    rc = gemm_plain(gl.cpl.out, gw.dst, gw.ldr, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dA, ldh, M, precision, s);
+    rc = fc_launch_gemm(fc_gemm_linear(gl.cpl.out, gw.dst, gw.ldr, gw.dA, ldh, M, precision), s);
     if (rc) return rc;
     float* cur = gw.dA; float* other = gw.dB;
     rc = mlp_backward(net, gl.cpl, gw.cpre, M, &cur, &other, ldh, precision, s);
     if (rc) return rc;
-    rc = gemm_plain(gl.cpl.in_x, cur, ldh, nullptr, 0, nullptr, 0, 0, g, ldx, FC_ACT_NONE, g, ldx, M, precision, s);
+    GemmArgs a = fc_gemm_linear(gl.cpl.in_x, cur, ldh, g, ldx, M, precision);
+    a.res = g; a.ldres = ldx;
+    rc = fc_launch_gemm(a, s);
     if (rc || !attn) return rc;
-    rc = gemm_plain(gl.cpl.in_o, cur, ldh, nullptr, 0, nullptr, 0, 0, nullptr, 0, FC_ACT_NONE, gw.dO, 64, M, precision, s);
+    rc = fc_launch_gemm(fc_gemm_linear(gl.cpl.in_o, cur, ldh, gw.dO, 64, M, precision), s);
     if (rc) return rc;
     return attn_backward(f, pre, gl, B, N, Nc, gw, g, ldx, precision, s);
 }
@@ -1053,9 +985,8 @@ extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const flo
     if (!f->glayers) return FC_ERR_MODEL;
     FC_REQUIRE((int64_t)B * N <= FC_GRAD_MAX_ROWS);
     FC_REQUIRE(eps || !f->has_aug);
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) return FC_ERR_WORKSPACE;
     GradWs gw = carve_grad_ws(f, B, N, Nc, workspace);
-    if (gw.total_bytes > workspace_bytes) return FC_ERR_WORKSPACE;
+    if (!ws_ok(workspace, gw.total_bytes, workspace_bytes)) return FC_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream_;
     int rc = flow_forward(f, x, context, extra, eps, nullptr, log_prob_out, nullptr, B, N, Nc, workspace, gw.fw.total_bytes, precision,
                           stream_, nullptr, 0, gw.ckpt);
@@ -1071,11 +1002,7 @@ extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const flo
         const FcGradLayer& gl = f->glayers[l];
         if (y.has_lu) {
             // dz = g (W' - diag) + diag * g: the forward's off-diagonal / diagonal split, transposed
-            GemmArgs a = fc_gemm_args_zero();
-            a.A1 = g; a.lda1 = ldx; a.K1 = gl.lu.K1; a.Wt = gl.lu.w; a.ldw = gl.lu.ldw; a.Whi = gl.lu.whi; a.Wlo = gl.lu.wlo;
-            a.ldk = gl.lu.ldk; a.tc_fmt = gl.lu.tc_fmt; a.res = g; a.ldres = ldx; a.res_scale = y.lu_diag;
-            a.C = g_other; a.ldc = ldx; a.M = M; a.N = gl.lu.N; a.precision = precision;
-            rc = fc_launch_gemm(a, s);
+            rc = lu_gemm(gl.lu, y.lu_diag, g, g_other, ldx, M, precision, s);
             if (rc) return rc;
             float* t = g; g = g_other; g_other = t;
         }
@@ -1087,9 +1014,5 @@ extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const flo
                                   precision, s);
         if (rc) return rc;
     }
-    const long long tot = (long long)M * f->d_in;
-    copy_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(g, ldx, grad_out, f->d_in, M, f->d_in);
-    fc_count_launch();
-    FC_LAUNCH_OK();
-    return FC_OK;
+    return copy_cols(g, ldx, grad_out, f->d_in, M, f->d_in, s);
 }

@@ -21,6 +21,17 @@ struct FcLinear {
     int tc_fmt = 0;            // format of whi / wlo (GemmArgs::tc_fmt)
 };
 
+// C = A1 l + l.b through the plain-store epilogue: every field of the packed Linear (K1, K2, N, its bias, the FFMA weights, the
+// tensor-core copies, their K stride and format) is bound here, so no caller can drop one and silently take another GEMM path
+// or format.  Callers set only what differs: A2 / lda2, a bias override, res / res_scale, act and the epilogue fields.
+static inline GemmArgs fc_gemm_linear(const FcLinear& l, const float* A1, int lda1, float* C, int ldc, int M, int precision) {
+    GemmArgs g = fc_gemm_args_zero();
+    g.A1 = A1; g.lda1 = lda1; g.K1 = l.K1; g.K2 = l.K2; g.N = l.N; g.bias = l.b;
+    g.Wt = l.w; g.ldw = l.ldw; g.Whi = l.whi; g.Wlo = l.wlo; g.ldk = l.ldk; g.tc_fmt = l.tc_fmt;
+    g.C = C; g.ldc = ldc; g.M = M; g.precision = precision;
+    return g;
+}
+
 struct FcMlp {
     FcLinear in;
     FcLinear hidden[FC_MAX_HIDDEN];
@@ -138,8 +149,6 @@ struct FcCursor {
 int fc_launch_ln_stats(const float* h, int ldh, int M, int width, float eps, float* mu, float* rstd, cudaStream_t s);
 int fc_launch_cross_attention(const float* q, int ldq, const float* kv, int ldkv, float* out, int ldo,
                               int B, int N, int Nc, int d, float scale, cudaStream_t stream);
-int fc_launch_cross_attention_mma(const float* q, int ldq, const float* kv, int ldkv, float* out, int ldo,
-                                  int B, int N, int Nc, int d, float scale, cudaStream_t stream);
 // tcgen05 / TMEM version (attention_tc.cu); scratch holds the TF32 hi/lo copies of k and v^T
 int64_t fc_attention_tc_scratch_floats(int B, int Nc);
 void fc_attention_tc_scratch_layout(int B, int Nc, float* scratch, float** khi, float** klo, float** vthi, float** vtlo,

@@ -425,13 +425,6 @@ PaWs carve_pa(const fc_embedder* e, const PaModel* pm, int B, int Nc, void* base
     return w;
 }
 
-int gemm_relu(const FcLinear& l, const float* A, int lda, int act, float* C, int ldc, long long M, int precision, cudaStream_t s) {
-    GemmArgs g = fc_gemm_args_zero();
-    g.A1 = A; g.lda1 = lda; g.K1 = l.K1; g.Wt = l.w; g.ldw = l.ldw; g.bias = l.b; g.act = act; g.Whi = l.whi; g.Wlo = l.wlo;
-    g.ldk = l.ldk; g.tc_fmt = l.tc_fmt; g.C = C; g.ldc = ldc; g.M = (int)M; g.N = l.N; g.precision = precision;
-    return fc_launch_gemm(g, s);
-}
-
 }  // namespace
 
 int fc_paconv_create(FcCursor& c, const int32_t* header, int n_header, fc_embedder* e) {
@@ -506,7 +499,9 @@ int fc_paconv_embed(const fc_embedder* e, const float* pts, float* out, int B, i
             const int ldx = PA_M * 2 * L.Cin;
             paconv_expand_kernel<<<(unsigned)(edges / PA_K), 256, 0, s>>>(cur, ldf, L.Cin, w.dxyz, L.score, w.X, ldx);
             fc_count_launch(); FC_LAUNCH_OK();
-            rc = gemm_relu(L.lin, w.X, ldx, FC_ACT_RELU, nxt, L.Cout, edges, precision, s);
+            GemmArgs g = fc_gemm_linear(L.lin, w.X, ldx, nxt, L.Cout, (int)edges, precision);
+            g.act = FC_ACT_RELU;
+            rc = fc_launch_gemm(g, s);
             if (rc) return rc;
             float* t = cur; cur = nxt; nxt = t;
             ldf = L.Cout;
@@ -535,7 +530,9 @@ int fc_paconv_embed(const fc_embedder* e, const float* pts, float* out, int B, i
         for (int j = 0; j < F.n_layers; ++j) {
             dst = (j == F.n_layers - 1) ? fp_out[lev & 1] : w.fph;
             if (dst == cur) dst = w.X;   // never in place
-            rc = gemm_relu(F.lin[j], cur, ldc, FC_ACT_RELU, dst, F.lin[j].N, pts_tot, precision, s);
+            GemmArgs g = fc_gemm_linear(F.lin[j], cur, ldc, dst, F.lin[j].N, (int)pts_tot, precision);
+            g.act = FC_ACT_RELU;
+            rc = fc_launch_gemm(g, s);
             if (rc) return rc;
             cur = dst; ldc = F.lin[j].N;
         }
@@ -547,7 +544,7 @@ int fc_paconv_embed(const fc_embedder* e, const float* pts, float* out, int B, i
     float* bufA = (known_feat == w.hA) ? w.hB : w.hA;
     rc = fc_run_mlp_hidden(e->out_mlp, in, B * Nc, bufA, w.X, 512, precision, s, &last);
     if (rc) return rc;
-    return gemm_relu(e->out_mlp.out, last, 512, FC_ACT_NONE, out, e->E, (long long)B * Nc, precision, s);
+    return fc_launch_gemm(fc_gemm_linear(e->out_mlp.out, last, 512, out, e->E, B * Nc, precision), s);
 }
 
 // ------------------------------------------------------------------------------------------ op-level C ABI (pointops)

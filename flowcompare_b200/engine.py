@@ -40,6 +40,11 @@ IW_MAX_PASS_ROWS = 1 << 20      # rows (draws x points) of one fc_flow_log_prob_
 GRAD_MAX_PASS_ROWS = 1 << 16    # points of one fc_flow_log_prob_grad pass (11.8 GB of workspace at the shipped widths)
 
 
+def _check_shape(what, name, t, shape):
+    if tuple(t.shape) != tuple(shape):
+        raise _lib.FlowCompareError(f"{what}: {name} must be {list(shape)}, got {list(t.shape)}")
+
+
 def _n_draws(n, what):
     if isinstance(n, bool) or not isinstance(n, (int, np.integer)) or n < 1:
         raise _lib.FlowCompareError(f"{what}: the number of draws must be a positive int, got {n!r}")
@@ -181,25 +186,19 @@ class FlowCompareB200:
         extra_context [B], [B,1] or the repeated [B,N,1] the reference passes; eps [B,N,latent-input_dim]
         optional (default: drawn on the device); eps_cif [L,B,N,cif_latent_dim-latent_dim] likewise, CIF flows only."""
         with torch.cuda.device(self.device):
-            x = _f32c(x[..., :self.d_in], self.device)
+            x, context, Nc, extra, eps, eps_cif = self._flow_inputs("log_prob", x, context, extra_context, eps, eps_cif)
             B, N = x.shape[0], x.shape[1]
-            context, Nc, extra = self._prep_context(context, extra_context, B)
-            eps = self.draw_eps(B, N) if eps is None else _f32c(eps, self.device)
-            assert eps.shape == (B, N, self.D - self.d_in), eps.shape
-            eps_arg = eps if self.D > self.d_in else None      # identity augmenter: no draw
             out = torch.empty((B, N), dtype=torch.float32, device=self.device)
             nbytes = self.lib.fc_flow_workspace_bytes(self._flow["handle"], B, N, Nc)
             ws = self._workspace(nbytes)
             if self.cif_S:
-                eps_cif = self.draw_eps_cif(B, N) if eps_cif is None else _f32c(eps_cif, self.device)
-                assert eps_cif.shape == (self.L, B, N, self.cif_S), eps_cif.shape
                 rc = self.lib.fc_flow_log_prob_cif(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra),
-                                                   _ptr(eps_arg), eps_cif.data_ptr(), out.data_ptr(), B, N, Nc, ws, nbytes,
+                                                   _ptr(eps), eps_cif.data_ptr(), out.data_ptr(), B, N, Nc, ws, nbytes,
                                                    self.precision, _stream())
                 _lib.check(rc, "fc_flow_log_prob_cif")
             else:
                 rc = self.lib.fc_flow_log_prob(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra),
-                                               _ptr(eps_arg), out.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
+                                               _ptr(eps), out.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
                 _lib.check(rc, "fc_flow_log_prob")
         return out
 
@@ -226,15 +225,12 @@ class FlowCompareB200:
             S = self.D - self.d_in
             if eps is not None:
                 eps = _f32c(eps, self.device)
-                if tuple(eps.shape) != (K, B, N, S):
-                    raise _lib.FlowCompareError(f"log_prob_iw: eps must be [{K}, {B}, {N}, {S}], got {list(eps.shape)}")
+                _check_shape("log_prob_iw", "eps", eps, (K, B, N, S))
             if eps_cif is not None:
                 if not self.cif_S:
                     raise _lib.FlowCompareError("log_prob_iw: eps_cif given but this flow has no CIF blocks")
                 eps_cif = _f32c(eps_cif, self.device)
-                if tuple(eps_cif.shape) != (K, self.L, B, N, self.cif_S):
-                    raise _lib.FlowCompareError(f"log_prob_iw: eps_cif must be [{K}, {self.L}, {B}, {N}, {self.cif_S}], "
-                                                f"got {list(eps_cif.shape)}")
+                _check_shape("log_prob_iw", "eps_cif", eps_cif, (K, self.L, B, N, self.cif_S))
             deterministic = S == 0 and not self.cif_S       # every draw is the same log_prob: one pass
             if N > IW_MAX_PASS_ROWS:
                 raise _lib.FlowCompareError(f"log_prob_iw: {N} points per cloud exceed one pass of {IW_MAX_PASS_ROWS} rows")
@@ -307,16 +303,8 @@ class FlowCompareB200:
         result does not depend on the split.  Affine-coupling flows only: spline / exponential couplings and CIF blocks raise."""
         self._ensure_grad()
         with torch.cuda.device(self.device):
-            x = _f32c(x[..., :self.d_in], self.device)
+            x, context, Nc, extra, eps, _ = self._flow_inputs("log_prob_grad", x, context, extra_context, eps, None)
             B, N = x.shape[0], x.shape[1]
-            context, Nc, extra = self._prep_context(context, extra_context, B)
-            S = self.D - self.d_in
-            if eps is None:
-                eps = self.draw_eps(B, N)
-            else:
-                eps = _f32c(eps, self.device)
-                if tuple(eps.shape) != (B, N, S):
-                    raise _lib.FlowCompareError(f"log_prob_grad: eps must be [{B}, {N}, {S}], got {list(eps.shape)}")
             if N > GRAD_MAX_PASS_ROWS:
                 raise _lib.FlowCompareError(f"log_prob_grad: {N} points per cloud exceed one pass of {GRAD_MAX_PASS_ROWS} rows")
             h = self._flow["handle"]
@@ -332,9 +320,9 @@ class FlowCompareB200:
                 nb = b1 - b0
                 nbytes = wsb(nb)
                 ws = self._workspace(nbytes)
-                pe = eps[b0:b1] if S else None
                 rc = self.lib.fc_flow_log_prob_grad(h, x[b0:b1].data_ptr(), context[b0:b1].data_ptr(),
-                                                    _ptr(None if extra is None else extra[b0:b1]), _ptr(pe),
+                                                    _ptr(None if extra is None else extra[b0:b1]),
+                                                    _ptr(None if eps is None else eps[b0:b1]),
                                                     lp[b0:b1].data_ptr(), grad[b0:b1].data_ptr(), nb, N, Nc, ws, nbytes,
                                                     self.precision, _stream())
                 _lib.check(rc, "fc_flow_log_prob_grad")
@@ -356,19 +344,36 @@ class FlowCompareB200:
             extra = _f32c(extra.reshape(B), self.device)
         return context, Nc, extra
 
+    def _eps_cif(self, what, eps_cif, B, N):
+        """The CIF blocks' draws [L, B, N, cif_latent_dim - latent_dim] as given (checked) or drawn; None without CIF blocks."""
+        if not self.cif_S:
+            return None
+        eps_cif = self.draw_eps_cif(B, N) if eps_cif is None else _f32c(eps_cif, self.device)
+        _check_shape(what, "eps_cif", eps_cif, (self.L, B, N, self.cif_S))
+        return eps_cif
+
+    def _flow_inputs(self, what, x, context, extra_context, eps, eps_cif):
+        """What a flow pass over x [B, N, >=input_dim] reads: (x cut to input_dim, context, Nc, extra context, eps, eps_cif).
+        Noise not given is drawn on the device; given noise of the wrong shape raises.  eps is None for an identity augmenter,
+        eps_cif None for a flow without CIF blocks (a given one is then ignored)."""
+        x = _f32c(x[..., :self.d_in], self.device)
+        B, N = x.shape[0], x.shape[1]
+        context, Nc, extra = self._prep_context(context, extra_context, B)
+        eps = self.draw_eps(B, N) if eps is None else _f32c(eps, self.device)
+        _check_shape(what, "eps", eps, (B, N, self.D - self.d_in))
+        return x, context, Nc, extra, eps if self.D > self.d_in else None, self._eps_cif(what, eps_cif, B, N)
+
     def forward(self, x, context, extra_context=None, eps=None):
         """The forward pass with its latent: returns (log_prob [B,N], z [B,N,latent]) -- `Flow.log_prob` plus the point at
         which the base density was evaluated (what `Flow.sample` inverts)."""
         with torch.cuda.device(self.device):
-            x = _f32c(x[..., :self.d_in], self.device)
+            x, context, Nc, extra, eps, _ = self._flow_inputs("forward", x, context, extra_context, eps, None)
             B, N = x.shape[0], x.shape[1]
-            context, Nc, extra = self._prep_context(context, extra_context, B)
-            eps = self.draw_eps(B, N) if eps is None else _f32c(eps, self.device)
             out = torch.empty((B, N), dtype=torch.float32, device=self.device)
             z = torch.empty((B, N, self.D), dtype=torch.float32, device=self.device)
             nbytes = self.lib.fc_flow_workspace_bytes(self._flow["handle"], B, N, Nc)
             ws = self._workspace(nbytes)
-            rc = self.lib.fc_flow_forward(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra), eps.data_ptr(),
+            rc = self.lib.fc_flow_forward(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra), _ptr(eps),
                                           out.data_ptr(), z.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
             _lib.check(rc, "fc_flow_forward")
         return out, z
@@ -400,9 +405,7 @@ class FlowCompareB200:
                                         if unknown else "attention_maps: no layers requested")
         slots = sorted({names.index(n) + first_slot for n in layers})
         with torch.cuda.device(self.device):
-            x = _f32c(x[..., :self.d_in], self.device)
             B, N = x.shape[0], x.shape[1]
-            context, Nc, extra = self._prep_context(context, extra_context, B)
             qidx, n_query = None, N
             if queries is not None:
                 q = torch.as_tensor(queries).reshape(-1)
@@ -410,20 +413,13 @@ class FlowCompareB200:
                     raise _lib.FlowCompareError(f"attention_maps: query indices must be integers in [0, {N})")
                 qidx = q.to(device=self.device, dtype=torch.int32).contiguous()
                 n_query = qidx.numel()
-            eps = self.draw_eps(B, N) if eps is None else _f32c(eps, self.device)
-            assert eps.shape == (B, N, self.D - self.d_in), eps.shape
-            eps_arg = eps if self.D > self.d_in else None
-            if self.cif_S:
-                eps_cif = self.draw_eps_cif(B, N) if eps_cif is None else _f32c(eps_cif, self.device)
-                assert eps_cif.shape == (self.L, B, N, self.cif_S), eps_cif.shape
-            else:
-                eps_cif = None
+            x, context, Nc, extra, eps, eps_cif = self._flow_inputs("attention_maps", x, context, extra_context, eps, eps_cif)
             slots_host = np.asarray(slots, dtype=np.int32)
             maps = torch.empty((len(slots), B, n_query, Nc), dtype=torch.float32, device=self.device)
             out = torch.empty((B, N), dtype=torch.float32, device=self.device)
             nbytes = self.lib.fc_flow_workspace_bytes(self._flow["handle"], B, N, Nc)
             ws = self._workspace(nbytes)
-            rc = self.lib.fc_flow_attention_maps(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra), _ptr(eps_arg),
+            rc = self.lib.fc_flow_attention_maps(self._flow["handle"], x.data_ptr(), context.data_ptr(), _ptr(extra), _ptr(eps),
                                                  _ptr(eps_cif), slots_host.ctypes.data, len(slots), _ptr(qidx), n_query,
                                                  maps.data_ptr(), out.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
             _lib.check(rc, "fc_flow_attention_maps")
@@ -459,9 +455,8 @@ class FlowCompareB200:
             out = torch.empty((B, n_points, self.d_in), dtype=torch.float32, device=self.device)
             nbytes = self.lib.fc_flow_workspace_bytes(self._flow["handle"], B, n_points, Nc)
             ws = self._workspace(nbytes)
+            eps_cif = self._eps_cif("sample", eps_cif, B, n_points)
             if self.cif_S:
-                eps_cif = self.draw_eps_cif(B, n_points) if eps_cif is None else _f32c(eps_cif, self.device)
-                assert eps_cif.shape == (self.L, B, n_points, self.cif_S), eps_cif.shape
                 rc = self.lib.fc_flow_sample_cif(self._flow["handle"], z.data_ptr(), context.data_ptr(), _ptr(extra),
                                                  eps_cif.data_ptr(), out.data_ptr(), B, n_points, Nc, ws, nbytes, self.precision,
                                                  _stream())
