@@ -321,10 +321,11 @@ extern "C" int64_t fc_flow_workspace_bytes(const fc_flow* f, int B, int N, int N
 }
 
 // ------------------------------------------------------------------------------------------ forward
-// Which attention blocks' softmax weights a forward pass writes (fc_flow_attention_maps).  Slot 0 is the augmenter's attention,
-// slot l + 1 coupling layer l's; `slots` strictly increasing; the i-th captured block's maps [B, n_query, Nc] start at
-// out + i * B * n_query * Nc.
-struct FcCapture { const int32_t* slots; int n_slots; const int32_t* qidx; int n_query; float* out; };
+// Which attention blocks' softmax weights a forward pass writes (fc_flow_attention_maps), or whose score gradients the
+// input-gradient pass writes (fc_flow_attention_score_grads).  Slot 0 is the augmenter's attention, slot l + 1 coupling layer
+// l's; `slots` strictly increasing; the i-th captured block's maps [B, n_query, Nc] start at out + i * B * n_query * Nc, or,
+// with `accumulate` (score gradients only), every block adds into the one [B, n_query, Nc] at out.
+struct FcCapture { const int32_t* slots; int n_slots; const int32_t* qidx; int n_query; float* out; bool accumulate; };
 
 // a caller's workspace: 256-byte aligned and at least `need` bytes
 static bool ws_ok(const void* workspace, int64_t need, int64_t workspace_bytes) {
@@ -659,7 +660,7 @@ extern "C" int fc_flow_attention_maps(const fc_flow* f, const float* x, const fl
     for (int i = 0; i < n_slots; ++i)
         FC_REQUIRE(slots_host[i] >= 0 && slots_host[i] <= f->L && (i == 0 || slots_host[i] > slots_host[i - 1]));
     FC_REQUIRE(slots_host[0] != 0 || f->has_aug);     // an identity augmenter has no attention
-    const FcCapture cap{slots_host, n_slots, query_idx, n_query, maps_out};
+    const FcCapture cap{slots_host, n_slots, query_idx, n_query, maps_out, false};
     return flow_forward(f, x, context, extra, eps, eps_cif, log_prob_out, nullptr, B, N, Nc, workspace, workspace_bytes, precision,
                         stream_, &cap);
 }
@@ -923,11 +924,20 @@ static int attn_recompute(const fc_flow* f, const FcMlp& pre, const FcAttn& at, 
     return fc_launch_gemm(fc_gemm_linear(at.kv, context, f->E, gw.fw.kv, 128, B * Nc, precision), s);
 }
 
-// with dL/do in gw.dO: dq, then LayerNorm and the pre-attention MLP backwards; g[:, :pre.in.K1] += dL/d(its input)
+// with dL/do in gw.dO: dq, then LayerNorm and the pre-attention MLP backwards; g[:, :pre.in.K1] += dL/d(its input).
+// sgrad: where this block's score gradients go (nullptr: not captured; `cap` then unused), added to it when sgrad_add.  They are
+// read from q, k|v, o and dO as the dq kernel reads them, before anything else of the block's backward runs.
 static int attn_backward(const fc_flow* f, const FcMlp& pre, const FcGradLayer& gl, int B, int N, int Nc, GradWs& gw, float* g,
-                         int ldg, int precision, cudaStream_t s) {
+                         int ldg, int precision, cudaStream_t s, float* sgrad, bool sgrad_add, const FcCapture* cap) {
     const int M = B * N, ldh = gw.fw.ldh;
-    int rc = fc_launch_attention_dq(gw.fw.q, gw.fw.kv, 128, gw.fw.o, gw.dO, gw.dq, B, N, Nc, 1.0f / sqrtf((float)f->inner), s);
+    const float scale = 1.0f / sqrtf((float)f->inner);
+    int rc;
+    if (sgrad) {
+        rc = fc_launch_attention_score_grad(gw.fw.q, 64, gw.fw.kv, 128, gw.fw.o, 64, gw.dO, 64, cap->qidx, cap->n_query, sgrad,
+                                            sgrad_add ? 1 : 0, B, N, Nc, scale, s);
+        if (rc) return rc;
+    }
+    rc = fc_launch_attention_dq(gw.fw.q, gw.fw.kv, 128, gw.fw.o, gw.dO, gw.dq, B, N, Nc, scale, s);
     if (rc) return rc;
     rc = fc_launch_gemm(fc_gemm_linear(gl.q, gw.dq, 64, gw.dA, ldh, M, precision), s);
     if (rc) return rc;
@@ -944,10 +954,11 @@ static int attn_backward(const fc_flow* f, const FcMlp& pre, const FcGradLayer& 
 }
 
 // One conditioner (a coupling layer's, or the augmenter's with aug = true) backwards.  lat: the block's input (its checkpoint);
-// g: dL/d(block output) on entry, dL/d(block input) on exit.
+// g: dL/d(block output) on entry, dL/d(block input) on exit.  sgrad / sgrad_add / cap: score-gradient capture as in attn_backward.
 static int conditioner_backward(const fc_flow* f, const FcMlp& pre, const FcAttn& at, const FcMlp& net, const FcGradLayer& gl,
                                 bool aug, const float* lat, int cb_slot, const float* context, const float* eps, int B, int N, int Nc,
-                                GradWs& gw, float* g, int precision, cudaStream_t s) {
+                                GradWs& gw, float* g, int precision, cudaStream_t s, float* sgrad, bool sgrad_add,
+                                const FcCapture* cap) {
     const int M = B * N, ldh = gw.fw.ldh, ldx = gw.fw.ldx;
     const bool attn = !f->is_global;
     int rc;
@@ -974,12 +985,14 @@ static int conditioner_backward(const fc_flow* f, const FcMlp& pre, const FcAttn
     if (rc || !attn) return rc;
     rc = fc_launch_gemm(fc_gemm_linear(gl.cpl.in_o, cur, ldh, gw.dO, 64, M, precision), s);
     if (rc) return rc;
-    return attn_backward(f, pre, gl, B, N, Nc, gw, g, ldx, precision, s);
+    return attn_backward(f, pre, gl, B, N, Nc, gw, g, ldx, precision, s, sgrad, sgrad_add, cap);
 }
 
-extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
-                                     float* log_prob_out, float* grad_out, int B, int N, int Nc, void* workspace,
-                                     int64_t workspace_bytes, int precision, fc_stream_t stream_) {
+// cap: the attention blocks whose score gradients are written (fc_flow_attention_score_grads); the walk meets them in
+// decreasing slot order, layers L-1 ... 0 then the augmenter
+static int flow_log_prob_grad(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
+                              float* log_prob_out, float* grad_out, int B, int N, int Nc, void* workspace, int64_t workspace_bytes,
+                              int precision, fc_stream_t stream_, const FcCapture* cap = nullptr) {
     FC_REQUIRE(f && x && context && log_prob_out && grad_out && B > 0 && N > 0 && Nc > 0);
     if (f->cpl_kind != FC_CPL_AFFINE || f->cif_dim) return FC_ERR_UNSUPPORTED;
     if (!f->glayers) return FC_ERR_MODEL;
@@ -997,6 +1010,15 @@ extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const flo
     float* g = gw.gA; float* g_other = gw.gB;
     rc = fc_launch_neg_copy(slot(f->L), ldx, g, ldx, M, f->D, s);
     if (rc) return rc;
+    int n_captured = 0;
+    bool sgrad_add = false;
+    auto sgrad_for = [&](int cslot) -> float* {
+        if (!cap || n_captured >= cap->n_slots || cap->slots[cap->n_slots - 1 - n_captured] != cslot) return nullptr;
+        const size_t i = cap->accumulate ? 0 : (size_t)(cap->n_slots - 1 - n_captured);
+        sgrad_add = cap->accumulate && n_captured > 0;       // the first block met stores, the later ones add
+        ++n_captured;
+        return cap->out + i * (size_t)B * (size_t)cap->n_query * (size_t)Nc;
+    };
     for (int l = f->L - 1; l >= 0; --l) {
         const FcFlowLayer& y = f->layers[l];
         const FcGradLayer& gl = f->glayers[l];
@@ -1006,13 +1028,43 @@ extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const flo
             if (rc) return rc;
             float* t = g; g = g_other; g_other = t;
         }
-        rc = conditioner_backward(f, y.pre, y.attn, y.cpl, gl, false, slot(l), l + 1, context, nullptr, B, N, Nc, gw, g, precision, s);
+        float* sg = sgrad_for(l + 1);
+        rc = conditioner_backward(f, y.pre, y.attn, y.cpl, gl, false, slot(l), l + 1, context, nullptr, B, N, Nc, gw, g, precision, s,
+                                  sg, sgrad_add, cap);
         if (rc) return rc;
     }
     if (f->has_aug) {
+        float* sg = sgrad_for(0);
         rc = conditioner_backward(f, f->augpre, f->augattn, f->aug, f->gaug, true, slot(0), 0, context, eps, B, N, Nc, gw, g,
-                                  precision, s);
+                                  precision, s, sg, sgrad_add, cap);
         if (rc) return rc;
     }
     return copy_cols(g, ldx, grad_out, f->d_in, M, f->d_in, s);
+}
+
+extern "C" int fc_flow_log_prob_grad(const fc_flow* f, const float* x, const float* context, const float* extra, const float* eps,
+                                     float* log_prob_out, float* grad_out, int B, int N, int Nc, void* workspace,
+                                     int64_t workspace_bytes, int precision, fc_stream_t stream_) {
+    return flow_log_prob_grad(f, x, context, extra, eps, log_prob_out, grad_out, B, N, Nc, workspace, workspace_bytes, precision,
+                              stream_);
+}
+
+// The input-gradient pass that also writes d lp_i / d s_ij of the attention blocks listed in slots_host (see FcCapture), read at
+// the start of each captured block's attention backward.  Only reads are added, so log_prob and grad are fc_flow_log_prob_grad's.
+extern "C" int fc_flow_attention_score_grads(const fc_flow* f, const float* x, const float* context, const float* extra,
+                                             const float* eps, const int32_t* slots_host, int n_slots, const int32_t* query_idx,
+                                             int n_query, int accumulate, float* maps_out, float* log_prob_out, float* grad_out,
+                                             int B, int N, int Nc, void* workspace, int64_t workspace_bytes, int precision,
+                                             fc_stream_t stream_) {
+    FC_REQUIRE(f && slots_host && n_slots > 0 && maps_out && n_query > 0);
+    if (f->is_global) return FC_ERR_UNSUPPORTED;       // no attention over context points: the device never runs one
+    if (f->cpl_kind != FC_CPL_AFFINE || f->cif_dim) return FC_ERR_UNSUPPORTED;
+    if (!f->glayers) return FC_ERR_MODEL;
+    FC_REQUIRE(query_idx || n_query == N);
+    for (int i = 0; i < n_slots; ++i)
+        FC_REQUIRE(slots_host[i] >= 0 && slots_host[i] <= f->L && (i == 0 || slots_host[i] > slots_host[i - 1]));
+    FC_REQUIRE(slots_host[0] != 0 || f->has_aug);     // an identity augmenter has no attention
+    const FcCapture cap{slots_host, n_slots, query_idx, n_query, maps_out, accumulate != 0};
+    return flow_log_prob_grad(f, x, context, extra, eps, log_prob_out, grad_out, B, N, Nc, workspace, workspace_bytes, precision,
+                              stream_, &cap);
 }

@@ -192,6 +192,11 @@ int fc_launch_ln_bwd(const float* h, int ldh, const float* mu, const float* rstd
 int fc_launch_neg_copy(const float* z, int ldz, float* g, int ldg, long long M, int cols, cudaStream_t s);
 int fc_launch_attention_dq(const float* q, const float* kv, int ldkv, const float* o, const float* dO, float* dq, int B, int N,
                            int Nc, float scale, cudaStream_t stream);
+// d lp_i / d s_ij = P_ij (dO_i . v_j - dO_i . o_i) of one attention block, [B, n_query, Nc] (attention_score_grad.cu); qidx: device
+// list of query rows or null; accumulate: out += value (one rounded add) instead of out = value
+int fc_launch_attention_score_grad(const float* q, int ldq, const float* kv, int ldkv, const float* o, int ldo, const float* dO,
+                                   int lddo, const int32_t* qidx, int n_query, float* out, int accumulate, int B, int N, int Nc,
+                                   float scale, cudaStream_t stream);
 constexpr int64_t FC_GRAD_MAX_ROWS = 1ll << 16;   // rows of one fc_flow_log_prob_grad pass
 bool fc_gemm_tc_supported(const GemmArgs& a);      // gemm_tc.cu
 

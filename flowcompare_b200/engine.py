@@ -393,26 +393,11 @@ class FlowCompareB200:
         `attention_layer_names` (None: all); `queries`: indices into the N points of x, any order, repeats allowed (None: all).
         Returns (log_prob [B,N], {name: weights [B, n_query, Nc]}); log_prob is bitwise what `log_prob` returns with the same
         eps, and the maps are views of one allocation."""
-        if self.is_global:
-            raise _lib.FlowCompareError("attention_maps: global-embedding configs attend to no context points")
+        slots, first_slot = self._attention_slots("attention_maps", layers)
         names = self.attention_layer_names
-        first_slot = 0 if self.D > self.d_in else 1      # slot 0 is the augmenter's attention (absent for an identity augmenter)
-        if layers is None:
-            layers = names
-        unknown = [n for n in layers if n not in names]
-        if unknown or not layers:
-            raise _lib.FlowCompareError(f"attention_maps: unknown layer names {unknown}; choose from attention_layer_names"
-                                        if unknown else "attention_maps: no layers requested")
-        slots = sorted({names.index(n) + first_slot for n in layers})
         with torch.cuda.device(self.device):
             B, N = x.shape[0], x.shape[1]
-            qidx, n_query = None, N
-            if queries is not None:
-                q = torch.as_tensor(queries).reshape(-1)
-                if q.numel() == 0 or q.is_floating_point() or int(q.min()) < 0 or int(q.max()) >= N:
-                    raise _lib.FlowCompareError(f"attention_maps: query indices must be integers in [0, {N})")
-                qidx = q.to(device=self.device, dtype=torch.int32).contiguous()
-                n_query = qidx.numel()
+            qidx, n_query = self._query_index("attention_maps", queries, N)
             x, context, Nc, extra, eps, eps_cif = self._flow_inputs("attention_maps", x, context, extra_context, eps, eps_cif)
             slots_host = np.asarray(slots, dtype=np.int32)
             maps = torch.empty((len(slots), B, n_query, Nc), dtype=torch.float32, device=self.device)
@@ -424,6 +409,85 @@ class FlowCompareB200:
                                                  maps.data_ptr(), out.data_ptr(), B, N, Nc, ws, nbytes, self.precision, _stream())
             _lib.check(rc, "fc_flow_attention_maps")
         return out, {names[s - first_slot]: maps[i] for i, s in enumerate(slots)}
+
+    def _attention_slots(self, what, layers):
+        """(sorted device slots of the named attention blocks, slot of attention_layer_names[0]); raises for global-embedding
+        configs, unknown names and an empty list."""
+        if self.is_global:
+            raise _lib.FlowCompareError(f"{what}: global-embedding configs attend to no context points")
+        names = self.attention_layer_names
+        first_slot = 0 if self.D > self.d_in else 1      # slot 0 is the augmenter's attention (absent for an identity augmenter)
+        if layers is None:
+            layers = names
+        unknown = [n for n in layers if n not in names]
+        if unknown or not layers:
+            raise _lib.FlowCompareError(f"{what}: unknown layer names {unknown}; choose from attention_layer_names"
+                                        if unknown else f"{what}: no layers requested")
+        return sorted({names.index(n) + first_slot for n in layers}), first_slot
+
+    def _query_index(self, what, queries, N):
+        """(device int32 query rows or None for all, n_query) from indices into the N points of a cloud."""
+        if queries is None:
+            return None, N
+        q = torch.as_tensor(queries).reshape(-1)
+        if q.numel() == 0 or q.is_floating_point() or int(q.min()) < 0 or int(q.max()) >= N:
+            raise _lib.FlowCompareError(f"{what}: query indices must be integers in [0, {N})")
+        qidx = q.to(device=self.device, dtype=torch.int32).contiguous()
+        return qidx, qidx.numel()
+
+    def attention_score_grads(self, x, context, extra_context=None, layers=None, queries=None, eps=None, sum_layers=False,
+                              workspace_budget=None):
+        """Attention score gradients: d log_prob[b, i] / d s_ij for the attention scores s = q k^T / 8 of chosen blocks (reference
+        models/perceiver.py:108-115) -- what `sim.grad` holds on the reference after `sim.retain_grad()` and
+        `flow.log_prob(x, context=...).sum().backward()`, with the augmentation noise eps held fixed.  The signed answer to which
+        context points raise (positive) or lower (negative) a target point's likelihood if its conditioner attended to them more;
+        a row sums to zero.  Formed from the input-gradient pass `log_prob_grad` runs; no gradient flows to the context.
+
+        Arguments as `attention_maps` (`layers` from `attention_layer_names`, None: all; `queries` any order, repeats allowed)
+        and `log_prob_grad` (passes of at most 2^16 points, fewer under `workspace_budget`; the result does not depend on the
+        split).  Returns (log_prob [B,N], grad [B,N,input_dim], maps): log_prob and grad bitwise `log_prob_grad`'s, maps
+        {name: [B, n_query, Nc]}, or with `sum_layers` one [B, n_query, Nc] tensor, the sum over the selected blocks (the
+        gradient with respect to a logit bias they all share; one block's memory for any number of blocks), added in fp32 in the
+        order of the backward walk: the last coupling layer's block first, the augmenter's last.  Affine-coupling flows only."""
+        slots, first_slot = self._attention_slots("attention_score_grads", layers)
+        names = self.attention_layer_names
+        with torch.cuda.device(self.device):
+            B, N = x.shape[0], x.shape[1]
+            qidx, n_query = self._query_index("attention_score_grads", queries, N)
+            self._ensure_grad()
+            x, context, Nc, extra, eps, _ = self._flow_inputs("attention_score_grads", x, context, extra_context, eps, None)
+            if N > GRAD_MAX_PASS_ROWS:
+                raise _lib.FlowCompareError(f"attention_score_grads: {N} points per cloud exceed one pass of {GRAD_MAX_PASS_ROWS} rows")
+            h = self._flow["handle"]
+            wsb = lambda bc: self.lib.fc_flow_log_prob_grad_workspace_bytes(h, bc, N, Nc)
+            bc = min(B, GRAD_MAX_PASS_ROWS // N)                              # clouds per pass
+            if workspace_budget is not None:
+                while bc > 1 and wsb(bc) > workspace_budget:
+                    bc = (bc + 1) // 2
+            slots_host = np.asarray(slots, dtype=np.int32)
+            lp = torch.empty((B, N), dtype=torch.float32, device=self.device)
+            grad = torch.empty((B, N, self.d_in), dtype=torch.float32, device=self.device)
+            shape = (B, n_query, Nc) if sum_layers else (len(slots), B, n_query, Nc)
+            maps = torch.empty(shape, dtype=torch.float32, device=self.device)
+            for b0 in range(0, B, bc):
+                b1 = min(B, b0 + bc)
+                nb = b1 - b0
+                dst = maps[b0:b1] if sum_layers else maps[:, b0:b1]
+                out = dst if dst.is_contiguous() else torch.empty(dst.shape, dtype=torch.float32, device=self.device)
+                nbytes = wsb(nb)
+                ws = self._workspace(nbytes)
+                rc = self.lib.fc_flow_attention_score_grads(h, x[b0:b1].data_ptr(), context[b0:b1].data_ptr(),
+                                                            _ptr(None if extra is None else extra[b0:b1]),
+                                                            _ptr(None if eps is None else eps[b0:b1]), slots_host.ctypes.data,
+                                                            len(slots), _ptr(qidx), n_query, 1 if sum_layers else 0,
+                                                            out.data_ptr(), lp[b0:b1].data_ptr(), grad[b0:b1].data_ptr(), nb, N,
+                                                            Nc, ws, nbytes, self.precision, _stream())
+                _lib.check(rc, "fc_flow_attention_score_grads")
+                if out is not dst:
+                    dst.copy_(out)
+        if sum_layers:
+            return lp, grad, maps
+        return lp, grad, {names[s - first_slot]: maps[i] for i, s in enumerate(slots)}
 
     # ------------------------------------------------------------------ inverse / sampling pass
     def _ensure_inverse(self):

@@ -48,6 +48,8 @@ SIGNATURES = {
     "fc_cross_attention_tc": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, c_i64, c_vp]),
     "fc_cross_attention_tc_f16": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_int, c_int, c_f, c_vp, c_i64, c_vp]),
     "fc_attention_maps": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int, c_f, c_vp]),
+    "fc_attention_score_grad": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_vp, c_int, c_int, c_int,
+                                        c_int, c_f, c_vp]),
     "fc_fps_points": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_int, c_vp]),
     "fc_co_unit_sphere": (c_int, [c_vp, c_int, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp]),
     "fc_flow_create": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_i64, ctypes.POINTER(c_vp)]),
@@ -71,6 +73,8 @@ SIGNATURES = {
     "fc_flow_set_grad": (c_int, [c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_i64]),
     "fc_flow_log_prob_grad_workspace_bytes": (c_i64, [c_vp, c_int, c_int, c_int]),
     "fc_flow_log_prob_grad": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_int, c_vp]),
+    "fc_flow_attention_score_grads": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int,
+                                              c_int, c_int, c_vp, c_i64, c_int, c_vp]),
     "fc_embedder_create": (c_int, [c_vp, c_int, c_vp, c_int, c_vp, c_i64, ctypes.POINTER(c_vp)]),
     "fc_embedder_destroy": (None, [c_vp]),
     "fc_embedder_workspace_bytes": (c_i64, [c_vp, c_int, c_int]),

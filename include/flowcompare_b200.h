@@ -184,6 +184,16 @@ FC_API int fc_cross_attention_tc_f16(const float* q, int ldq, const float* kv, i
 FC_API int fc_attention_maps(const float* q, int ldq, const float* kv, int ldkv, const int32_t* query_idx, int n_query,
                       float* out, int B, int N, int Nc, float scale, fc_stream_t stream);
 
+/* The gradient of each query row's scalar with respect to its attention scores s = q k^T * scale, given dO = d(scalar) / d o for
+ * the attention output o = softmax(s) v:  out[b, r, j] = P_ij (dO_i . v_j - D_i), D_i = dO_i . o_i, i = query_idx[r] (q, o and
+ * dO rows b*N + i; query_idx as in fc_attention_maps, or NULL with n_query == N).  kv: k | v, [B*Nc, >= 128].  accumulate != 0:
+ * out[b, r, j] += value with one rounded fp32 add.  Exact fp32, each dot product a sequential fma chain over d = 64: every value is
+ * deterministic and independent of the batch and of the query list.  A NaN in q, dO, o or a key k_j gives NaN rows.  The kernel
+ * fc_flow_attention_score_grads runs per captured block.                                                                  */
+FC_API int fc_attention_score_grad(const float* q, int ldq, const float* kv, int ldkv, const float* o, int ldo, const float* dO,
+                            int lddo, const int32_t* query_idx, int n_query, float* out, int accumulate, int B, int N, int Nc,
+                            float scale, fc_stream_t stream);
+
 /* ------------------------------------------------------------------ data-side ops ----------
  * What the reference's loader does between reading a voxel and calling `inner_loop` (SURVEY.md 8f rank 4).
  * fc_fps_points replaces `voxel[fps(voxel, batch, ratio=n_samples/len(voxel), random_start=False)][:n_samples]`
@@ -333,6 +343,24 @@ FC_API int64_t fc_flow_log_prob_grad_workspace_bytes(const fc_flow* h, int B, in
 FC_API int fc_flow_log_prob_grad(const fc_flow* h, const float* x, const float* context, const float* extra, const float* eps,
                           float* log_prob_out, float* grad_out, int B, int N, int Nc, void* workspace,
                           int64_t workspace_bytes, int precision, fc_stream_t stream);
+
+/* Attention score gradients: the same input-gradient pass, additionally writing d log_prob[b, i] / d s_ij for chosen attention
+ * blocks, s = q k^T * 64^-1/2 the scores of reference models/perceiver.py:108-115 -- what `sim.grad` holds there after
+ * `sim.retain_grad()` and `flow.log_prob(...).sum().backward()` (a point's log-prob depends on its own query row only).  Positive:
+ * attending more to context point j would raise point i's log-likelihood.  Each block's values are formed from the q, k, v, o and
+ * dL/do the backward pass already holds; nothing new is differentiated (no gradient flows to the context).
+ *   slots_host, n_slots, query_idx, n_query: as fc_flow_attention_maps (slot 0 the augmenter's attention, slot l+1 coupling
+ *   layer l's).  maps_out [n_slots, B, n_query, Nc], or with accumulate != 0 the one [B, n_query, Nc] sum over the listed blocks
+ *   (the first block the backward walk meets -- layers L-1 ... 0, then the augmenter -- stores, the later ones add in that order):
+ *   the gradient with respect to a logit bias those blocks share.  The rest as fc_flow_log_prob_grad; log_prob_out and grad_out are
+ *   bitwise what it returns, and fc_flow_log_prob_grad_workspace_bytes(h, B, N, Nc) sizes the workspace.
+ * FC_ERR_UNSUPPORTED for global-embedding flows and the flows fc_flow_log_prob_grad rejects; FC_ERR_MODEL before
+ * fc_flow_set_grad; FC_ERR_INVALID_ARG for slot 0 of a flow with an identity augmenter, unsorted or out-of-range slots, or
+ * query_idx == NULL with n_query != N; FC_ERR_WORKSPACE as usual.                                                        */
+FC_API int fc_flow_attention_score_grads(const fc_flow* h, const float* x, const float* context, const float* extra,
+                                  const float* eps, const int32_t* slots_host, int n_slots, const int32_t* query_idx, int n_query,
+                                  int accumulate, float* maps_out, float* log_prob_out, float* grad_out, int B, int N, int Nc,
+                                  void* workspace, int64_t workspace_bytes, int precision, fc_stream_t stream);
 
 FC_API int fc_embedder_create(const int32_t* header_host, int n_header, const int64_t* table_host, int n_table,
                        const float* arena, int64_t arena_floats, fc_embedder** out);
