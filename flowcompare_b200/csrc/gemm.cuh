@@ -1,7 +1,6 @@
 // fp32 GEMM with fused epilogues -- the contraction workhorse of the path
 // (reference: every nn.Linear / 1x1 conv on the path, SURVEY.md 2.2 F3-F8).
 #pragma once
-#include <cstdlib>
 #include "common.cuh"
 
 enum { FC_ACT_NONE = 0, FC_ACT_GELU = 1, FC_ACT_LRELU = 2, FC_ACT_RELU = 3 };
@@ -52,13 +51,7 @@ struct GemmArgs {
 
 // tcgen05 tiling of the N dimension: n_tiles = ceil(N/96), BN = ceil(N/n_tiles) rounded up to 16.
 // BN <= 96: two double-buffered accumulators (main + compensation) take 384 of the 512 TMEM columns, the A operand the rest.
-// (FC_TC_BNMAX=64|80: A/B knob; any value <= 96 reads the same packed weights, rows are indexed by output column)
-static inline int fc_tc_bnmax() {
-    static int v = 0;
-    if (!v) { const char* e = getenv("FC_TC_BNMAX"); v = e ? atoi(e) : 96; if (v < 16 || v > 96 || (v & 15)) v = 96; }
-    return v;
-}
-static inline int fc_tc_n_tiles(int N) { const int m = fc_tc_bnmax(); return (N + m - 1) / m; }
+static inline int fc_tc_n_tiles(int N) { return (N + 95) / 96; }
 static inline int fc_tc_bn(int N) { const int t = fc_tc_n_tiles(N); return fc_round_up((N + t - 1) / t, 16); }
 static inline int fc_tc_kpad(int K) { return fc_round_up(K, 32); }
 

@@ -14,26 +14,27 @@
 // of the magnitude), and the one GEMM whose output is the latent itself (ActNorm+LinearLU) applies its
 // diagonal in fp32 in the epilogue (flow.cu), so the residual bias is below the fp32 noise of the reference.
 //
-// PERSISTENT kernel, one CTA per SM (14 warps, all 512 TMEM columns, ~225 KB of shared memory).  The CTA walks the
+// PERSISTENT kernel, one CTA per SM (18 warps, all 512 TMEM columns, ~225 KB of shared memory).  The CTA walks the
 // list of 128 x BN output tiles (BN <= 96; N is cut into equal-ish multiples of 16, no padded columns) with stride
 // gridDim.x.  The accumulators are DOUBLE BUFFERED in TMEM, so the epilogue of tile j runs while the tensor core is
 // on tile j+1, and the TMA / converter / MMA pipelines never drain between tiles:
-//   warp 0       TMA producer (one lane): 5 shared-memory stages of (A raw 16 KB, Whi, Wlo)
+//   warp 0       TMA producer (one lane): 5 (3xTF32) or 6 (3xFP16) shared-memory stages of (A raw 16 KB, Whi, Wlo)
 //   warp 1       TMEM allocator + MMA issuer (whole warp loops, one elected lane issues).  Issue is effectively
 //                synchronous (the tensor queue is a couple of MMAs deep), so the warp PROBES the next stage's barriers
 //                before it blocks in the issue and skips the wait when they have fired.  ONE issuer, in program
 //                order: the accumulation order, and with it every output bit, is the same on every run (two issuer
 //                warps sharing a k-block were 3-5 % faster on single GEMMs, equal on the whole step, and measurably
 //                non-deterministic; one warp per accumulator was deterministic but 5 % slower).
-//   warps 2-5    converters (one thread per tile row): fp32 smem row -> TF32 hi/lo -> tcgen05.st, published one half
-//                k-block late so the store latency overlaps the next split
-//   warps 6-13   epilogue (two warps per TMEM lane quadrant, alternate 16-column chunks): bias row prefetched while the
+//   warps 2-9    converters (two threads per tile row): fp32 smem row -> hi/lo -> tcgen05.st, published one step late
+//                so the store latency overlaps the next split.  3xFP16: warps 2-5 take the even k-blocks, 6-9 the odd
+//                ones (a thread converts its whole row); 3xTF32: each thread converts its half of every k-block
+//   warps 10-17  epilogue (two warps per TMEM lane quadrant, alternate 16-column chunks): bias row prefetched while the
 //                tile is still being accumulated; global traffic staged per warp through shared memory (16-byte
 //                coalesced accesses)
 // TMEM (512 columns): accumulator buffer b = [192b, 192b+96) main | [192b+96, 192b+192) compensation;
-//                     [384,512) four stages of A, each HALF a k-block: 16 columns hi + 16 columns lo.
-// Pipeline (mbarriers): full[s] (TMA bytes landed) -> converter -> a_free[s] (A smem reusable) and conv[ts] (A half
-//   block in TMEM) -> MMA -> tcgen05.commit -> tfree[ts], w_free[s], acc_full[b] -> epilogue -> acc_free[b].
+//                     [384,512) the A operand, in stages of HALF a k-block: hi columns then lo columns.
+// Pipeline (mbarriers): full[s] (TMA bytes landed) -> converter -> conv[ts] (A k-block in TMEM) -> MMA ->
+//   tcgen05.commit -> tfree[ts], w_free[s] (stage reusable), acc_full[b] -> epilogue -> acc_free[b].
 // Measured on the way here (B200; numbers in DESIGN.md section 4): two CTAs per SM with single-buffered accumulators
 // (the previous design: 372 -> 390 pairs/s going persistent), the barrier probe (+6 %), a branch-free GELU, hand TF32
 // rounding and 16-byte staged stores (+23 %); dropped: a 4-accumulator split of the main product (no accuracy gain),
@@ -44,7 +45,6 @@
 #include "tcgen05.cuh"
 #include <cuda.h>
 #include <cstdio>
-#include <cstdlib>
 #include <atomic>
 #include <mutex>
 #include <unordered_map>
@@ -54,94 +54,13 @@ namespace {
 constexpr int TC_BM = 128;
 constexpr int TC_BK = 32;                      // 32 fp32 = one 128-byte swizzle row
 constexpr int TC_STAGES = 5;                   // shared-memory stages: a load is issued 4 k-blocks of tensor time (~1.4 us) ahead
-#ifndef TC_BN_CAP
-#define TC_BN_CAP 96                           // widest tile (accumulator width); 80 leaves room for 6 A stages (measured slower)
-#endif
-#ifndef TC_HINT_EPI
-#define TC_HINT_EPI 0                          // suspend-time hints (ns) of the epilogue's accumulator wait / the converters' waits
-#endif
-#ifndef TC_HINT_CONV
-#define TC_HINT_CONV 0
-#endif
-#ifndef TC_EARLY_ACC_FREE
-#define TC_EARLY_ACC_FREE 0                    // 1: accumulator buffer released after a warp's last tcgen05.ld of the tile (measured: no gain, 516.7 vs 517.6 pairs/s)
-#endif
-#ifndef TC_CONV_FLAGS
-#define TC_CONV_FLAGS 0                        // 3xFP16 parity converters publish a k-block through shared-memory sequence flags (st.release /
-#endif                                         // ld.acquire, ~30 cycles a poll) instead of the conv[] mbarrier (~100 cycles per wait even when complete)
-#ifndef TC_FUSE_WLO
-#define TC_FUSE_WLO 1                          // 3xFP16: Ahi.Whi and Ahi.Wlo as one MMA of N = 96 + tile_bn over the adjacent [Whi; Wlo] boxes
-#endif
-#ifndef TC_RES_PREFETCH
-#define TC_RES_PREFETCH 1                      // 3xFP16 mode: the residual of an epilogue chunk arrives by cp.async one chunk ahead (the first
-#endif                                         // chunk's before the accumulator wait) in a second per-warp staging tile; costs one pipeline stage
-#ifndef TC_STAGES_F16
-#define TC_STAGES_F16 (TC_RES_PREFETCH ? 6 : 7)                        // 3xFP16 mode: a stage is 16 KB of A + 2 x 6 KB of W, tensor time per k-block is halved
-#endif
-// Knock-out switches for bottleneck hunting (scripts/build_variant.sh ... "-DTC_KO_MMA=1"): the pipeline keeps its shape and
-// barrier traffic, one stage of work is skipped; the RESULTS ARE GARBAGE, only the timing is meaningful.
-#ifndef TC_KO_MMA
-#define TC_KO_MMA 0     // no tcgen05.mma (commits stay)
-#endif
-#ifndef TC_KO_CONV
-#define TC_KO_CONV 0    // converters neither read shared memory nor write tensor memory
-#endif
-#ifndef TC_KO_WTMA
-#define TC_KO_WTMA 0    // no weight loads
-#endif
-#ifndef TC_KO_ATMA
-#define TC_KO_ATMA 0    // no activation loads
-#endif
-#ifndef TC_KO_EPI
-#define TC_KO_EPI 0     // epilogue reads the accumulators but touches no global memory
-#endif
-#ifndef TC_CPL_STAGED
-#define TC_CPL_STAGED 1 // coupling epilogue: latent chunk through the staging tile (coalesced global accesses)
-#endif
-#ifndef TC_KO_CPLMEM
-#define TC_KO_CPLMEM 0  // coupling epilogue: no latent load / store (math stays)
-#endif
-#ifndef TC_KO_CPLMATH
-#define TC_KO_CPLMATH 0 // coupling epilogue: no exp / log (memory traffic stays)
-#endif
-#ifndef TC_ISSUE_KBLOCK
-#define TC_ISSUE_KBLOCK 1                      // MMA issuer: one synchronisation point per k-block (0: per half k-block)
-#endif
-#ifndef TC_CONV_WARPS
-#define TC_CONV_WARPS 8                        // 4: one converter thread per tile row; 8: two (one per half k-block; measured +10 % in 3xFP16 mode)
-#endif
-#ifndef TC_WARP_ARRIVE
-#define TC_WARP_ARRIVE 0                       // (measured: no gain, 437 vs 441 pairs/s) converter / epilogue warps arrive on their mbarriers ONCE PER WARP (lane 0 after a
-#endif                                         // __syncwarp) instead of once per thread: 8 arrivals per barrier phase instead of 256
-#ifndef TC_CONV_PARITY
-#define TC_CONV_PARITY 1                       // 3xFP16 mode, 8 converter warps: warps 2-5 convert the even k-blocks, 6-9 the odd ones
-#endif                                         // (whole rows), so TWO k-blocks are in conversion at any time
-#ifndef TC_NO_AFREE
-#define TC_NO_AFREE 1                          // the TMA producer waits on w_free[] only: MMAs that have retired imply that the
-#endif                                         // converters finished reading the stage's activation tile long before
-#ifndef TC_SPLIT_ISSUE
-#define TC_SPLIT_ISSUE 0                       // 1: two MMA issuer warps, one per ACCUMULATOR (warp 1 the main product Ahi Whi, warp 2 the
-#endif                                         // two compensation products; each accumulator keeps ONE issuer in program order, so the
-                                               // bits stay reproducible).  Measured equal to one issuer (146.2 vs 145.4 us at
-                                               // M=65536 N=K=512): the issuer is not what paces the k-block, see DESIGN.md section 4
-#ifndef TC_PROBE
-#define TC_PROBE 1                             // issuer probes the next k-block's barrier before it blocks in the issue
-#endif
-constexpr int TC_CONV_WARPS_N = TC_CONV_WARPS;
-static_assert(TC_CONV_WARPS_N == 4 || TC_CONV_WARPS_N == 8, "converter warps: 4 or 8");
-#ifndef TC_PINGPONG
-#define TC_PINGPONG 0                          // 1: two MMA issuer warps that take turns on K-BLOCKS, ordered by a hand-off barrier.
-#endif                                         // Bitwise reproducible (tested) and 12 % faster with loads / conversion / epilogue knocked out
-                                               // (499 vs 569 cycles per k-block), but equal in the real kernel (145.2 vs 145.6 us): the
-                                               // k-block is paced by the TMA -> converter -> MMA -> commit latency chain (DESIGN.md 4)
-#ifndef TC_PP_FENCE
-#define TC_PP_FENCE 1                          // tcgen05 fences around the hand-off (the PTX memory model's ordering of the two issuers' MMAs)
-#endif
-static_assert(!(TC_PINGPONG && TC_SPLIT_ISSUE), "one issuer scheme at a time");
-constexpr int TC_MMA_WARPS = (TC_SPLIT_ISSUE || TC_PINGPONG) ? 2 : 1;
-constexpr int TC_CONV_WARP0 = 1 + TC_MMA_WARPS;               // first converter warp (any 4 consecutive warps cover the 4 TMEM lane quadrants)
-constexpr int TC_EPI_WARP0 = TC_CONV_WARP0 + TC_CONV_WARPS_N; // first epilogue warp
-constexpr int TC_THREADS = 32 * (TC_EPI_WARP0 + 8);           // TMA, MMA issuer(s), converter warps, 8 epilogue warps
+constexpr int TC_STAGES_F16 = 6;               // 3xFP16: a stage is 16 KB of A + 2 x 6 KB of W, tensor time per k-block is halved;
+                                               // 7 fit, 6 leave room for the epilogue's residual prefetch tiles
+constexpr int TC_BN_CAP = 96;                  // widest tile (accumulator width); 80 leaves room for 6 A stages (measured slower)
+constexpr int TC_CONV_WARPS = 8;               // two converter threads per tile row (measured +10 % in 3xFP16 mode over one)
+constexpr int TC_CONV_WARP0 = 2;               // first converter warp (any 4 consecutive warps cover the 4 TMEM lane quadrants)
+constexpr int TC_EPI_WARP0 = TC_CONV_WARP0 + TC_CONV_WARPS;   // first epilogue warp
+constexpr int TC_THREADS = 32 * (TC_EPI_WARP0 + 8);           // TMA, MMA issuer, converter warps, 8 epilogue warps
 // Per operand format: F16 = false 3xTF32 (weights as fp32 TF32 hi/lo), true 3xFP16 (weights as fp16 hi / 2^11-scaled lo)
 template <bool F16> struct TcCfg {
     static constexpr int STAGES = F16 ? TC_STAGES_F16 : TC_STAGES;
@@ -149,19 +68,12 @@ template <bool F16> struct TcCfg {
     static constexpr int TS_COLS = F16 ? 16 : 32;                     // TMEM columns of one A stage (HALF a k-block: hi | lo)
     static constexpr int TSTAGES = (512 - 4 * TC_BN_CAP) / TS_COLS;   // TMEM stages of the A operand
     // stages x (16 KB A + Whi + Wlo at BN = 96) + 8 staging tiles of the epilogue + 1 KB alignment slack
-    static constexpr bool RES_PF = F16 && TC_RES_PREFETCH;            // residual prefetch (two 2 KB swizzled tiles per epilogue warp)
-    static constexpr int STG_FLOATS = RES_PF ? 1024 : 32 * 20;        // per-warp staging floats
+    // 3xFP16 mode: the residual of an epilogue chunk arrives by cp.async one chunk ahead (the first chunk's before the
+    // accumulator wait) in a second per-warp staging tile (two 2 KB swizzled tiles per epilogue warp)
+    static constexpr bool RES_PF = F16;
+    static constexpr int STG_FLOATS = F16 ? 1024 : 32 * 20;           // per-warp staging floats
     static constexpr int SMEM_BYTES = STAGES * (TC_BM * TC_BK * 4 + 2 * 96 * TC_BK * W_ELT) + 8 * STG_FLOATS * 4 + 1024;
 };
-// phase timers (scripts/tc_phases.py): compiled out by default, build a variant with -DTC_PHASE_TIMERS=1
-#ifndef TC_PHASE_TIMERS
-#define TC_PHASE_TIMERS 0
-#endif
-#if TC_PHASE_TIMERS
-#define TC_CLOCK() clock64()
-#else
-#define TC_CLOCK() 0ll
-#endif
 constexpr int TC_A_BYTES = TC_BM * TC_BK * 4;  // 16 KB
 constexpr int TC_TMEM_COLS = 512;                // one persistent CTA per SM
 constexpr int TC_COL_ACC = 2 * TC_BN_CAP;      // accumulator buffer b: main at 192*b, compensation at 192*b + 96
@@ -173,21 +85,8 @@ struct TcParams {
     int BN;        // widest N tile of the launch (multiple of 16, <= TC_BN_CAP = 96)
     int T1, T2;    // k-blocks of segment 1 / 2
     int n_tiles, m_tiles;
-    int pdl;       // launched with programmatic stream serialization
     int tma_store; // STORE / LNQ epilogues: full 32 x 16 chunks leave through TMA stores (mapC) instead of per-thread stores
 };
-
-// phase counters (a -DTC_PHASE_TIMERS=1 build, scripts/tc_phases.py): per CTA, cycles
-//  [0] CTAs  [1] MMA warp total  [2] MMA waits on full[]  [3] on conv[]  [4] on acc_free[]
-//  [5] converter total  [6] converter waits on full[]  [7] on tfree[]  [8] epilogue total  [9] epilogue waits on acc_full[]
-__device__ unsigned long long fc_tc_dbg[16];
-#if TC_PHASE_TIMERS
-#define TC_T(v) const long long v = clock64()
-#define TC_ACC(dst, a, b) dst += (b) - (a)
-#else
-#define TC_T(v) const int v = 0
-#define TC_ACC(dst, a, b) (void)0
-#endif
 
 // ----------------------------------------------------------------------------- kernel
 // One instantiation per (epilogue kind, activation, residual): with every variant inlined behind runtime branches the
@@ -203,12 +102,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                const __grid_constant__ CUtensorMap mapWhi, const __grid_constant__ CUtensorMap mapWlo,
                const __grid_constant__ CUtensorMap mapC, const TcParams p) {
     constexpr int TC_STAGES = TcCfg<F16>::STAGES, TC_TSTAGES = TcCfg<F16>::TSTAGES, TS_COLS = TcCfg<F16>::TS_COLS;   // shadow the globals
-    constexpr bool PARITY = F16 && TC_CONV_PARITY && TC_CONV_WARPS_N == 8;
+    constexpr bool PARITY = F16;   // 3xFP16: the converter groups take turns on k-blocks
     extern __shared__ unsigned char smem_raw[];
-    __shared__ __align__(8) uint64_t bars[3 * TC_STAGES + 2 * TC_TSTAGES + 4];
-    __shared__ __align__(8) uint64_t turn_bar;   // ping-pong issuers: phase g completes when k-block g has been issued
+    __shared__ __align__(8) uint64_t bars[2 * TC_STAGES + 2 * TC_TSTAGES + 4];
     __shared__ uint32_t tmem_base_slot;
-    __shared__ __align__(16) uint32_t conv_flag[8][4];   // [TMEM A stage][converter warp of the group]: use count of the stage
     __shared__ float ldj_sm[2][TC_BM];        // by tile parity: the only barrier between the two halves is the one inside a tile
     // the bias (and LayerNorm-q column sums) of the columns each epilogue warp handles in the current tile: chunk i of the warp
     // (columns half*16 + 32*i ..+15 of the tile) at [16*i ..+15].  Per warp, so the epilogue needs no CTA-wide barrier.
@@ -220,28 +117,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
     const int BN = p.BN;                    // widest tile of this launch: shared-memory layout and TMA box
     const int w_box_bytes = BN * TC_BK * TcCfg<F16>::W_ELT;          // what one weight TMA box brings
     // 3xFP16: the Wlo box always sits 96 rows behind the Whi box (rows BN..95 of the slot are never written: they only feed
-    // accumulator columns nobody reads), so that one MMA can run over [Whi; Wlo] whatever BN is (TC_FUSE_WLO)
-    const int w_bytes = (F16 && TC_FUSE_WLO) ? TC_BN_CAP * TC_BK * TcCfg<F16>::W_ELT : w_box_bytes;
+    // accumulator columns nobody reads), so that one MMA can run over [Whi; Wlo] whatever BN is
+    const int w_bytes = F16 ? TC_BN_CAP * TC_BK * TcCfg<F16>::W_ELT : w_box_bytes;
     const int stage_bytes = TC_A_BYTES + 2 * w_bytes;
     auto a_raw = [&](int s) { return smem + s * stage_bytes; };
     auto w_hi = [&](int s) { return smem + s * stage_bytes + TC_A_BYTES; };
     auto w_lo = [&](int s) { return smem + s * stage_bytes + TC_A_BYTES + w_bytes; };
     float* stage_out = reinterpret_cast<float*>(smem + TC_STAGES * stage_bytes);   // 8 warps x [32][20] staging tiles
     uint64_t* full = bars;                                   // [TC_STAGES]  TMA bytes landed
-    uint64_t* a_free = bars + TC_STAGES;                     // [TC_STAGES]  converters done reading A smem
-    uint64_t* w_free = bars + 2 * TC_STAGES;                 // [TC_STAGES]  MMAs done reading W smem
-    uint64_t* conv = bars + 3 * TC_STAGES;                   // [TC_TSTAGES] A hi/lo written to TMEM
-    uint64_t* tfree = bars + 3 * TC_STAGES + TC_TSTAGES;     // [TC_TSTAGES] MMAs done reading A TMEM
-    uint64_t* acc_full = bars + 3 * TC_STAGES + 2 * TC_TSTAGES;   // [2] accumulators of a tile complete
+    uint64_t* w_free = bars + TC_STAGES;                     // [TC_STAGES]  MMAs done reading the stage (A and W smem)
+    uint64_t* conv = bars + 2 * TC_STAGES;                   // [TC_TSTAGES] A hi/lo written to TMEM
+    uint64_t* tfree = bars + 2 * TC_STAGES + TC_TSTAGES;     // [TC_TSTAGES] MMAs done reading A TMEM
+    uint64_t* acc_full = bars + 2 * TC_STAGES + 2 * TC_TSTAGES;   // [2] accumulators of a tile complete
     uint64_t* acc_free = acc_full + 2;                            // [2] epilogue has drained them (256 arrivals)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // One arrival per warp: every lane has finished (and fenced) its part, __syncwarp orders the lanes, lane 0 arrives with
-    // release semantics for all of them.  256 per-thread arrivals on one mbarrier serialise in the shared-memory atomic unit.
-    auto warp_arrive = [&](uint64_t* bar) {
-        if (TC_WARP_ARRIVE) { __syncwarp(); if (lane == 0) mbar_arrive(bar); }
-        else mbar_arrive(bar);
-    };
     const int T = p.T1 + p.T2;
     const int n_tiles = p.n_tiles, total_tiles = p.n_tiles * p.m_tiles;
     // N is cut into n_tiles tiles whose widths are multiples of 16 and differ by at most 16 (512 -> 96,96,80,80,80,80):
@@ -250,15 +140,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
     auto tile_n0_of = [&](int nt) { return 16 * (nt * n_base + min(nt, n_rem)); };
     auto tile_bn_of = [&](int nt) { return 16 * (n_base + (nt < n_rem ? 1 : 0)); };
 
-    constexpr bool CFLAGS = PARITY && TC_CONV_FLAGS && !TC_SPLIT_ISSUE && !TC_PINGPONG && TC_ISSUE_KBLOCK == 1;
-    if (threadIdx.x < 32) conv_flag[threadIdx.x >> 2][threadIdx.x & 3] = 0u;
     if (threadIdx.x == 0) {
-        constexpr int PER_WARP = TC_WARP_ARRIVE ? 1 : 32;   // arrivals a warp contributes per event
         constexpr int CONV_GROUPS = PARITY ? 2 : 1;         // converter groups that take turns on k-blocks
-        for (int s = 0; s < TC_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&a_free[s], PER_WARP * TC_CONV_WARPS_N / CONV_GROUPS); mbar_init(&w_free[s], TC_SPLIT_ISSUE ? 2 : 1); }
-        for (int s = 0; s < TC_TSTAGES / 2; ++s) { mbar_init(&conv[s], PER_WARP * 8 / CONV_GROUPS); mbar_init(&tfree[s], TC_SPLIT_ISSUE ? 2 : 1); }   // one pair per K-BLOCK of A in tensor memory
-        for (int s = 0; s < 2; ++s) { mbar_init(&acc_full[s], TC_MMA_WARPS); mbar_init(&acc_free[s], PER_WARP * 8); }
-        mbar_init(&turn_bar, 1);
+        for (int s = 0; s < TC_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&w_free[s], 1); }
+        for (int s = 0; s < TC_TSTAGES / 2; ++s) { mbar_init(&conv[s], 32 * 8 / CONV_GROUPS); mbar_init(&tfree[s], 1); }   // one pair per K-BLOCK of A in tensor memory
+        for (int s = 0; s < 2; ++s) { mbar_init(&acc_full[s], 1); mbar_init(&acc_free[s], 32 * 8); }   // one arrival per thread
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -269,13 +155,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = tmem_base_slot;
-    // Programmatic dependent launch: everything above (barrier init, TMEM allocation) may run while the previous kernel
-    // of the stream is still draining; let the NEXT kernel do the same, and touch no global memory before the
-    // previous kernel has completed and flushed.
-    if (p.pdl) {
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-    }
 
     if (warp == 0) {
         // ===================================================== TMA producer
@@ -287,121 +166,33 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                 for (int t = 0; t < T; ++t, ++g) {
                     const int s = g % TC_STAGES;
                     const uint32_t ph = (g / TC_STAGES) & 1;
-                    if (!TC_NO_AFREE) mbar_wait(&a_free[s], ph ^ 1, 100 + t);
+                    // the stage is free once its MMAs have retired: they imply that the converters finished reading its
+                    // activation tile long before
                     mbar_wait(&w_free[s], ph ^ 1, 150 + t);
-                    mbar_expect_tx(&full[s], (uint32_t)((TC_KO_ATMA ? 0 : TC_A_BYTES) + (TC_KO_WTMA ? 0 : 2 * w_box_bytes)));
-                    if (!TC_KO_ATMA) {
-                        if (t < p.T1) tma_load_2d(&mapA1, a_raw(s), &full[s], t * TC_BK, m0);
-                        else          tma_load_2d(&mapA2, a_raw(s), &full[s], (t - p.T1) * TC_BK, m0);
-                    }
-                    if (!TC_KO_WTMA) {
-                        tma_load_2d(&mapWhi, w_hi(s), &full[s], t * TC_BK, tile_n0);
-                        tma_load_2d(&mapWlo, w_lo(s), &full[s], t * TC_BK, tile_n0);
-                    }
+                    mbar_expect_tx(&full[s], (uint32_t)(TC_A_BYTES + 2 * w_box_bytes));
+                    if (t < p.T1) tma_load_2d(&mapA1, a_raw(s), &full[s], t * TC_BK, m0);
+                    else          tma_load_2d(&mapA2, a_raw(s), &full[s], (t - p.T1) * TC_BK, m0);
+                    tma_load_2d(&mapWhi, w_hi(s), &full[s], t * TC_BK, tile_n0);
+                    tma_load_2d(&mapWlo, w_lo(s), &full[s], t * TC_BK, tile_n0);
                 }
             }
         }
     } else if (warp < TC_CONV_WARP0) {
-        // ===================================================== MMA issuer(s)
-        const int role = TC_SPLIT_ISSUE ? warp : 0;   // 0: every product; 1: main product only; 2: compensation products only
+        // ===================================================== MMA issuer
         // The whole warp runs the loop and ONE ELECTED lane issues: inside a divergent `if (lane == 0)` the compiler
         // cannot keep the descriptors in uniform registers and wraps every UTCHMMA in an ELECT/vote loop with R2UR moves.
         //
         // This warp is a serial program and MMA issue blocks (the tensor queue is a couple of MMAs deep), so everything it
-        // does besides issuing is dead time for the tensor pipe.  Measured with the knock-out builds (TC_KO_*): with NO
-        // MMAs, NO loads and NO conversion the loop still took ~780 cycles per k-block -- every mbarrier check costs
-        // ~40 cycles, a commit ~30 -- against 288 tensor cycles for a 3xFP16 k-block.  Hence: ONE barrier per k-block
+        // does besides issuing is dead time for the tensor pipe.  Measured with knock-out builds (DESIGN.md section 4):
+        // with NO MMAs, NO loads and NO conversion the loop still took ~780 cycles per k-block -- every mbarrier check
+        // costs ~40 cycles, a commit ~30 -- against 288 tensor cycles for a 3xFP16 k-block.  Hence: ONE barrier per k-block
         // towards the converters (conv[]; it implies full[]: the converters only publish after they have seen the stage's
         // TMA bytes land, and the weights arrive on the same transaction barrier), one probe of the next one, two commits
-        // (tfree[], w_free[]), ring positions kept as counters (no division), and optionally TC_ISSUE_KBLOCK k-blocks per
-        // synchronisation point.
-        constexpr int KBI = (TC_TSTAGES / 2 >= 4) ? TC_ISSUE_KBLOCK : 1;   // 3xTF32 has only 2 k-blocks of A stages in tensor memory
+        // (tfree[], w_free[]) and ring positions kept as counters (no division).
         int it = 0;
-        long long m_conv = 0, m_acc = 0, m_probe = 0, m_issue = 0;
-        if constexpr (TC_PINGPONG) {
-            // TWO issuers taking turns on k-blocks.  Knock-out builds showed the single issuer's loop to be ADDITIVE: ~285 cycles
-            // of barrier work per k-block (wait, fence, probe, commits) plus the ~288 cycles it sits blocked in the issue of its
-            // six MMAs (the tensor queue holds about two), 569 together with everything else removed -- the tensor pipe idled
-            // while the warp did its bookkeeping.  Here warp 1 issues the even k-blocks and warp 2 the odd ones; each does its
-            // bookkeeping while the other is blocked issuing.  The accumulation ORDER stays fixed (bitwise reproducible
-            // results): k-block g is only issued after the hand-off barrier says that k-block g-1 has been issued completely,
-            // and the MMAs of one CTA execute in issue order.
-            const int me = warp - 1;
-            uint32_t g = 0;
-            int s = 0, ks = 0; uint32_t kph = 0;
-            TC_T(m_t0);
-            for (int L = blockIdx.x; L < total_tiles; L += gridDim.x, ++it) {
-                const int n_tile = L % n_tiles;
-                const int tile_bn = tile_bn_of(n_tile);
-                const int buf = it & 1;
-                const uint32_t idesc = (1u << 4) | ((F16 ? 0u : 2u) << 7) | ((F16 ? 0u : 2u) << 10) | ((uint32_t)(tile_bn >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
-                const uint32_t d_main = tmem + TC_COL_ACC * buf, d_corr = d_main + TC_COL_CORR;
-                bool acc_ok = false;
-                for (int t = 0; t < T; ++t, ++g) {
-                    if ((int)(g & 1) == me) {
-                        if (!acc_ok) { mbar_wait(&acc_free[buf], ((it >> 1) & 1) ^ 1, 190); acc_ok = true; }   // epilogue of tile it-2 drained this buffer
-                        TC_T(mc0);
-                        mbar_wait(&conv[ks], kph, 300 + t);
-                        TC_T(mc1);
-                        TC_ACC(m_conv, mc0, mc1);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        if (g > 0) {
-                            mbar_wait(&turn_bar, (g - 1) & 1, 360);                  // k-block g-1 has been issued
-                            if (TC_PP_FENCE) asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        }
-                        TC_T(mp1);
-                        TC_ACC(m_probe, mc1, mp1);
-                        if (elect_one()) {
-                            const uint64_t dbh = F16 ? make_kmajor_sw64_desc(smem_u32(w_hi(s))) : make_kmajor_sw128_desc(smem_u32(w_hi(s)));
-                            const uint64_t dbl = F16 ? make_kmajor_sw64_desc(smem_u32(w_lo(s))) : make_kmajor_sw128_desc(smem_u32(w_lo(s)));
-#pragma unroll
-                            for (int h = 0; h < 2; ++h) {
-                                const uint32_t t_hi = tmem + TC_COL_A + TS_COLS * (2 * ks + h), t_lo = t_hi + TS_COLS / 2;
-                                if (F16) {
-                                    const uint64_t adv = (uint64_t)(h * 32 >> 4);
-                                    umma_f16_ts(d_corr, t_lo, dbh + adv, idesc, (t | h) != 0);
-                                    umma_f16_ts(d_corr, t_hi, dbl + adv, idesc, 1);
-                                    umma_f16_ts(d_main, t_hi, dbh + adv, idesc, (t | h) != 0);
-                                } else {
-#pragma unroll
-                                    for (int kk = 0; kk < 2; ++kk) {
-                                        const int k = 2 * h + kk;
-                                        const uint64_t adv = (uint64_t)(k * 32 >> 4);
-                                        umma_tf32_ts(d_corr, t_lo + 8 * kk, dbh + adv, idesc, (t | k) != 0);
-                                        umma_tf32_ts(d_corr, t_hi + 8 * kk, dbl + adv, idesc, 1);
-                                        umma_tf32_ts(d_main, t_hi + 8 * kk, dbh + adv, idesc, (t | k) != 0);
-                                    }
-                                }
-                            }
-                            if (TC_PP_FENCE) asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                            mbar_arrive(&turn_bar);                      // the other issuer may go
-                            umma_commit(&tfree[ks]);
-                            umma_commit(&w_free[s]);
-                        }
-                        TC_T(mi1);
-                        TC_ACC(m_issue, mp1, mi1);
-                        __syncwarp();
-                    }
-                    s = s + 1 == TC_STAGES ? 0 : s + 1;
-                    ks = ks + 1 == TC_TSTAGES / 2 ? 0 : ks + 1; if (ks == 0) kph ^= 1;
-                }
-                // both issuers sign the tile off (an issuer without a k-block in this tile has nothing outstanding)
-                if (elect_one()) umma_commit(&acc_full[buf]);
-                __syncwarp();
-            }
-#if TC_PHASE_TIMERS
-            if (lane == 0 && warp == 1) {
-                atomicAdd(&fc_tc_dbg[0], 1ull); atomicAdd(&fc_tc_dbg[1], (unsigned long long)(clock64() - m_t0));
-                atomicAdd(&fc_tc_dbg[3], (unsigned long long)m_conv); atomicAdd(&fc_tc_dbg[4], (unsigned long long)m_acc);
-                atomicAdd(&fc_tc_dbg[10], (unsigned long long)m_probe); atomicAdd(&fc_tc_dbg[11], (unsigned long long)m_issue);
-            }
-#endif
-        } else {
         bool conv_seen = false;   // the next k-block's barrier was seen complete by the probe
-        uint32_t kuse = 1;        // use count of the current TMEM A stage (flag value the converters publish)
         int s = 0;                // shared-memory stage of the next k-block
         int ks = 0; uint32_t kph = 0;   // tensor-memory A stage (one per k-block) of the next k-block and its barrier phase
-        TC_T(m_t0);
         for (int L = blockIdx.x; L < total_tiles; L += gridDim.x, ++it) {
             const int n_tile = L % n_tiles;
             const int tile_bn = tile_bn_of(n_tile);
@@ -410,152 +201,96 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
             // (kind::f16: A = B = fp16 is format 0)
             const uint32_t idesc = (1u << 4) | ((F16 ? 0u : 2u) << 7) | ((F16 ? 0u : 2u) << 10) | ((uint32_t)(tile_bn >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
             const uint32_t d_main = tmem + TC_COL_ACC * buf, d_corr = d_main + TC_COL_CORR;
-            const bool fuse_wlo = F16 && TC_FUSE_WLO && !TC_SPLIT_ISSUE;   // the Wlo box sits 96 rows behind the Whi box
             const uint32_t idesc_wide = (idesc & ~(0x3fu << 17)) | ((uint32_t)((TC_BN_CAP + tile_bn) >> 3) << 17);
-            TC_T(ma0);
             mbar_wait(&acc_free[buf], ((it >> 1) & 1) ^ 1, 190);     // the epilogue of tile it-2 has drained this buffer
-            TC_T(ma1);
-            TC_ACC(m_acc, ma0, ma1);
-            for (int t = 0; t < T;) {
-                const int nb = min(KBI, T - t);
-                TC_T(mc0);
-                if constexpr (CFLAGS) {
-                    // the four converter warps of the k-block's group have each stored the stage's use count (release) after
-                    // their tcgen05.st completed; one 16-byte acquire load reads all four
-                    const uint32_t fa = smem_u32(&conv_flag[ks][0]);
-                    uint32_t f0, f1, f2, f3, spin = 0;
-                    for (;;) {
-                        asm volatile("ld.acquire.cta.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(f0), "=r"(f1), "=r"(f2), "=r"(f3) : "r"(fa) : "memory");
-                        if (min(min(f0, f1), min(f2, f3)) >= kuse) break;
-                        if (++spin > (1u << 24)) mbar_timeout(300 + t, kuse);
-                    }
-                } else {
+            for (int t = 0; t < T; ++t) {
                 if (!conv_seen) mbar_wait(&conv[ks], kph, 300 + t);
-                if (nb > 1) { const int k2 = ks + 1 == TC_TSTAGES / 2 ? 0 : ks + 1; mbar_wait(&conv[k2], k2 ? kph : kph ^ 1, 350 + t); }
-                }
-                TC_T(mc1);
-                TC_ACC(m_conv, mc0, mc1);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                if constexpr (!CFLAGS) {   // probe the NEXT group's first k-block now: a wait after the issue is dead time for the tensor pipe
-                    int kn = ks + nb; uint32_t pn = kph;
+                {   // probe the NEXT k-block now: a wait after the issue is dead time for the tensor pipe
+                    int kn = ks + 1; uint32_t pn = kph;
                     if (kn >= TC_TSTAGES / 2) { kn -= TC_TSTAGES / 2; pn ^= 1; }
-                    conv_seen = TC_PROBE ? mbar_test(&conv[kn], pn) : false;
+                    conv_seen = mbar_test(&conv[kn], pn);
                 }
-                TC_T(mp1);
-                TC_ACC(m_probe, mc1, mp1);
                 if (elect_one()) {
-                    int sj = s, kj = ks;
-                    for (int j = 0; j < nb; ++j) {
-                        const uint64_t dbh = F16 ? make_kmajor_sw64_desc(smem_u32(w_hi(sj))) : make_kmajor_sw128_desc(smem_u32(w_hi(sj)));
-                        const uint64_t dbl = F16 ? make_kmajor_sw64_desc(smem_u32(w_lo(sj))) : make_kmajor_sw128_desc(smem_u32(w_lo(sj)));
-                        const int tt = t + j;
+                    const uint64_t dbh = F16 ? make_kmajor_sw64_desc(smem_u32(w_hi(s))) : make_kmajor_sw128_desc(smem_u32(w_hi(s)));
+                    const uint64_t dbl = F16 ? make_kmajor_sw64_desc(smem_u32(w_lo(s))) : make_kmajor_sw128_desc(smem_u32(w_lo(s)));
 #pragma unroll
-                        for (int h = 0; h < 2; ++h) {
-                            // the k-block's A operand: two half k-blocks of TS_COLS columns each (first half hi, second half lo)
-                            const uint32_t t_hi = tmem + TC_COL_A + TS_COLS * (2 * kj + h), t_lo = t_hi + TS_COLS / 2;
-                            if (F16) {
-                                // one kind::f16 MMA covers the half k-block (16 k = 32 bytes of the 64-byte weight row)
-                                const uint64_t adv = (uint64_t)(h * 32 >> 4);
-                                if (fuse_wlo) {
-                                    // Whi and Wlo are adjacent 96-row boxes of the stage and the two accumulators adjacent 96-column
-                                    // blocks of TMEM: ONE MMA of N = 96 + tile_bn computes Ahi.[Whi; Wlo] -> [main | compensation].
-                                    // A TS-form kind::f16 MMA costs the same issue time at N = 192 as at N = 96
-                                    // (scripts/micro/peaks.cu), so two instructions per half k-block instead of three.
-                                    // (Columns tile_bn..95 of main receive the next tile's weight rows: never read.)
-                                    umma_f16_ts(d_main, t_hi, dbh + adv, idesc_wide, (tt | h) != 0);
-                                    umma_f16_ts(d_corr, t_lo, dbh + adv, idesc, 1);               // (A - Ahi) 2^11 . Whi
-                                } else {
-                                if (role != 1) {
-                                    umma_f16_ts(d_corr, t_lo, dbh + adv, idesc, (tt | h) != 0);   // (A - Ahi) 2^11 . Whi
-                                    umma_f16_ts(d_corr, t_hi, dbl + adv, idesc, 1);               // Ahi . (W - Whi) 2^11
-                                }
-                                if (role != 2) umma_f16_ts(d_main, t_hi, dbh + adv, idesc, (tt | h) != 0);
-                                }
-                            } else {
+                    for (int h = 0; h < 2; ++h) {
+                        // the k-block's A operand: two half k-blocks of TS_COLS columns each (first half hi, second half lo)
+                        const uint32_t t_hi = tmem + TC_COL_A + TS_COLS * (2 * ks + h), t_lo = t_hi + TS_COLS / 2;
+                        if (F16) {
+                            // one kind::f16 MMA covers the half k-block (16 k = 32 bytes of the 64-byte weight row).
+                            // Whi and Wlo are adjacent 96-row boxes of the stage and the two accumulators adjacent 96-column
+                            // blocks of TMEM: ONE MMA of N = 96 + tile_bn computes Ahi.[Whi; Wlo] -> [main | compensation].
+                            // A TS-form kind::f16 MMA costs the same issue time at N = 192 as at N = 96
+                            // (scripts/micro/peaks.cu), so two instructions per half k-block instead of three.
+                            // (Columns tile_bn..95 of main receive the next tile's weight rows: never read.)
+                            const uint64_t adv = (uint64_t)(h * 32 >> 4);
+                            umma_f16_ts(d_main, t_hi, dbh + adv, idesc_wide, (t | h) != 0);
+                            umma_f16_ts(d_corr, t_lo, dbh + adv, idesc, 1);               // (A - Ahi) 2^11 . Whi
+                        } else {
 #pragma unroll
-                                for (int kk = 0; kk < 2; ++kk) {
-                                    const int k = 2 * h + kk;
-                                    const uint64_t adv = (uint64_t)(k * 32 >> 4);   // 8 tf32 = 32 bytes per k-step
-                                    if (role != 1) {
-                                        umma_tf32_ts(d_corr, t_lo + 8 * kk, dbh + adv, idesc, (tt | k) != 0);
-                                        umma_tf32_ts(d_corr, t_hi + 8 * kk, dbl + adv, idesc, 1);
-                                    }
-                                    if (role != 2) umma_tf32_ts(d_main, t_hi + 8 * kk, dbh + adv, idesc, (tt | k) != 0);
-                                }
+                            for (int kk = 0; kk < 2; ++kk) {
+                                const int k = 2 * h + kk;
+                                const uint64_t adv = (uint64_t)(k * 32 >> 4);   // 8 tf32 = 32 bytes per k-step
+                                umma_tf32_ts(d_corr, t_lo + 8 * kk, dbh + adv, idesc, (t | k) != 0);
+                                umma_tf32_ts(d_corr, t_hi + 8 * kk, dbl + adv, idesc, 1);
+                                umma_tf32_ts(d_main, t_hi + 8 * kk, dbh + adv, idesc, (t | k) != 0);
                             }
                         }
-                        umma_commit(&tfree[kj]);                     // TMEM A stage reusable once these MMAs retire
-                        umma_commit(&w_free[sj]);                    // W smem stage reusable once these MMAs retire
-                        sj = sj + 1 == TC_STAGES ? 0 : sj + 1;
-                        kj = kj + 1 == TC_TSTAGES / 2 ? 0 : kj + 1;
                     }
+                    umma_commit(&tfree[ks]);                     // TMEM A stage reusable once these MMAs retire
+                    umma_commit(&w_free[s]);                     // W smem stage reusable once these MMAs retire
                 }
-                TC_T(mi1);
-                TC_ACC(m_issue, mp1, mi1);
                 __syncwarp();
-                t += nb;
-                s += nb; if (s >= TC_STAGES) s -= TC_STAGES;
-                ks += nb; if (ks >= TC_TSTAGES / 2) { ks -= TC_TSTAGES / 2; kph ^= 1; ++kuse; }
+                s = s + 1 == TC_STAGES ? 0 : s + 1;
+                ks = ks + 1 == TC_TSTAGES / 2 ? 0 : ks + 1; if (ks == 0) kph ^= 1;
             }
             if (elect_one()) umma_commit(&acc_full[buf]);        // accumulators of this tile complete
             __syncwarp();
         }
-#if TC_PHASE_TIMERS
-        if (lane == 0 && warp == TC_MMA_WARPS) {   // the busier issuer (all products, or the compensation products)
-            atomicAdd(&fc_tc_dbg[0], 1ull); atomicAdd(&fc_tc_dbg[1], (unsigned long long)(clock64() - m_t0));
-            atomicAdd(&fc_tc_dbg[3], (unsigned long long)m_conv); atomicAdd(&fc_tc_dbg[4], (unsigned long long)m_acc);
-            atomicAdd(&fc_tc_dbg[10], (unsigned long long)m_probe); atomicAdd(&fc_tc_dbg[11], (unsigned long long)m_issue);
-        }
-#endif
-        }   // single issuer / per-accumulator issuers
     } else if (warp < TC_EPI_WARP0) {
         // ===================================================== converters: fp32 smem row -> (hi, lo) in TMEM
         const int quad = warp & 3;                   // TMEM lane quadrant this warp may touch
         const int row_in_tile = quad * 32 + lane;
         const uint32_t lane_addr = (uint32_t)(quad * 32) << 16;
-        const int my_half = (warp - TC_CONV_WARP0) >> 2;   // 8 converter warps: the first four take the first half of every k-block, the others the second
-        // Software pipelined by one half k-block: the tcgen05.st of a half is in flight while the next one is loaded and
-        // split; only then is it awaited and published (one arrival per thread and half on the k-block's conv[] barrier,
-        // 256 arrivals per k-block with 4 or 8 converter warps), so the store latency is off the critical path.
+        const int my_half = (warp - TC_CONV_WARP0) >> 2;   // 3xTF32: the first four warps take the first half of every k-block, the others the second
+        // Software pipelined by one step: the tcgen05.st of a k-block (3xTF32: of a half) is in flight while the next one is
+        // loaded and split; only then is it awaited and published (one arrival per thread on the k-block's conv[] barrier),
+        // so the store latency is off the critical path.
         int s = 0; uint32_t sph = 0;   // shared-memory stage / phase of the current k-block
         int ks = 0; uint32_t kph = 0;  // tensor-memory A stage (one per k-block) / phase
         int pending = -1;              // k-block stage whose store has been issued but not yet published
-        long long c_full = 0, c_tfree = 0;
-        TC_T(c_t0);
         if constexpr (PARITY) {
             // Two converter groups take turns on k-blocks: every role of this kernel pays ~100 cycles per mbarrier wait (even on a
             // completed phase) plus the tcgen05.st round trip, so ONE group working through every k-block was a ~500-cycle serial
             // chain per k-block (knock-out builds: the pipeline ran at that pace with all the work removed).  A thread converts
             // its whole 32-float row of the k-block and writes it with one 32-column tcgen05.st.
             const int grp = (warp - TC_CONV_WARP0) >> 2;
-            uint32_t g = 0, cuse = 1, pend_use = 0;
+            uint32_t g = 0;
             auto publish = [&]() {
                 asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                 asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                if constexpr (CFLAGS) {
-                    __syncwarp();
-                    if (lane == 0)
-                        asm volatile("st.release.cta.shared.u32 [%0], %1;" :: "r"(smem_u32(&conv_flag[pending][(warp - TC_CONV_WARP0) & 3])), "r"(pend_use) : "memory");
-                } else {
-                    warp_arrive(&conv[pending]);
-                }
+                mbar_arrive(&conv[pending]);
                 pending = -1;
             };
             for (int L = blockIdx.x; L < total_tiles; L += gridDim.x) {
                 for (int t = 0; t < T; ++t, ++g) {
                     if ((int)(g & 1) == grp) {
                         if (pending >= 0) publish();
-                        TC_T(cf0);
-                        mbar_wait_hint(&full[s], sph, 400 + t, TC_HINT_CONV);
-                        TC_T(cf1);
-                        TC_ACC(c_full, cf0, cf1);
+                        mbar_wait(&full[s], sph, 400 + t);
                         const float4* rowp = reinterpret_cast<const float4*>(a_raw(s) + row_in_tile * 128);
                         uint32_t hl[32];   // [half 0: hi x8 | lo x8 | half 1: hi x8 | lo x8], two fp16 per column
 #pragma unroll
-                        for (int j = 0; j < (TC_KO_CONV ? 0 : 8); ++j) {
+                        for (int j = 0; j < 8; ++j) {
+                            // 128B swizzle: logical 16-byte chunk j of row r sits at physical chunk j ^ (r & 7); a quarter
+                            // warp (8 consecutive rows) therefore hits all 32 banks exactly once
                             const float4 x = rowp[j ^ (row_in_tile & 7)];
                             const float xv[4] = {x.x, x.y, x.z, x.w};
                             const int base = 16 * (j >> 2) + 2 * (j & 3);
+                            // hi = fp16(x) (11-bit significand, like TF32), lo = fp16((x - hi) * 2^11): the residual is
+                            // taken from the value the tensor core will actually see, so fp16 subnormals lose nothing;
+                            // |x| >= 65520 becomes inf and the row's result NaN (loud, never silently clipped)
 #pragma unroll
                             for (int e = 0; e < 4; e += 2) {
                                 const uint32_t hp = pack_f16x2(xv[e], xv[e + 1]);
@@ -566,19 +301,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                                 hl[base + 8 + (e >> 1)] = pack_f16x2(d2.x, d2.y);
                             }
                         }
-                        if (!TC_NO_AFREE) warp_arrive(&a_free[s]);
-                        TC_T(ct0);
-                        mbar_wait_hint(&tfree[ks], kph ^ 1, 450 + t, TC_HINT_CONV);
-                        TC_T(ct1);
-                        TC_ACC(c_tfree, ct0, ct1);
+                        mbar_wait(&tfree[ks], kph ^ 1, 450 + t);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        const uint32_t dst = tmem + lane_addr + TC_COL_A + TS_COLS * (2 * ks);
-                        if constexpr (TC_KO_CONV) { (void)hl; (void)dst; }
-                        else tmem_st32(dst, hl);
-                        pending = ks; pend_use = cuse;
+                        tmem_st32(tmem + lane_addr + TC_COL_A + TS_COLS * (2 * ks), hl);
+                        pending = ks;
                     }
                     s = s + 1 == TC_STAGES ? 0 : s + 1; if (s == 0) sph ^= 1;
-                    ks = ks + 1 == TC_TSTAGES / 2 ? 0 : ks + 1; if (ks == 0) { kph ^= 1; ++cuse; }
+                    ks = ks + 1 == TC_TSTAGES / 2 ? 0 : ks + 1; if (ks == 0) kph ^= 1;
                 }
             }
             if (pending >= 0) publish();
@@ -588,66 +317,37 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                 if (pending >= 0) {      // never hold a finished stage back while waiting for the next k-block's data
                     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                    warp_arrive(&conv[pending]);
+                    mbar_arrive(&conv[pending]);
                     pending = -1;
                 }
-                TC_T(cf0);
-                mbar_wait_hint(&full[s], sph, 400 + t, TC_HINT_CONV);
-                TC_T(cf1);
-                TC_ACC(c_full, cf0, cf1);
+                mbar_wait(&full[s], sph, 400 + t);
                 const float4* rowp = reinterpret_cast<const float4*>(a_raw(s) + row_in_tile * 128);
 #pragma unroll
                 for (int h = 0; h < 2; ++h) {
-                    if (TC_CONV_WARPS_N == 8 && h != my_half) continue;   // two threads per row: each converts its own half k-block
+                    if (h != my_half) continue;   // two threads per row: each converts its own half k-block
                     uint32_t hl[TS_COLS];   // this half k-block: first half hi, second half lo
 #pragma unroll
-                    for (int jj = 0; jj < (TC_KO_CONV ? 0 : 4); ++jj) {
-                        // 128B swizzle: logical 16-byte chunk j of row r sits at physical chunk j ^ (r & 7); a quarter
-                        // warp (8 consecutive rows) therefore hits all 32 banks exactly once
+                    for (int jj = 0; jj < 4; ++jj) {
                         const int j = 4 * h + jj;
-                        const float4 x = rowp[j ^ (row_in_tile & 7)];
+                        const float4 x = rowp[j ^ (row_in_tile & 7)];   // 128B swizzle, as above
                         const float xv[4] = {x.x, x.y, x.z, x.w};
-                        if (F16) {
-                            // hi = fp16(x) (11-bit significand, like TF32), lo = fp16((x - hi) * 2^11): the residual is
-                            // taken from the value the tensor core will actually see, so fp16 subnormals lose nothing;
-                            // |x| >= 65520 becomes inf and the row's result NaN (loud, never silently clipped)
 #pragma unroll
-                            for (int e = 0; e < 4; e += 2) {
-                                const uint32_t hp = pack_f16x2(xv[e], xv[e + 1]);
-                                float h0, h1;
-                                unpack_f16x2(hp, h0, h1);
-                                hl[2 * jj + (e >> 1)] = hp;
-                                const float2 d2 = __fmul2_rn(__fadd2_rn(make_float2(xv[e], xv[e + 1]), make_float2(-h0, -h1)), make_float2(2048.0f, 2048.0f));
-                                hl[TS_COLS / 2 + 2 * jj + (e >> 1)] = pack_f16x2(d2.x, d2.y);
-                            }
-                        } else {
-#pragma unroll
-                            for (int e = 0; e < 4; ++e) {
-                                // cvt.rna.tf32.f32 by hand (add half a TF32 ulp to the magnitude, clear the low 13 bits):
-                                // 2 ALU ops instead of the 4 (add, inf test, select, mask) ptxas emits; inputs are finite
-                                const uint32_t u = (__float_as_uint(xv[e]) + 0x1000u) & 0xffffe000u;
-                                hl[4 * jj + e] = u;
-                                hl[TS_COLS / 2 + 4 * jj + e] = __float_as_uint(xv[e] - __uint_as_float(u));
-                            }
+                        for (int e = 0; e < 4; ++e) {
+                            // cvt.rna.tf32.f32 by hand (add half a TF32 ulp to the magnitude, clear the low 13 bits):
+                            // 2 ALU ops instead of the 4 (add, inf test, select, mask) ptxas emits; inputs are finite
+                            const uint32_t u = (__float_as_uint(xv[e]) + 0x1000u) & 0xffffe000u;
+                            hl[4 * jj + e] = u;
+                            hl[TS_COLS / 2 + 4 * jj + e] = __float_as_uint(xv[e] - __uint_as_float(u));
                         }
                     }
-                    if (!TC_NO_AFREE && (h == 1 || TC_CONV_WARPS_N == 8)) warp_arrive(&a_free[s]);   // this thread's part of the row is in registers: the A smem stage may be refilled
                     if (pending >= 0) {
                         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                        warp_arrive(&conv[pending]);
+                        mbar_arrive(&conv[pending]);
                     }
-                    if (h == 0 || TC_CONV_WARPS_N == 8) {   // once per k-block: the MMAs that read this TMEM stage have retired
-                        TC_T(ct0);
-                        mbar_wait_hint(&tfree[ks], kph ^ 1, 450 + t, TC_HINT_CONV);
-                        TC_T(ct1);
-                        TC_ACC(c_tfree, ct0, ct1);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    }
-                    const uint32_t dst = tmem + lane_addr + TC_COL_A + TS_COLS * (2 * ks + h);
-                    if constexpr (TC_KO_CONV) { (void)hl; (void)dst; }
-                    else if constexpr (F16) tmem_st16(dst, hl);
-                    else tmem_st32(dst, hl);
+                    mbar_wait(&tfree[ks], kph ^ 1, 450 + t);   // the MMAs that read this TMEM stage have retired
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    tmem_st32(tmem + lane_addr + TC_COL_A + TS_COLS * (2 * ks + h), hl);
                     pending = ks;
                 }
                 s = s + 1 == TC_STAGES ? 0 : s + 1; if (s == 0) sph ^= 1;
@@ -657,14 +357,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
         if (pending >= 0) {
             asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            warp_arrive(&conv[pending]);
+            mbar_arrive(&conv[pending]);
         }
-#if TC_PHASE_TIMERS
-        if (threadIdx.x == 32 * TC_CONV_WARP0) {
-            atomicAdd(&fc_tc_dbg[5], (unsigned long long)(clock64() - c_t0));
-            atomicAdd(&fc_tc_dbg[6], (unsigned long long)c_full); atomicAdd(&fc_tc_dbg[7], (unsigned long long)c_tfree);
-        }
-#endif
     } else {
         // ===================================================== epilogue (8 warps, 256 threads)
         // TMEM lane = row within the tile; the two warps of a quadrant take alternate 16-column chunks
@@ -679,9 +373,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
         // conflict free, the transposed ones 2-way at worst)
         float* stg = stage_out + ew * TcCfg<F16>::STG_FLOATS;
         int it = 0;
-        long long e_wait = 0;
         bool tma_pending = false;
-        TC_T(e_t0);
         for (int L = blockIdx.x; L < total_tiles; L += gridDim.x, ++it) {
             const int n_tile = L % n_tiles, m0 = (L / n_tiles) * TC_BM;
             const int tile_n0 = tile_n0_of(n_tile), tile_bn = tile_bn_of(n_tile);
@@ -744,7 +436,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
             }
             // Same for the coupling epilogue's latent values (8 per row and chunk): copied ahead into a compact [32][12] tile
             // behind the [32][20] staging tile.
-            const bool cpl_pf = TcCfg<F16>::RES_PF && EPI == FC_EPI_COUPLING && !TC_KO_CPLMEM && TC_CPL_STAGED && row0 + 32 <= a.M &&
+            const bool cpl_pf = TcCfg<F16>::RES_PF && EPI == FC_EPI_COUPLING && row0 + 32 <= a.M &&
                                 ((a.ldx | a.col0) & 1) == 0 && (reinterpret_cast<uintptr_t>(a.x) & 7) == 0;
             auto cpl_prefetch = [&](int c0n) {
                 const int coln = tile_n0 + c0n;
@@ -760,10 +452,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
             if (cpl_pf) cpl_prefetch(half * 16);
             float mu = 0.f, rstd = 0.f;
             if (EPI == FC_EPI_LNQ && m0 + row_in_tile < a.M) { mu = a.row_mu[m0 + row_in_tile]; rstd = a.row_rstd[m0 + row_in_tile]; }
-            TC_T(ea0);
-            mbar_wait_hint(&acc_full[buf], (it >> 1) & 1, 500, TC_HINT_EPI);
-            TC_T(ea1);
-            TC_ACC(e_wait, ea0, ea1);
+            mbar_wait(&acc_full[buf], (it >> 1) & 1, 500);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             __syncwarp();                                      // bias_sm / csum_sm visible to the whole warp
             const uint32_t acc_main = tmem + lane_addr + TC_COL_ACC * buf, acc_corr = acc_main + TC_COL_CORR;
@@ -775,7 +464,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
             if (a.bias && a.bias_group > 0 && row_ok) bias_row = a.bias + (size_t)(row / a.bias_group) * a.bias_ld;
             // the accumulator loads of chunk c+1 are in flight while chunk c goes through its bias / activation / stores
             uint32_t r[16], rc[16];
-            bool acc_released = false;
             if (half * 16 < tile_bn) tmem_ld16x2_issue(acc_main + (uint32_t)(half * 16), acc_corr + (uint32_t)(half * 16), r, rc);
             for (int c0 = half * 16; c0 < tile_bn; c0 += 32) {
                 float v[16];
@@ -793,16 +481,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                     v[j] = o2.x; v[j + 1] = o2.y;
                 }
                 if (c0 + 32 < tile_bn) tmem_ld16x2_issue(acc_main + (uint32_t)(c0 + 32), acc_corr + (uint32_t)(c0 + 32), r, rc);
-                else if (TC_EARLY_ACC_FREE) {
-                    // that was this warp's last read of the accumulator: hand the buffer back to the MMA issuer now, not after the
-                    // chunk's arithmetic and stores
-                    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                    warp_arrive(&acc_free[buf]);
-                    acc_released = true;
-                }
                 const int col = n0 + c0;
                 if (col >= a.N) continue;                     // warp-uniform
-                if (TC_KO_EPI) { if (v[0] == 123.456f) a.C[0] = v[1]; continue; }
                 if (EPI == FC_EPI_LNQ) {
     #pragma unroll
                     for (int j = 0; j < 16; ++j)
@@ -1036,7 +716,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
     #pragma unroll
                         for (int j = 0; j < 16; ++j) { th[(size_t)j * a.kv_ncp] = v[j]; tl[(size_t)j * a.kv_ncp] = lo16[j]; }
                     }
-                } else if (EPI == FC_EPI_COUPLING && !TC_KO_CPLMEM && TC_CPL_STAGED && row0 + 32 <= a.M && col + 16 <= a.N &&
+                } else if (EPI == FC_EPI_COUPLING && row0 + 32 <= a.M && col + 16 <= a.N &&
                            ((a.ldx | a.col0) & 1) == 0 && (reinterpret_cast<uintptr_t>(a.x) & 7) == 0) {
                     // reference models/affine_coupling.py:40-46.  Interior chunk of a full 32-row quadrant: the chunk's 8 latent
                     // values per row go through the warp's staging tile so that the global accesses are COALESCED (a warp
@@ -1087,23 +767,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                         // interior chunk: the row's 8 latent values move as four 8-byte accesses, loads first
                         float2 xv[4];
     #pragma unroll
-                        for (int q = 0; q < 4; ++q) xv[q] = TC_KO_CPLMEM ? make_float2(v[q], v[q + 4]) : *reinterpret_cast<const float2*>(xrow + 2 * q);
+                        for (int q = 0; q < 4; ++q) xv[q] = *reinterpret_cast<const float2*>(xrow + 2 * q);
     #pragma unroll
                         for (int q = 0; q < 4; ++q) {
-                            const float sig0 = TC_KO_CPLMATH ? v[4 * q] : 1.0f / (1.0f + expf(-v[4 * q]));
+                            const float sig0 = 1.0f / (1.0f + expf(-v[4 * q]));
                             const float sc0 = (2.0f * sig0 - 1.0f) + 1.0f;
-                            const float sig1 = TC_KO_CPLMATH ? v[4 * q + 2] : 1.0f / (1.0f + expf(-v[4 * q + 2]));
+                            const float sig1 = 1.0f / (1.0f + expf(-v[4 * q + 2]));
                             const float sc1 = (2.0f * sig1 - 1.0f) + 1.0f;
                             xv[q].x = fmaf(xv[q].x, sc0, v[4 * q + 1]);
                             xv[q].y = fmaf(xv[q].y, sc1, v[4 * q + 3]);
-                            ldj += TC_KO_CPLMATH ? sc0 : logf(sc0);
-                            ldj += TC_KO_CPLMATH ? sc1 : logf(sc1);
+                            ldj += logf(sc0);
+                            ldj += logf(sc1);
                         }
-                        if (TC_KO_CPLMEM) { if (xv[0].x + xv[1].y + xv[2].x + xv[3].y == 123.456f) xrow[0] = 1.f; }
-                        else {
     #pragma unroll
                         for (int q = 0; q < 4; ++q) *reinterpret_cast<float2*>(xrow + 2 * q) = xv[q];
-                        }
                     } else {
     #pragma unroll
                         for (int q = 0; q < 8; ++q) {
@@ -1153,17 +830,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA1, const __grid_constant_
                 }
             }
             // this thread's TMEM reads of the tile are complete (every tcgen05.ld above is followed by its wait)
-            if (!acc_released) {
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                warp_arrive(&acc_free[buf]);
-            }
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            mbar_arrive(&acc_free[buf]);
         }
         if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");    // this warp's TMA stores have landed
-#if TC_PHASE_TIMERS
-        if (threadIdx.x == 32 * TC_EPI_WARP0) {
-            atomicAdd(&fc_tc_dbg[8], (unsigned long long)(clock64() - e_t0)); atomicAdd(&fc_tc_dbg[9], (unsigned long long)e_wait);
-        }
-#endif
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -1292,12 +962,10 @@ int fc_launch_gemm_tc(const GemmArgs& a, cudaStream_t stream) {
     const int f16 = a.tc_fmt ? 1 : 0;
     if (!get_map(a.Whi, (uint64_t)a.ldk, (uint64_t)p.n_tiles * p.BN, (uint64_t)a.ldk, (uint32_t)p.BN, &mWh, f16)) return FC_ERR_CUDA;
     if (!get_map(a.Wlo, (uint64_t)a.ldk, (uint64_t)p.n_tiles * p.BN, (uint64_t)a.ldk, (uint32_t)p.BN, &mWl, f16)) return FC_ERR_CUDA;
-    // TMA-store epilogue (FC_TC_TMASTORE=0 turns it off for A/B runs): plain-store epilogues whose output rows are 16-byte aligned
-    static int tma_store_env = -1;
-    if (tma_store_env < 0) { const char* e = getenv("FC_TC_TMASTORE"); tma_store_env = (e && e[0] == '0') ? 0 : 1; }
+    // TMA-store epilogue: plain-store epilogues whose output rows are 16-byte aligned
     CUtensorMap mC = mA1;
     p.tma_store = 0;
-    if (tma_store_env && (a.epi == FC_EPI_STORE || a.epi == FC_EPI_LNQ) && (a.ldc & 3) == 0 && (reinterpret_cast<uintptr_t>(a.C) & 15) == 0) {
+    if ((a.epi == FC_EPI_STORE || a.epi == FC_EPI_LNQ) && (a.ldc & 3) == 0 && (reinterpret_cast<uintptr_t>(a.C) & 15) == 0) {
         if (!get_map(a.C, (uint64_t)a.N, (uint64_t)a.M, (uint64_t)a.ldc, 32, &mC, 2)) return FC_ERR_CUDA;
         p.tma_store = 1;
     }
@@ -1314,15 +982,6 @@ int fc_launch_gemm_tc(const GemmArgs& a, cudaStream_t stream) {
     cfg.gridDim = dim3(total_tiles < nsm ? total_tiles : nsm);      // persistent: one CTA per SM
     cfg.blockDim = dim3(TC_THREADS);
     cfg.stream = stream;
-    // FC_TC_PDL=1 turns programmatic dependent launch on: measured +0.5 % on the step (406.8 vs 405.0 pairs/s, all
-    // parity tests green), off by default until it has been through the multi-GPU runs
-    static int pdl_env = -1;
-    if (pdl_env < 0) { const char* e = getenv("FC_TC_PDL"); pdl_env = (e && e[0] == '1') ? 1 : 0; }
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    if (pdl_env) { cfg.attrs = attr; cfg.numAttrs = 1; }
-    p.pdl = pdl_env;
     const bool res = a.res != nullptr;
     cudaError_t le = cudaErrorInvalidValue;
     if (a.epi == FC_EPI_STORE) {
@@ -1351,12 +1010,4 @@ int fc_launch_gemm_tc(const GemmArgs& a, cudaStream_t stream) {
     fc_count_launch();
     FC_LAUNCH_OK();
     return FC_OK;
-}
-
-// phase counters: valid only in a -DTC_PHASE_TIMERS=1 build (scripts/build_variant.sh timers gemm_tc "-DTC_PHASE_TIMERS=1")
-extern "C" __attribute__((visibility("default"))) int fc_debug_tc_phases(unsigned long long* out16) {
-    if (cudaMemcpyFromSymbol(out16, fc_tc_dbg, 16 * sizeof(unsigned long long)) != cudaSuccess) return FC_ERR_CUDA;
-    unsigned long long z[16] = {};
-    if (cudaMemcpyToSymbol(fc_tc_dbg, z, sizeof(z)) != cudaSuccess) return FC_ERR_CUDA;
-    return TC_PHASE_TIMERS ? FC_OK : FC_ERR_UNSUPPORTED;
 }

@@ -40,22 +40,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int ta
     }
     mbar_timeout(tag, parity);
 }
-// same, with a suspend-time hint (ns): the hardware may park the waiting thread for up to that long per try instead of
-// returning after its short default limit, so long waits do not fill issue slots with the spin loop
-__device__ __forceinline__ void mbar_wait_hint(uint64_t* bar, uint32_t parity, int tag, uint32_t hint_ns) {
-    if (hint_ns == 0) { mbar_wait(bar, parity, tag); return; }
-    uint32_t done = 0;
-    for (uint32_t spin = 0; spin < (1u << 22); ++spin) {
-        asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t"
-            "}" : "=r"(done) : "r"(smem_u32(bar)), "r"(parity), "r"(hint_ns) : "memory");
-        if (done) return;
-    }
-    mbar_timeout(tag, parity);
-}
 // non-blocking probe of a phase: lets an issuing warp check the NEXT stage before it blocks on the tensor queue
 __device__ __forceinline__ bool mbar_test(uint64_t* bar, uint32_t parity) {
     uint32_t done;
@@ -72,14 +56,6 @@ __device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, void* smem_d
         "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
         ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
 }
-// same load, delivered to the same shared-memory offset (data and mbarrier) of every CTA in `mask`
-__device__ __forceinline__ void tma_load_2d_mcast(const CUtensorMap* map, void* smem_dst, uint64_t* bar, int c0, int c1,
-                                                  uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask) : "memory");
-}
 // TMA store of a shared-memory tile (bulk async group): generic-proxy writes must be fenced (fence.proxy.async) before it
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* smem_src, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
@@ -88,40 +64,28 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void*
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// arrive on the barrier at the same offset in every CTA of `mask` once the MMAs issued so far retire
-__device__ __forceinline__ void umma_commit_mcast(uint64_t* bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
 __device__ __forceinline__ bool elect_one() {   // one lane of a converged warp
     uint32_t pred;
     asm volatile("{\n\t.reg .b32 rx;\n\t.reg .pred px;\n\telect.sync rx|px, 0xffffffff;\n\tselp.u32 %0, 1, 0, px;\n\t}" : "=r"(pred));
     return pred != 0;
 }
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 // D[tmem] (+)= A[tmem] * B[smem descriptor]   (A: 128 lanes x 8 columns of TF32, B: K-major tile)
 __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    #if !(defined(TC_KO_MMA) && TC_KO_MMA)
     asm volatile(
         "{\n\t"
         ".reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t"
         "}" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
-#endif
 }
 // D[tmem] (+)= A[tmem] * B[smem descriptor]   (kind::f16: A = 128 lanes x 8 columns, each column two fp16 (k even in the low half); B: K-major fp16 tile, K = 16)
 __device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    #if !(defined(TC_KO_MMA) && TC_KO_MMA)
     asm volatile(
         "{\n\t"
         ".reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t"
         "}" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
-#endif
 }
 // K-major operand tile, 64-byte rows (32 fp16), SWIZZLE_64B: 8-row groups are 512 B apart (SBO)
 __device__ __forceinline__ uint64_t make_kmajor_sw64_desc(uint32_t smem_addr) {

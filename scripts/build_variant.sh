@@ -1,7 +1,7 @@
 #!/bin/bash
 # A/B helper: builds flowcompare_b200/variants/lib_<name>.so with extra -D flags for ONE source file.
-#   scripts/build_variant.sh conv4 gemm_tc "-DTC_CONV8=0"
-# and run with FLOWCOMPARE_B200_LIB=flowcompare_b200/variants/lib_conv4.so python bench.py ...
+#   scripts/build_variant.sh spl2 attention_tc "-DA_SPL=2"
+# and run with FLOWCOMPARE_B200_LIB=flowcompare_b200/variants/lib_spl2.so python bench.py ...
 set -e
 name=$1; src=$2; flags=$3
 mkdir -p build/var_$name flowcompare_b200/variants

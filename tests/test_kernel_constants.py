@@ -58,15 +58,18 @@ def test_gemm_tile_partition_covers_n_without_padding_columns():
         assert n0[-1] + packing.tc_bn(N) <= packing.tc_n_tiles(N) * packing.tc_bn(N)
 
 
+def _tc_source():
+    return open(os.path.join(ROOT, "flowcompare_b200", "csrc", "gemm_tc.cu")).read()
+
+
 def _tc_define(name):
-    src = open(os.path.join(ROOT, "flowcompare_b200", "csrc", "gemm_tc.cu")).read()
-    m = re.search(r"#define\s+%s\s+(\d+)" % name, src) or re.search(r"constexpr int %s\s*=\s*([^;]+);" % name, src)
+    m = re.search(r"constexpr int %s\s*=\s*([^;]+);" % name, _tc_source())
     assert m, name
     return m.group(1).strip()
 
 
-def test_fused_whi_wlo_mma_layout_invariants():
-    """TC_FUSE_WLO (gemm_tc.cu): ONE tcgen05.mma of N = TC_BN_CAP + tile_bn runs over the adjacent [Whi; Wlo] boxes of a stage and
+def test_fused_whi_wlo_mma_tmem_layout_and_smem_budget():
+    """3xFP16 (gemm_tc.cu): ONE tcgen05.mma of N = TC_BN_CAP + tile_bn runs over the adjacent [Whi; Wlo] boxes of a stage and
     lands in the adjacent [main | compensation] accumulators.  The layout facts that makes legal, checked against the source's
     constants: the compensation accumulator sits exactly TC_BN_CAP columns behind the main one, every wide N is a legal UMMA
     shape for M = 128 (multiple of 16, <= 256) and fits the 6-bit N field of the instruction descriptor, the wide write stays
@@ -74,7 +77,12 @@ def test_fused_whi_wlo_mma_layout_invariants():
     8-row swizzle atom of the 64-byte fp16 weight rows so that one descriptor walks both boxes."""
     cap = int(_tc_define("TC_BN_CAP"))
     bk = int(_tc_define("TC_BK"))
-    assert _tc_define("TC_FUSE_WLO") == "1"
+    src = _tc_source()
+    # the fp16 issue path is the fused one: the wide descriptor carries N = TC_BN_CAP + tile_bn, and the MMA that uses it
+    # writes from the main accumulator on, so that its upper TC_BN_CAP columns land in the compensation accumulator
+    assert re.search(r"idesc_wide = \(idesc & ~\(0x3fu << 17\)\) \| \(\(uint32_t\)\(\(TC_BN_CAP \+ tile_bn\) >> 3\) << 17\);", src)
+    assert re.search(r"umma_f16_ts\(d_main, t_hi, dbh \+ adv, idesc_wide,", src)
+    assert "umma_f16_ts(d_corr, t_hi, dbl" not in src            # no separate Ahi.Wlo MMA (the unfused three-MMA form)
     assert _tc_define("TC_COL_CORR").replace(" ", "") == "TC_BN_CAP"
     assert _tc_define("TC_COL_ACC").replace(" ", "") == "2*TC_BN_CAP"
     assert _tc_define("TC_COL_A").replace(" ", "") == "4*TC_BN_CAP"
@@ -90,10 +98,9 @@ def test_fused_whi_wlo_mma_layout_invariants():
     row_bytes = bk * 2                                  # fp16 weights: 64-byte rows, SWIZZLE_64B atoms of 8 rows = 512 B
     assert (cap * row_bytes) % (8 * row_bytes) == 0
     # shared memory of the launch (TcCfg<true>::SMEM_BYTES: stages sized for 96-row boxes whatever BN is) fits the 227 KB opt-in
-    src = open(os.path.join(ROOT, "flowcompare_b200", "csrc", "gemm_tc.cu")).read()
-    m = re.search(r"#define TC_STAGES_F16 \(TC_RES_PREFETCH \? (\d+) : (\d+)\)", src)
-    stages = int(m.group(1)) if _tc_define("TC_RES_PREFETCH") == "1" else int(m.group(2))
-    stg_floats = 1024 if _tc_define("TC_RES_PREFETCH") == "1" else 32 * 20
+    stages = int(_tc_define("TC_STAGES_F16"))
+    assert re.search(r"static constexpr int STAGES = F16 \? TC_STAGES_F16 : TC_STAGES;", src)
+    stg_floats = int(re.search(r"static constexpr int STG_FLOATS = F16 \? (\d+) :", src).group(1))
     smem = stages * (128 * bk * 4 + 2 * cap * bk * 2) + 8 * stg_floats * 4 + 1024
     assert smem <= 227 * 1024
 
